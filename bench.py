@@ -2,6 +2,7 @@
 """bench.py - agent-steps/s of the hot path (env step K1 + GAE scan K2) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload large|small]
+                    [--dump-outputs DIR]
 
 One bench "step" is one rollout segment: SEG env steps of all E environments (one marlsc_env_step call each =
 four launches of the split step K1a-K1d, or one fused launch; plus a reset launch when an episode ends) followed
@@ -101,6 +102,30 @@ def algorithmic_bytes_per_env_step(W, S, L, obs_dim, mean_orders, qty_bytes=1, l
     if layout == "compact":
         return W * S * (4 + 4 + L + 1 + 8) + 2 * mean_lines + 4 + tail
     return 4 * W * S * (L + 8) + mean_orders * (S * qty_bytes + 2) + tail
+
+
+# --------------------------------------------------------------------------------------- --dump-outputs
+DUMP_BYTES = 60 << 20    # what --dump-outputs writes stays under 64 MB in all
+
+
+def dump_outputs(out_dir, arrays, n_envs):
+    """Write the timed path's outputs as ``out_dir/<name>.npy`` (float32, float64 stays float64) so that two builds can be
+    compared output for output. ``arrays`` maps a name to (device tensor, axis of the environment index). When the whole
+    batch does not fit DUMP_BYTES, the same environments are kept in every array: a fixed seeded sample, identical from
+    run to run."""
+    import numpy as np
+    import torch
+    wide = {name: t.dtype == torch.float64 for name, (t, _) in arrays.items()}
+    per_env = sum(t.numel() // n_envs * (8 if wide[name] else 4) for name, (t, _) in arrays.items())
+    k = min(n_envs, DUMP_BYTES // per_env)
+    if k == 0:
+        raise ValueError(f"--dump-outputs: one environment's outputs ({per_env} bytes) exceed the {DUMP_BYTES}-byte cap")
+    idx = np.arange(n_envs) if k == n_envs else np.sort(np.random.default_rng(0).choice(n_envs, k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (t, axis) in arrays.items():
+        sel = t.index_select(axis, torch.from_numpy(idx).to(t.device))
+        np.save(os.path.join(out_dir, name + ".npy"), sel.to(torch.float64 if wide[name] else torch.float32).cpu().numpy())
+    print(f"dump-outputs: {', '.join(arrays)} of {k} of {n_envs} environments -> {out_dir}", file=sys.stderr, flush=True)
 
 
 # --------------------------------------------------------------------------------------- clocks
@@ -260,7 +285,7 @@ def _cpu_worker(args):
 
 
 def _ref_worker(args):
-    """The reference's own InventoryEnvironment (oracle/_ref, or /root/reference in the build container) under the
+    """The reference's own InventoryEnvironment (the checkout at MARLSC_REFERENCE_ROOT, or its copy in oracle/_ref) under the
     base-stock heuristic with its own Poisson demand sampler: the same segment the GPU arm times, on one host core."""
     env_dict, n_envs, steps, seed, z = args
     import numpy as np
@@ -315,8 +340,8 @@ def cpu_port(env_dict, n_envs_per_worker, steps, workers, kind="port", z=2.0):
 
 
 def reference_kind():
-    """"reference" when the reference's own env can be imported here (oracle/_ref made by oracle/make_ref.py, or the build
-    container's /root/reference), else "port" (oracle/inventory_oracle.py)."""
+    """"reference" when the reference's own env can be imported here (oracle/_ref made by oracle/make_ref.py, or the
+    checkout at MARLSC_REFERENCE_ROOT), else "port" (oracle/inventory_oracle.py)."""
     try:
         from oracle import ref_harness as H
         return "reference" if H.available() else "port"
@@ -359,7 +384,8 @@ def run_reference(args):
                 e2e=dict(value=value, unit=UNIT, h2d_bytes_per_step=0, d2h_bytes_per_step=0), gpu_launches=0,
                 note=("timed: the reference's own Python env step + a NumPy GAE restatement (RLlib, which owns GAE in the "
                       "reference, is not installable here)") if kind == "reference" else
-                     "oracle/_ref is missing (run oracle/make_ref.py where /root/reference is mounted): timed the CPU oracle port")
+                     "oracle/_ref is missing (run oracle/make_ref.py with MARLSC_REFERENCE_ROOT set to a marl-sc checkout): "
+                     "timed the CPU oracle port")
     print(json.dumps(line), flush=True)
 
 
@@ -554,6 +580,10 @@ def run_ours(args):
     elapsed_ms = start.elapsed_time(stop)
     launches = L.marlsc_launch_count() - launches0
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the last timed segment: its rewards, GAE advantages / targets and the observations of its last env step
+        dump_outputs(args.dump_outputs, dict(observations=(obs_buf[(counter[0] - 1) & 1], 0), rewards=(rewards, 1),
+                                             advantages=(adv, 1), targets=(tgt, 1)), E)
     # per-launch durations of the step's kernels: a separate short pass with the library's own CUDA events
     # around each launch (marlsc_env_set_timing); each step is read back before the next one starts
     per_launch = []
@@ -932,6 +962,9 @@ def run_rollout(args):
     b.record()
     barrier()
     ms = a.elapsed_time(b)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {name: (getattr(ro, name), 1) for name in
+                                         ("obs", "actions", "logp", "rewards", "values", "advantages", "targets")}, E)
     if world > 1:
         tm = torch.tensor([ms], device=dev)
         dist.all_reduce(tm, op=dist.ReduceOp.MAX)
@@ -1015,7 +1048,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-spot-check", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (at most 64 MB; a fixed sample of "
+                         "environments when the batch is larger; with several GPUs, rank 0's environments)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.workload in ("ippo", "mappo"):

@@ -1,13 +1,13 @@
-"""Generate tests/golden/*.npz from the UNMODIFIED reference env (run in the build container only).
+"""Generate tests/golden/*.npz from the UNMODIFIED reference env (needs a checkout of Jakoebly/marl-sc).
 
-    python tests/golden/make_golden.py [scenario ...]
+    MARLSC_REFERENCE_ROOT=<marl-sc checkout> python tests/golden/make_golden.py [scenario ...]
 
 For every scenario in scenarios.py this steps ``n_envs`` reference ``InventoryEnvironment`` instances
-(/root/reference/src/environment/envs/multi_env.py) seeded ``derive_env_seed(base_seed, 0, i)``
+(src/environment/envs/multi_env.py of the checkout) seeded ``derive_env_seed(base_seed, 0, i)``
 (src/utils/seed_manager.py:166-186) with pre-sampled float32 actions, records the demand orders and
 lead times its own samplers drew, and stores inputs + every per-step output (SURVEY.md section 8c
 parity classes). The committed vectors are what pins ``oracle/inventory_oracle.py`` and, through it,
-the CUDA path; ``/root/reference`` itself never travels to the GPU box.
+the CUDA path; no test needs the checkout itself.
 
 numpy's argsort tie-break is SIMD-dispatch dependent, so the script re-execs itself with
 NPY_DISABLE_CPU_FEATURES set (see oracle/ref_harness.py).
@@ -149,7 +149,7 @@ def generate(name: str) -> str:
             allow_region_mismatch=sc["allow_region_mismatch"], base_seed=sc["base_seed"],
             n_envs=N, steps=T, stochastic_lead=stochastic, lite=bool(sc.get("lite")), policy=sc.get("policy"),
             empirical=bool(sc.get("empirical")),
-            numpy=np.__version__, reference="Jakoebly/marl-sc @ /root/reference"))),
+            numpy=np.__version__, reference="Jakoebly/marl-sc"))),
         env_seeds=np.asarray(seeds, dtype=np.int64),
         actions=actions,
         order_ptr=np.asarray(ptr, dtype=np.int64),          # CSR over (env, step): row = i*T + t

@@ -18,9 +18,13 @@ from marlsc_b200.config import (ConfigFileError, ConfigValidationError, algorith
 from marlsc_b200.demand import pack_orders
 from marlsc_b200.seeds import ENVIRONMENT_SEEDS, SeedManager
 from marlsc_b200.spec import build_env_spec, local_obs_dim
+from oracle import ref_harness
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = ref_harness.REF_ROOT           # a checkout of the reference project (MARLSC_REFERENCE_ROOT), or its copy in oracle/_ref
+# the live comparisons run when a checkout is named (and fail if it is not one); without one they skip
+REF_GIVEN = bool(os.environ.get("MARLSC_REFERENCE_ROOT"))
+NO_REF = "compares with a checkout of the reference project: set MARLSC_REFERENCE_ROOT"
 
 IPPO = dict(algorithm=dict(
     name="ippo",
@@ -47,13 +51,15 @@ def test_env_yaml_roundtrip(tmp_path):
     assert cfg.features.rolling_demand_mean and not cfg.features.stockout
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted")
+@pytest.mark.skipif(not REF_GIVEN, reason=NO_REF)
 def test_reference_yaml_files_load_unmodified():
     import glob
     cwd = os.getcwd()
     os.chdir(REF)
     try:
-        for f in glob.glob("config_files/environments/*.yaml"):
+        envs = glob.glob("config_files/environments/*.yaml")
+        assert envs, f"no config_files/environments/*.yaml under {REF}"
+        for f in envs:
             cfg = load_environment_config(f)
             assert cfg.n_regions == cfg.n_warehouses
         for f in ("ippo", "mappo", "ippo_test", "mappo_test", "cppo"):
@@ -143,7 +149,7 @@ def test_custom_component_registration():
         registry.LOST_SALES_HANDLER_REGISTRY.pop("mine")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted")
+@pytest.mark.skipif(not (REF_GIVEN or ref_harness.available()), reason=NO_REF)
 def test_seed_manager_matches_reference():
     from oracle import ref_harness as H
     H.activate()
@@ -157,6 +163,34 @@ def test_seed_manager_matches_reference():
             assert a.get_rng(name).integers(0, 1 << 30) == b.get_rng(name).integers(0, 1 << 30)
     assert SeedManager.derive_env_seed(7, 1, 5) == RefSM.derive_env_seed(7, 1, 5)
     assert a.spawn_child_seeds("inventory", 4) == b.spawn_child_seeds("inventory", 4)
+
+
+def test_seed_manager_matches_recorded_reference_streams():
+    """What the reference's SeedManager gave, as recorded in every golden file: the per-environment seeds
+    derive_env_seed(base_seed, 0, i), and the first episode's "inventory" stream (uniform initial stock) and
+    "lead_time_sampler" stream (stochastic lead times, sampled through our registry component)."""
+    from golden_io import NAMES, Golden
+    streams = 0
+    for name in NAMES + ["empirical_regionmap"]:
+        g = Golden(name)
+        seeds = [SeedManager.derive_env_seed(g.meta["base_seed"], 0, i) for i in range(g.N)]
+        assert seeds == g["env_seeds"].tolist(), name
+        ic = g.env["initial_inventory"]
+        cfg = environment_config_from_dict(g.env) if g.meta["stochastic_lead"] else None
+        for i, seed in enumerate(seeds):
+            sm = SeedManager(seed, ENVIRONMENT_SEEDS)
+            sm.advance_episode()                              # what the first reset() does (multi_env.py:218-231)
+            if ic["type"] == "uniform":
+                drawn = sm.get_rng("inventory").integers(ic["params"]["min"], ic["params"]["max"] + 1, size=(g.W, g.S))
+                assert np.array_equal(drawn, g["init_inventory"][i]), (name, i)
+                streams += 1
+            if cfg is not None:
+                lt = registry.get_lead_time_sampler(cfg)
+                lt.reset(sm.get_rng("lead_time_sampler"))
+                for t in range(g.T):
+                    assert np.array_equal(lt.sample(), g["lead_times"][i, t]), (name, i, t)
+                streams += 1
+    assert streams == 24                                      # 8 initial stocks, 16 lead-time trajectories
 
 
 def test_seed_manager_basics():
@@ -526,8 +560,8 @@ def test_pack_lines_roundtrip_and_balance():
 def test_reference_arm_prints_the_contract_line():
     """`bench.py --impl reference` (no GPU needed): one JSON line with the reference arm's keys - the same metric / unit /
     config as the GPU arm, `impl`, a `cpu_baseline` describing this run and an `e2e` object with zero copy bytes. Runs the
-    reference's own env modules when oracle/_ref is populated (build() does that where /root/reference is mounted), else
-    the oracle port."""
+    reference's own env modules when oracle/_ref is populated (build() does that when MARLSC_REFERENCE_ROOT names a marl-sc
+    checkout), else the oracle port."""
     import json
     import subprocess
     import sys
@@ -543,6 +577,30 @@ def test_reference_arm_prints_the_contract_line():
     assert cb["kind"] in ("reference", "port") and cb["cores"] >= 1 and cb["value"] == line["value"] and cb["sample"]
     assert line["e2e"] == dict(value=line["value"], unit=line["unit"], h2d_bytes_per_step=0, d2h_bytes_per_step=0)
     assert "BASELINE configs[2]" in line["config"]["workload"]
+
+
+def test_bench_dump_outputs_writes_a_fixed_environment_sample(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: under the byte cap every array keeps the same seeded sample of environments (float32,
+    float64 kept), a second run writes identical files, and a batch that fits is written whole."""
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 20)
+    E, W, D, T = 4096, 3, 40, 20
+    obs, rew = torch.randn(E, W, D), torch.randn(T, E, W, dtype=torch.float64)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), dict(observations=(obs, 0), rewards=(rew, 1)), E)
+    o, r = np.load(tmp_path / "a" / "observations.npy"), np.load(tmp_path / "a" / "rewards.npy")
+    k = o.shape[0]
+    assert 0 < k < E and r.shape == (T, k, W) and o.dtype == np.float32 and r.dtype == np.float64
+    assert o.nbytes + r.nbytes <= bench.DUMP_BYTES
+    idx = np.flatnonzero(np.isin(obs[:, 0, 0].numpy(), o[:, 0, 0]))                # the sampled environments
+    assert len(idx) == k and np.array_equal(o, obs[idx].numpy()) and np.array_equal(r, rew[:, idx].numpy())
+    for name in ("observations", "rewards"):
+        assert np.array_equal(np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy"))
+    bench.dump_outputs(str(tmp_path / "whole"), dict(rewards=(rew[:, :64], 1)), 64)
+    assert np.array_equal(np.load(tmp_path / "whole" / "rewards.npy"), rew[:, :64].numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100)                # one environment's observations alone are 480 bytes
+    with pytest.raises(ValueError, match="exceed"):
+        bench.dump_outputs(str(tmp_path / "none"), dict(observations=(obs, 0)), E)
 
 
 def test_line_streams_carry_the_allocation_the_oracle_computes():
