@@ -324,7 +324,8 @@ int marlsc_lines_from_orders(marlsc_env_t* env, int64_t num_envs, const marlsc_s
 
 /* Test hook: the Poisson inversion K4 uses, evaluated for n given (lambda, u) pairs (device float32 arrays):
  * k_out[i] = the order count drawn from uniform u[i] at rate lambda[i] (tabulated == 0), or the quantity drawn through
- * the tabulated-CDF search the per-SKU quantities use (tabulated != 0; synchronises the stream). */
+ * the tabulated-CDF search the per-SKU quantities use (tabulated != 0). Rates >= 30 take the float64 walk from the
+ * mode in both cases. Synchronises the stream. */
 int marlsc_poisson_inverse(const float* lambda, const float* u, int64_t n, int32_t tabulated, int32_t* k_out, void* stream);
 
 /* Device lead-time sampler: the distribution of the reference's StochasticLeadTimeSampler.sample

@@ -5,8 +5,11 @@
 // per order a Bernoulli(probability_skus[r]) mask over SKUs and quantities max(1, Poisson(lambda_quantity[r,s])).
 // Orders are emitted region-major like the reference. The random stream is Philox4x32-10 keyed by
 // (seed; env, step, row, lane block), so it is reproducible and independent of the launch geometry, but it is
-// NOT the reference's PCG64 stream: equality is distributional (tests compare moments and the quantity
-// histogram against the reference sampler), replay/host sampling stays the bit-exact path.
+// NOT the reference's PCG64 stream: equality with the reference is distributional, replay/host sampling stays the
+// bit-exact path. The law is the reference's at every parameter: Poisson draws invert the exact CDF (float32 search
+// below rate 30, a float64 walk from the mode above) and a SKU is included with probability p to within 2^-33.
+// tests/sampler_reference.py recomputes every draw from the counters; tests/test_device_samplers.py replays the
+// kernels against it and checks the law against scipy.
 // Output is the padded order layout marlsc_step_io accepts: env e owns rows [e*max_orders, e*max_orders + count[e]).
 //
 // K5 evaluates the reference's base-stock heuristic (src/experiments/run_baselines.py:133-207) for every
@@ -39,10 +42,37 @@ __device__ __forceinline__ void philox4x32(uint32_t (&c)[4], uint64_t seed) {
 
 __device__ __forceinline__ float u01(uint32_t x) { return (x >> 8) * (1.0f / 16777216.0f); }   // [0,1)
 
-// Poisson(lambda) from uniforms: inversion by sequential search below 30, rounded normal above.
-__device__ __forceinline__ int poisson_from(float lambda, float u, float u2) {
+constexpr float kModeRate = 30.f;   // from this rate on, Poisson inversion starts at the mode instead of at 0
+
+// Poisson(lambda) by inversion: the smallest k with u <= P(X <= k).
+// Below kModeRate: sequential search from 0 in float32. At and above: a float64 walk from the mode m = floor(lambda),
+// starting from F(m) and P(m) (mode: the host's float64 values for this rate), up while u > F, down while
+// u <= F - P. This stays exact where a search from 0 would need ~lambda terms and lose float32 precision on the way.
+__device__ __forceinline__ int poisson_from_mode(float lambda, float u, const double* __restrict__ mode) {
+  const double lam = (double)lambda, ud = (double)u;
+  int k = (int)floorf(lambda);
+  double F = mode[0], p = mode[1];
+  if (ud > F) {
+    while (ud > F) {
+      ++k;
+      p *= lam / (double)k;
+      const double Fn = F + p;
+      if (Fn == F) break;                              // the float64 sum has stopped growing (u is at most 1 - 2^-24)
+      F = Fn;
+    }
+  } else {
+    while (k > 0 && ud <= F - p) {
+      F -= p;
+      p *= (double)k / lam;
+      --k;
+    }
+  }
+  return k;
+}
+
+__device__ __forceinline__ int poisson_from(float lambda, float u, const double* __restrict__ mode) {
   if (lambda <= 0.f) return 0;
-  if (lambda < 30.f) {
+  if (lambda < kModeRate) {
     // float32 running sum: in the far tail the terms drop below half an ulp of F and the sum plateaus a few ulp
     // short of 1 (2-3 x 2^-24 for lambda = 1, 3, 5), below the largest uniform 1 - 2^-24 - the search then has to stop
     // where the sum stops growing instead of running on to the cap.
@@ -57,25 +87,44 @@ __device__ __forceinline__ int poisson_from(float lambda, float u, float u2) {
     }
     return k;
   }
-  const float z = sqrtf(-2.f * __logf(fmaxf(u, 1e-7f))) * __cosf(6.2831853f * u2);
-  const float v = floorf(lambda + sqrtf(lambda) * z + 0.5f);
-  return v < 0.f ? 0 : (int)v;
+  return poisson_from_mode(lambda, u, mode);
 }
 
 constexpr int kCdf = 16;     // tabulated Poisson CDF entries per (region, SKU): P(X <= k), k < kCdf
+struct Inclusion {           // SKU inclusion with probability p (included): t = floor(4096 p), f = round(frac(4096 p) 2^20)
+  uint32_t t, f;
+  float inv_f;               // float(1 / f), 0 when f == 0
+};
 struct DemandParams {
   const float* lam_orders;   // [R]
   const float* prob;         // [R]
   const float* lam_qty;      // [R,S], or [R] when the rate does not vary over the SKUs of a region (sku_stride 0)
   const float* cdf_qty;      // [R,S,kCdf], or [R,kCdf]: 3 KB that stay in L1 instead of 320 KB of L2 lookups
-  int region_stride, sku_stride;   // cell (r, s) of lam_qty / cdf_qty is entry r * region_stride + s * sku_stride
+  const Inclusion* incl;     // [R]: inclusion split of prob
+  const double* mode_orders; // [R,2]: F(m), P(m) at the mode of lam_orders (rates >= kModeRate only)
+  const double* mode_qty;    // [R,S,2] or [R,2], like lam_qty
+  int region_stride, sku_stride;   // cell (r, s) of lam_qty / cdf_qty / mode_qty is entry r * region_stride + s * sku_stride
 };
+
+// SKU inclusion with probability p from one 32-bit word w, whose low 12 bits b12 and high 20 bits b20 are uniform:
+// included when b12 < t, or when b12 == t and b20 < f, with t = floor(4096 p) and f = round(frac(4096 p) * 2^20)
+// (host-computed from the double p): probability p to within 2^-33. The quantity uniform is b20 / 2^20, or
+// b20 * float(1 / f) for a cell included on the boundary bucket b12 == t (b20 is uniform below f there; the product
+// stays below 1). When 4096 p is an integer f is 0 and this is the plain 12-bit test.
+__device__ __forceinline__ bool included(uint32_t w, const Inclusion& in, float& uq) {
+  const uint32_t b12 = w & 0xfffu, b20 = w >> 12;
+  uq = (float)b20 * (1.0f / 1048576.0f);
+  if (b12 < in.t) return true;
+  if (b12 != in.t || b20 >= in.f) return false;
+  uq = (float)b20 * in.inv_f;
+  return true;
+}
 
 // Quantity max(1, Poisson(lambda)) by inversion: the smallest k with u <= P(X <= k), found by a four-step search of the
 // tabulated CDF (same result as poisson_from's sequential search up to float rounding of the table); beyond the table
-// the sequential search continues from its last entry. lambda >= 30 keeps the rounded-normal branch.
-__device__ __forceinline__ int quantity_from(const float* __restrict__ cdf, float lambda, float u, float u2) {
-  if (lambda >= 30.f || lambda <= 0.f) return poisson_from(lambda, u, u2);
+// the sequential search continues from its last entry. Rates >= kModeRate walk from the mode like poisson_from.
+__device__ __forceinline__ int quantity_from(const float* __restrict__ cdf, float lambda, float u, const double* __restrict__ mode) {
+  if (lambda >= kModeRate || lambda <= 0.f) return poisson_from(lambda, u, mode);
   int k = u > cdf[7] ? 8 : 0;
   k += u > cdf[k + 3] ? 4 : 0;
   k += u > cdf[k + 1] ? 2 : 0;
@@ -95,10 +144,10 @@ __device__ __forceinline__ int quantity_from(const float* __restrict__ cdf, floa
 
 // test hook: the inversions K4 uses, for given (lambda, u) pairs
 __global__ void poisson_inverse_kernel(const float* __restrict__ lambda, const float* __restrict__ u, long long n,
-                                       const float* __restrict__ cdf, int32_t* __restrict__ out) {
+                                       const float* __restrict__ cdf, const double* __restrict__ mode, int32_t* __restrict__ out) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  out[i] = cdf ? quantity_from(cdf + i * kCdf, lambda[i], u[i], 0.5f) : poisson_from(lambda[i], u[i], 0.5f);
+  out[i] = cdf ? quantity_from(cdf + i * kCdf, lambda[i], u[i], mode + 2 * i) : poisson_from(lambda[i], u[i], mode + 2 * i);
 }
 
 // one warp per environment
@@ -118,12 +167,12 @@ sample_demand_kernel(DemandParams dp, int R, int S, long long E, uint64_t seed, 
     if (r < R) {
       uint32_t c[4] = {(uint32_t)e, (uint32_t)(e >> 32) ^ 0x5bd1e995u, (uint32_t)step, (uint32_t)r};
       philox4x32(c, seed);
-      n = poisson_from(dp.lam_orders[r], u01(c[0]), u01(c[1]));
+      n = poisson_from(dp.lam_orders[r], u01(c[0]), dp.mode_orders + 2 * r);
     }
     for (int l = 0; l < 32 && r0 + l < R; ++l) {      // regions in ascending order, like the reference
       const int nr = __shfl_sync(0xffffffffu, n, l);
       const int rr = r0 + l;
-      const float p = dp.prob[rr];
+      const Inclusion in = dp.incl[rr];
       for (int i = 0; i < nr; ++i) {
         if (row >= omax) {                             // staging is full: drop the order and flag it
           if (lane == 0) atomicExch(overflow, 1);
@@ -139,11 +188,11 @@ sample_demand_kernel(DemandParams dp, int R, int S, long long E, uint64_t seed, 
             const int s = s0 + lane + 32 * j;
             if (s < S) {
               // one 32-bit word per SKU: 12 bits decide inclusion, the other 20 drive the Poisson inversion
-              const float ub = (float)(c[j] & 0xfffu) * (1.0f / 4096.0f);
-              const float uq = (float)(c[j] >> 12) * (1.0f / 1048576.0f);
+              float uq;
               int q = 0;
-              if (ub < p) {
-                q = quantity_from(dp.cdf_qty + (size_t)(rr * dp.region_stride + s * dp.sku_stride) * kCdf, dp.lam_qty[rr * dp.region_stride + s * dp.sku_stride], uq, ub * (1.0f / p));
+              if (included(c[j], in, uq)) {
+                const int cell = rr * dp.region_stride + s * dp.sku_stride;
+                q = quantity_from(dp.cdf_qty + (size_t)cell * kCdf, dp.lam_qty[cell], uq, dp.mode_qty + 2 * cell);
                 q = q < 1 ? 1 : (q > 255 ? 255 : q);
               }
               qty_e[(long long)row * S + s] = (uint8_t)q;
@@ -178,20 +227,18 @@ sample_demand_lines_kernel(DemandParams dp, int R, int S, long long E, uint64_t 
     if (r < R) {
       uint32_t c[4] = {(uint32_t)e, (uint32_t)(e >> 32) ^ 0x5bd1e995u, (uint32_t)step, (uint32_t)r};
       philox4x32(c, seed);
-      n = poisson_from(dp.lam_orders[r], u01(c[0]), u01(c[1]));
+      n = poisson_from(dp.lam_orders[r], u01(c[0]), dp.mode_orders + 2 * r);
     }
     for (int l = 0; l < 32 && r0 + l < R; ++l) {      // regions in ascending order, like the reference
       const int nr = __shfl_sync(0xffffffffu, n, l);
       const int rr = r0 + l;
-      const float p = dp.prob[rr];
       const int rm = region_map ? region_map[rr] : rr;
-      // The inclusion test on the raw 12 bits (ub < p  <=>  bits < ceil(4096 p), 4096 p being exact in float32), then only
-      // the cells that passed - 20 % - go through the quantity inversion: a lane walks its hit bits, so a trip of the
-      // inner loop serves one hit of every lane instead of one SKU slot of every lane. Orders are taken two at a time
-      // (two Philox calls in flight, hit counts of a pair are better balanced over the lanes than those of one order);
-      // within a lane the first order's lines still precede the second's.
-      const uint32_t thr = (uint32_t)ceilf(p * 4096.0f);
-      const float inv_p = 1.0f / p;
+      // The inclusion test first (included(), on the raw word), then only the cells that passed - 20 % - go through
+      // the quantity inversion: a lane walks its hit bits, so a trip of the inner loop serves one hit of every lane
+      // instead of one SKU slot of every lane. Orders are taken two at a time (two Philox calls in flight, hit counts
+      // of a pair are better balanced over the lanes than those of one order); within a lane the first order's lines
+      // still precede the second's.
+      const Inclusion in = dp.incl[rr];
       const float* const cdf_r = dp.cdf_qty + (size_t)rr * dp.region_stride * kCdf;
       const float* const lam_r = dp.lam_qty + (size_t)rr * dp.region_stride;
       for (int i = 0; i < nr; i += 2) {
@@ -205,8 +252,9 @@ sample_demand_lines_kernel(DemandParams dp, int R, int S, long long E, uint64_t 
 #pragma unroll
           for (int j = 0; j < 4; ++j) {
             const bool named = lane + 32 * j < S;
-            if (named && (c0[j] & 0xfffu) < thr) hits |= 1u << j;
-            if (named && two && (c1[j] & 0xfffu) < thr) hits |= 16u << j;
+            float uq;
+            if (named && included(c0[j], in, uq)) hits |= 1u << j;
+            if (named && two && included(c1[j], in, uq)) hits |= 16u << j;
           }
         }
         while (hits) {
@@ -216,9 +264,10 @@ sample_demand_lines_kernel(DemandParams dp, int R, int S, long long E, uint64_t 
           const uint32_t hi = j == 0 ? c1[0] : (j == 1 ? c1[1] : (j == 2 ? c1[2] : c1[3]));
           const uint32_t cj = b < 4 ? lo : hi;
           const int s = lane + 32 * j;
-          const float ub = (float)(cj & 0xfffu) * (1.0f / 4096.0f);
-          const float uq = (float)(cj >> 12) * (1.0f / 1048576.0f);
-          int q = quantity_from(cdf_r + (size_t)(s * dp.sku_stride) * kCdf, lam_r[s * dp.sku_stride], uq, ub * inv_p);
+          float uq;
+          (void)included(cj, in, uq);               // the cell passed: this only recomputes its quantity uniform
+          int q = quantity_from(cdf_r + (size_t)(s * dp.sku_stride) * kCdf, lam_r[s * dp.sku_stride], uq,
+                                dp.mode_qty + 2 * ((size_t)rr * dp.region_stride + s * dp.sku_stride));
           q = q < 1 ? 1 : (q > 255 ? 255 : q);
           if (cnt < stride) out[(long long)(cnt >> 1) * 64 + (cnt & 1)] = (uint16_t)(q | (rm << 8) | (j << 14));
           else over = true;
@@ -258,8 +307,8 @@ sample_demand_thread_kernel(DemandParams dp, int R, int S, long long E, uint64_t
   for (int r = 0; r < R; ++r) {
     uint32_t c[4] = {(uint32_t)e, (uint32_t)(e >> 32) ^ 0x5bd1e995u, (uint32_t)step, (uint32_t)r};
     philox4x32(c, seed);
-    const int nr = poisson_from(dp.lam_orders[r], u01(c[0]), u01(c[1]));
-    const float p = dp.prob[r];
+    const int nr = poisson_from(dp.lam_orders[r], u01(c[0]), dp.mode_orders + 2 * r);
+    const Inclusion in = dp.incl[r];
     for (int i = 0; i < nr; ++i) {
       if (row >= omax) {
         atomicExch(overflow, 1);
@@ -270,11 +319,11 @@ sample_demand_thread_kernel(DemandParams dp, int R, int S, long long E, uint64_t
         const int s0 = s & ~127, lane = s & 31, j = (s >> 5) & 3;   // the warp kernel's (block, lane, word) of SKU s
         uint32_t d[4] = {(uint32_t)e, (uint32_t)row | 0x80000000u, (uint32_t)step, (uint32_t)(s0 + lane)};
         philox4x32(d, seed);
-        const float ub = (float)(d[j] & 0xfffu) * (1.0f / 4096.0f);
-        const float uq = (float)(d[j] >> 12) * (1.0f / 1048576.0f);
+        float uq;
         int q = 0;
-        if (ub < p) {
-          q = quantity_from(dp.cdf_qty + (size_t)(r * dp.region_stride + s * dp.sku_stride) * kCdf, dp.lam_qty[r * dp.region_stride + s * dp.sku_stride], uq, ub * (1.0f / p));
+        if (included(d[j], in, uq)) {
+          const int cell = r * dp.region_stride + s * dp.sku_stride;
+          q = quantity_from(dp.cdf_qty + (size_t)cell * kCdf, dp.lam_qty[cell], uq, dp.mode_qty + 2 * cell);
           q = q < 1 ? 1 : (q > 255 ? 255 : q);
         }
         qty_e[(long long)row * S + s] = (uint8_t)q;
@@ -376,8 +425,37 @@ int launch_base_stock(const DevSpec& ds, const marlsc_env_state_t& st, const flo
 
 using namespace marlsc;
 
+namespace {
+
+// F(m) and P(m) at the mode m = floor(lambda) of Poisson(lambda), in double (poisson_from_mode). The sum runs down from
+// the mode until the terms stop counting, about 40 sqrt(lambda) of them; rates below kModeRate get zeros (unused).
+void mode_cdf(double lam, double* out) {
+  out[0] = out[1] = 0.0;
+  if (!(lam >= (double)kModeRate)) return;
+  const double m = std::floor(lam);
+  const double pm = std::exp(-lam + m * std::log(lam) - std::lgamma(m + 1.0));
+  double F = pm, p = pm;
+  for (double k = m; k > 0.0; k -= 1.0) {
+    p *= k / lam;
+    F += p;
+    if (p < F * 1e-18) break;
+  }
+  out[0] = F;
+  out[1] = pm;
+}
+
+// the Inclusion of included() for inclusion probability p
+Inclusion inclusion_split(double p) {
+  const double x = p * 4096.0, t = std::floor(x);
+  const double f = std::nearbyint((x - t) * 1048576.0);
+  if (f >= 1048576.0) return Inclusion{(uint32_t)t + 1u, 0u, 0.f};
+  return Inclusion{(uint32_t)t, (uint32_t)f, f > 0.0 ? (float)(1.0 / f) : 0.f};
+}
+
+}  // namespace
+
 struct marlsc_demand {
-  float* blob = nullptr;
+  void* blob = nullptr;
   DemandParams dp{};
   int R = 0, S = 0, device = 0;
 };
@@ -398,12 +476,23 @@ int marlsc_demand_create(int32_t n_regions, int32_t n_skus, const double* lambda
       }
   const int cols = per_region ? 1 : n_skus;
   const size_t n_cells = (size_t)n_regions * cols;
-  std::vector<float> host((size_t)2 * n_regions + n_cells * (1 + kCdf));
+  // one upload: floats (rates, CDF tables), then the inclusion splits, then the mode CDFs in double
+  const size_t n_f = (size_t)2 * n_regions + n_cells * (1 + kCdf);
+  const size_t off_i = (n_f * sizeof(float) + 7) & ~(size_t)7;
+  const size_t off_d = (off_i + (size_t)n_regions * sizeof(Inclusion) + 7) & ~(size_t)7;
+  const size_t bytes = off_d + (size_t)2 * (n_regions + n_cells) * sizeof(double);
+  std::vector<double> raw((bytes + 7) / 8);
+  unsigned char* base = reinterpret_cast<unsigned char*>(raw.data());
+  float* host = reinterpret_cast<float*>(base);
+  Inclusion* incl = reinterpret_cast<Inclusion*>(base + off_i);
+  double* mode = reinterpret_cast<double*>(base + off_d);
   for (int r = 0; r < n_regions; ++r) {
     if (!(lambda_orders[r] >= 0.0) || !(probability_skus[r] >= 0.0 && probability_skus[r] <= 1.0))
       return set_error(MARLSC_EINVAL, "lambda_orders must be >= 0 and probability_skus in [0,1]");
     host[r] = (float)lambda_orders[r];
     host[n_regions + r] = (float)probability_skus[r];
+    incl[r] = inclusion_split(probability_skus[r]);
+    mode_cdf((double)(float)lambda_orders[r], mode + 2 * r);
   }
   for (size_t i = 0; i < (size_t)n_regions * n_skus; ++i)
     if (!(lambda_quantity[i] >= 0.0)) return set_error(MARLSC_EINVAL, "lambda_quantity must be >= 0");
@@ -420,6 +509,7 @@ int marlsc_demand_create(int32_t n_regions, int32_t n_skus, const double* lambda
       }
       host[2 * n_regions + n_cells + i * kCdf + k] = (float)F;
     }
+    mode_cdf(lam, mode + 2 * (n_regions + i));
   }
   marlsc_demand* d = new (std::nothrow) marlsc_demand();
   if (!d) return set_error(MARLSC_ENOMEM, "out of host memory");
@@ -427,17 +517,21 @@ int marlsc_demand_create(int32_t n_regions, int32_t n_skus, const double* lambda
   d->S = n_skus;
   d->device = device;
   cudaError_t ce = cudaSetDevice(device);
-  if (ce == cudaSuccess) ce = cudaMalloc(&d->blob, host.size() * sizeof(float));
-  if (ce == cudaSuccess) ce = cudaMemcpy(d->blob, host.data(), host.size() * sizeof(float), cudaMemcpyHostToDevice);
+  if (ce == cudaSuccess) ce = cudaMalloc(&d->blob, bytes);
+  if (ce == cudaSuccess) ce = cudaMemcpy(d->blob, base, bytes, cudaMemcpyHostToDevice);
   if (ce != cudaSuccess) {
     if (d->blob) cudaFree(d->blob);
     delete d;
     return set_error(MARLSC_ECUDA, std::string("uploading demand parameters: ") + cudaGetErrorString(ce));
   }
-  d->dp.lam_orders = d->blob;
-  d->dp.prob = d->blob + n_regions;
-  d->dp.lam_qty = d->blob + 2 * n_regions;
-  d->dp.cdf_qty = d->blob + 2 * n_regions + n_cells;
+  const float* fb = static_cast<const float*>(d->blob);
+  d->dp.lam_orders = fb;
+  d->dp.prob = fb + n_regions;
+  d->dp.lam_qty = fb + 2 * n_regions;
+  d->dp.cdf_qty = fb + 2 * n_regions + n_cells;
+  d->dp.incl = reinterpret_cast<const Inclusion*>(static_cast<const unsigned char*>(d->blob) + off_i);
+  d->dp.mode_orders = reinterpret_cast<const double*>(static_cast<const unsigned char*>(d->blob) + off_d);
+  d->dp.mode_qty = d->dp.mode_orders + 2 * n_regions;
   d->dp.region_stride = cols;
   d->dp.sku_stride = per_region ? 0 : 1;
   *out = d;
@@ -488,11 +582,18 @@ int marlsc_demand_sample_lines(marlsc_demand_t* d, int64_t num_envs, uint64_t se
 int marlsc_poisson_inverse(const float* lambda, const float* u, int64_t n, int32_t tabulated, int32_t* k_out, void* stream) {
   if (!lambda || !u || !k_out || n < 1) return set_error(MARLSC_EINVAL, "null argument or n < 1");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
+  // the tables marlsc_demand_create builds, for these rates: mode CDFs always, CDF rows when tabulated
+  std::vector<float> hl((size_t)n);
+  std::vector<double> hm((size_t)n * 2);
+  MARLSC_CUDA(cudaMemcpyAsync(hl.data(), lambda, sizeof(float) * n, cudaMemcpyDeviceToHost, s));
+  MARLSC_CUDA(cudaStreamSynchronize(s));
+  for (int64_t i = 0; i < n; ++i) mode_cdf((double)hl[i], hm.data() + 2 * i);
+  double* mode = nullptr;
+  MARLSC_CUDA(cudaMalloc(&mode, hm.size() * sizeof(double)));
+  MARLSC_CUDA(cudaMemcpyAsync(mode, hm.data(), hm.size() * sizeof(double), cudaMemcpyHostToDevice, s));
   float* cdf = nullptr;
-  if (tabulated) {   // the table marlsc_demand_create builds, for these rates
-    std::vector<float> hl((size_t)n), hc((size_t)n * kCdf);
-    MARLSC_CUDA(cudaMemcpyAsync(hl.data(), lambda, sizeof(float) * n, cudaMemcpyDeviceToHost, s));
-    MARLSC_CUDA(cudaStreamSynchronize(s));
+  if (tabulated) {
+    std::vector<float> hc((size_t)n * kCdf);
     for (int64_t i = 0; i < n; ++i) {
       const double lam = (double)hl[i];
       double pk = std::exp(-lam), F = pk;
@@ -507,13 +608,12 @@ int marlsc_poisson_inverse(const float* lambda, const float* u, int64_t n, int32
     MARLSC_CUDA(cudaMalloc(&cdf, hc.size() * sizeof(float)));
     MARLSC_CUDA(cudaMemcpyAsync(cdf, hc.data(), hc.size() * sizeof(float), cudaMemcpyHostToDevice, s));
   }
-  poisson_inverse_kernel<<<(unsigned)((n + 127) / 128), 128, 0, s>>>(lambda, u, n, cdf, k_out);
+  poisson_inverse_kernel<<<(unsigned)((n + 127) / 128), 128, 0, s>>>(lambda, u, n, cdf, mode, k_out);
   g_launches.fetch_add(1, std::memory_order_relaxed);
   MARLSC_CUDA(cudaGetLastError());
-  if (cdf) {
-    MARLSC_CUDA(cudaStreamSynchronize(s));
-    MARLSC_CUDA(cudaFree(cdf));
-  }
+  MARLSC_CUDA(cudaStreamSynchronize(s));
+  MARLSC_CUDA(cudaFree(mode));
+  if (cdf) MARLSC_CUDA(cudaFree(cdf));
   return MARLSC_OK;
 }
 

@@ -206,8 +206,9 @@ class BatchedInventoryEnv:
     # ------------------------------------------------------------------ on-device demand (K4)
     def enable_device_demand(self, seed: int = 0, max_orders_per_env: Optional[int] = None) -> None:
         """Draw demand on the device with the distribution of the reference's PoissonDemandSampler
-        (components/demand_sampler.py:105-163). The stream is Philox keyed by (seed, env, step): reproducible,
-        but not the reference's NumPy stream - use host samplers or replay when trajectories must match."""
+        (components/demand_sampler.py:105-163): Poisson order counts and quantities by exact inversion at every rate,
+        SKU inclusion with probability p (to within 2^-33). The stream is Philox keyed by (seed, env, step):
+        reproducible, but not the reference's NumPy stream - use host samplers or replay when trajectories must match."""
         smp = self.spec.components["demand_sampler"]
         if not hasattr(smp, "dense_params"):
             raise ValueError("device demand needs the 'poisson' demand sampler")
