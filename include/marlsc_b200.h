@@ -294,6 +294,37 @@ int marlsc_env_rollout_host(marlsc_env_t* env, const marlsc_env_state_t* state, 
                             const marlsc_host_step_t* host, int32_t n_steps, int32_t t0, float* rewards_dev,
                             void* stream);
 
+/* ---- per-episode metrics ---------------------------------------------------------------------------- */
+
+/* What an inventory study reports about an episode (reference: collect_step_info, multi_env.py:330-362, summed over the
+ * steps by the reference's baseline runs and seed evaluations): float64 DEVICE accumulators owned by the caller, summed
+ * over the steps since the last marlsc_env_reset. Costs are unscaled, with the definitions of marlsc_step_io.cost_breakdown.
+ * Per environment, demand_units == sum_w shipped_units + lost_units exactly; with agent-scope rewards
+ * episode_return ~= -scale_factor * (holding + penalty + outbound + inbound) row by row. */
+typedef struct marlsc_episode_metrics {
+  double* holding_cost;    /* [E,W] */
+  double* penalty_cost;    /* [E,W] lost-sales cost as the configured handler attributes it */
+  double* outbound_cost;   /* [E,W] */
+  double* inbound_cost;    /* [E,W] */
+  double* ordered_units;   /* [E,W] units placed (after rescale / clipping) */
+  double* shipped_units;   /* [E,W] units shipped from the warehouse to any region */
+  double* episode_return;  /* [E,W] sum of the float32 rewards the steps wrote */
+  double* demand_units;    /* [E]   units demanded (after the region map) */
+  double* lost_units;      /* [E]   units not fulfilled */
+} marlsc_episode_metrics_t;
+
+/* Register accumulators with the handle (it keeps a copy of the pointers; every one is required, else MARLSC_EINVAL),
+ * or m == NULL to stop accumulating. While set, marlsc_env_reset zeroes them on its stream (cudaMemsetAsync) and every
+ * step the handle runs (marlsc_env_step, marlsc_env_step_host, marlsc_env_rollout_host) adds to them, for the
+ * num_envs of the state it is given. Observations, rewards and state are the same as without metrics.
+ *   COMPACT: the split step's kernels accumulate as they go, plus one small launch that adds the rewards. The fused
+ *            kernel (marlsc_env_set_fused) has no metrics: the combination is MARLSC_EUNSUPPORTED.
+ *   WIDE:    the step's diagnostic outputs are folded into the accumulators by one extra launch, so marlsc_step_io must
+ *            carry cost_breakdown, d_ordered, d_ship and d_unfulfilled (else MARLSC_EINVAL); that selects the generic
+ *            step kernel. d_ship and d_unfulfilled accumulate, so the caller zeroes them before every step, which
+ *            marlsc_env_rollout_host cannot do: it returns MARLSC_EUNSUPPORTED on a WIDE handle with metrics. */
+int marlsc_env_set_metrics(marlsc_env_t* env, const marlsc_episode_metrics_t* m);
+
 /* ---- on-device samplers and heuristic policies (SURVEY.md section 8f) -------------------------------- */
 
 /* Device Poisson demand sampler: same distribution as the reference's PoissonDemandSampler

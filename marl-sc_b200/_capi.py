@@ -69,6 +69,13 @@ class HostStepC(C.Structure):
                 ("n_rounds", C.c_int64), ("action_qty", C.c_void_p)]
 
 
+class EpisodeMetricsC(C.Structure):
+    """marlsc_episode_metrics: float64 device accumulators, [E,W] except demand_units / lost_units [E]."""
+    _fields_ = [("holding_cost", C.c_void_p), ("penalty_cost", C.c_void_p), ("outbound_cost", C.c_void_p),
+                ("inbound_cost", C.c_void_p), ("ordered_units", C.c_void_p), ("shipped_units", C.c_void_p),
+                ("episode_return", C.c_void_p), ("demand_units", C.c_void_p), ("lost_units", C.c_void_p)]
+
+
 class MarlscError(RuntimeError):
     pass
 
@@ -111,6 +118,8 @@ def lib() -> C.CDLL:
     L.marlsc_env_set_generic.restype = C.c_int
     L.marlsc_env_set_fused.argtypes = [vp, i32]
     L.marlsc_env_set_fused.restype = C.c_int
+    L.marlsc_env_set_metrics.argtypes = [vp, C.POINTER(EpisodeMetricsC)]
+    L.marlsc_env_set_metrics.restype = C.c_int
     L.marlsc_env_set_timing.argtypes = [vp, i32]
     L.marlsc_env_set_timing.restype = C.c_int
     L.marlsc_env_last_timing.argtypes = [vp, C.POINTER(C.c_float), i32]

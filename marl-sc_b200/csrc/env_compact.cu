@@ -550,10 +550,13 @@ env_step_compact_kernel(const __grid_constant__ DevSpec sp, const __grid_constan
 // the ordinary one a resident CTA per SM)
 // LT: the lead-time horizon L as a compile-time constant (1..16; the plane loops then unroll without predicates: the
 // runtime-L form spent 16 instructions per plane load on them), 0 = read it from the spec.
-template <bool MS, bool POLICY, int LT>
+// STATS: also add the row's inbound cost and ordered units to the episode accumulators m (marlsc_env_set_metrics; only
+// instantiated with LT = 0, the other kernels ignore m).
+template <bool MS, bool POLICY, int LT, bool STATS = false>
 __global__ void __launch_bounds__(256)
 compact_place_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__ marlsc_env_state_t st,
-                     const __grid_constant__ marlsc_step_io_t io, double* __restrict__ cost_rows, int t) {
+                     const __grid_constant__ marlsc_step_io_t io, double* __restrict__ cost_rows, int t,
+                     const __grid_constant__ marlsc_episode_metrics_t m) {
   extern __shared__ __align__(16) unsigned char smem[];           // [8 warps][L * S] row images
   constexpr int KMAX = LT ? LT : kCompactMaxL;
   const int W = sp.W, S = sp.S, L = LT ? LT : sp.L, WS = W * S;
@@ -659,6 +662,13 @@ compact_place_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
     for (int o = 16; o > 0; o >>= 1) inb += __shfl_xor_sync(FULL, inb, o);
     if (lane == 0) cost_rows[row] = inb;
   }
+  if (STATS) {                                        // one warp per row: lane 0 owns the row's accumulators
+    if (!by_row) nQ = __reduce_add_sync(FULL, nQ);
+    if (lane == 0) {
+      m.inbound_cost[row] += by_row ? (double)nPos * sp.in_fixed[w * S] + ((double)nQ * sp.skw[0]) * sp.in_var[w * S] : inb;
+      m.ordered_units[row] += (double)nQ;
+    }
+  }
   __syncwarp();                                       // image complete
   if (mine) {                                         // the ring row, every plane as whole words
     int po = po0;
@@ -686,11 +696,13 @@ compact_place_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
 
 // K1b': one warp per environment - stock into shared memory, allocation chains over the environment's lines, stock back,
 // outbound + lost-sales cost per warehouse to cost_alloc. A lane owns the SKUs its stream's map word names.
-template <int NCH, int FS>
+// STATS: also add each warehouse's outbound cost, lost-sales cost and shipped units, and the environment's lost and
+// demanded units, to the episode accumulators m (marlsc_env_set_metrics; the other kernels ignore m).
+template <int NCH, int FS, bool STATS = false>
 __global__ void __launch_bounds__(kCompactWarps * 32, MARLSC_ALLOC_CTAS)
 compact_alloc_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__ marlsc_env_state_t st,
                      const __grid_constant__ marlsc_step_io_t io, const __grid_constant__ CompactSmem lay,
-                     double* __restrict__ cost_alloc, int t) {
+                     double* __restrict__ cost_alloc, int t, const __grid_constant__ marlsc_episode_metrics_t m) {
   extern __shared__ __align__(16) unsigned char smem[];
   const int W = sp.W, S = sp.S, R = sp.R, WS = W * S;
   {
@@ -794,15 +806,51 @@ compact_alloc_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
     for (int d = 0; d < 4; ++d) {
       if (w0 + d < W) {
         double c = 0.0;
+        double c_out = 0.0, c_pen = 0.0;              // STATS: the two parts of c
 #pragma unroll
         for (int qq = 0; qq < 2; ++qq) {
           if (sq[d][qq] > 0u) c += (double)sq[d][qq] * (ov[d][qq] + rate[qq]);
           if (close_w[qq] == w0 + d) c += lump[qq];
+          if (STATS) {
+            c_out += (double)sq[d][qq] * ov[d][qq];
+            c_pen += (double)sq[d][qq] * rate[qq] + (close_w[qq] == w0 + d ? lump[qq] : 0.0);
+          }
         }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(FULL, c, o);
         if (lane == 0) cost_alloc[e * W + w0 + d] = c;
+        if (STATS) {                                  // one warp per environment: lane 0 owns its accumulators
+#pragma unroll
+          for (int o = 16; o > 0; o >>= 1) {
+            c_out += __shfl_xor_sync(FULL, c_out, o);
+            c_pen += __shfl_xor_sync(FULL, c_pen, o);
+          }
+          const uint32_t shipped = __reduce_add_sync(FULL, sq[d][0] + sq[d][1]);
+          if (lane == 0) {
+            const int64_t i = e * W + w0 + d;
+            m.outbound_cost[i] += c_out;
+            m.penalty_cost[i] += c_pen;
+            m.shipped_units[i] += (double)shipped;
+          }
+        }
       }
+    }
+  }
+  if (STATS) {                                        // units demanded = shipped + lost (every line is one or the other)
+    uint32_t lost = 0u, shipped = 0u;
+#pragma unroll
+    for (int qq = 0; qq < 2; ++qq) {
+      const int r = lane + 32 * qq;
+      if (r < R) {
+        lost += s_lostU[r];
+        for (int w = 0; w < W; ++w) shipped += s_shipq[w * R + r];
+      }
+    }
+    lost = __reduce_add_sync(FULL, lost);
+    shipped = __reduce_add_sync(FULL, shipped);
+    if (lane == 0) {
+      m.lost_units[e] += (double)lost;
+      m.demand_units[e] += (double)shipped + (double)lost;
     }
   }
 }
@@ -814,11 +862,13 @@ compact_alloc_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
 #ifndef MARLSC_FEAT_CTAS
 #define MARLSC_FEAT_CTAS 8
 #endif
-template <bool MS>
+// STATS: also add the row's holding cost to the episode accumulators m (marlsc_env_set_metrics; the other kernels ignore m).
+template <bool MS, bool STATS = false>
 __global__ void __launch_bounds__(256, MARLSC_FEAT_CTAS)
 compact_feature_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__ marlsc_env_state_t st,
                        const __grid_constant__ marlsc_step_io_t io, double* __restrict__ cost_rows,
-                       const double* __restrict__ cost_alloc, int t, int write_rewards) {
+                       const double* __restrict__ cost_alloc, int t, int write_rewards,
+                       const __grid_constant__ marlsc_episode_metrics_t m) {
   extern __shared__ __align__(16) unsigned char smem[];           // [8 warps][3 * S] floats: inventory | home demand | rolling mean
   const int W = sp.W, S = sp.S, WS = W * S;
   const int lane = threadIdx.x & 31;
@@ -892,6 +942,7 @@ compact_feature_kernel(const __grid_constant__ DevSpec sp, const __grid_constant
   }
   float* const obs_w = io.obs + (size_t)row * sp.obs_dim;
   if (lane == 0) {
+    if (STATS) m.holding_cost[row] += cost;           // one warp per row: lane 0 owns the row's accumulators
     cost += cost_in;                                  // + the inbound cost K1a' left there
     if (write_rewards) {                              // agent scope (multi_env.py:316-327): no reward kernel needed
       io.rewards[row] = (float)(-((cost + cost_al) * sp.scale));
@@ -1287,6 +1338,18 @@ int launch_split_nch(const LaunchArgs& a, const marlsc_step_io_t& io, const Spli
     MARLSC_CUDA(cudaFuncSetAttribute((const void*)compact_alloc_kernel<NCH, FS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (dev < kMaxDevices) configured_for[dev] = (int)smem;
   }
+  // episode metrics (marlsc_env_set_metrics): the STATS instantiations of K1a' (runtime lead horizon), K1b' and K1c'
+  const bool stats = wk.metrics != nullptr;
+  const marlsc_episode_metrics_t m = stats ? *wk.metrics : marlsc_episode_metrics_t{};
+  if (stats) {
+    static int stats_configured_for[kMaxDevices] = {0};
+    if (dev >= kMaxDevices || stats_configured_for[dev] < (int)smem) {
+      MARLSC_CUDA(cudaFuncSetAttribute((const void*)compact_alloc_kernel<NCH, FS, true>, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                       (int)cudaSharedmemCarveoutMaxShared));
+      MARLSC_CUDA(cudaFuncSetAttribute((const void*)compact_alloc_kernel<NCH, FS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      if (dev < kMaxDevices) stats_configured_for[dev] = (int)smem;
+    }
+  }
   const int64_t rows = a.st.num_envs * a.ds.W;
   const unsigned grid_rows = (unsigned)((rows + 7) / 8);
   const unsigned grid_envs = (unsigned)((a.st.num_envs + kCompactWarps - 1) / kCompactWarps);
@@ -1296,29 +1359,33 @@ int launch_split_nch(const LaunchArgs& a, const marlsc_step_io_t& io, const Spli
     const size_t img = (size_t)8 * a.ds.L * a.ds.S;
 #define MARLSC_PLACE_L(LT)                                                                                          \
   case LT:                                                                                                          \
-    if (policy) compact_place_kernel<MS, true, LT><<<grid_rows, 256, img, s>>>(a.ds, a.st, io, wk.cost_rows, t);     \
-    else compact_place_kernel<MS, false, LT><<<grid_rows, 256, img, s>>>(a.ds, a.st, io, wk.cost_rows, t);           \
+    if (policy) compact_place_kernel<MS, true, LT><<<grid_rows, 256, img, s>>>(a.ds, a.st, io, wk.cost_rows, t, m);  \
+    else compact_place_kernel<MS, false, LT><<<grid_rows, 256, img, s>>>(a.ds, a.st, io, wk.cost_rows, t, m);        \
     break;
-    switch (a.ds.L) {
+    if (stats) {
+      if (policy) compact_place_kernel<MS, true, 0, true><<<grid_rows, 256, img, s>>>(a.ds, a.st, io, wk.cost_rows, t, m);
+      else compact_place_kernel<MS, false, 0, true><<<grid_rows, 256, img, s>>>(a.ds, a.st, io, wk.cost_rows, t, m);
+    } else switch (a.ds.L) {
       MARLSC_PLACE_L(1) MARLSC_PLACE_L(2) MARLSC_PLACE_L(3) MARLSC_PLACE_L(4) MARLSC_PLACE_L(5) MARLSC_PLACE_L(6)
       MARLSC_PLACE_L(7) MARLSC_PLACE_L(8) MARLSC_PLACE_L(9) MARLSC_PLACE_L(10) MARLSC_PLACE_L(11) MARLSC_PLACE_L(12)
       MARLSC_PLACE_L(13) MARLSC_PLACE_L(14) MARLSC_PLACE_L(15) MARLSC_PLACE_L(16)
       default:
-        if (policy) compact_place_kernel<MS, true, 0><<<grid_rows, 256, img, s>>>(a.ds, a.st, io, wk.cost_rows, t);
-        else compact_place_kernel<MS, false, 0><<<grid_rows, 256, img, s>>>(a.ds, a.st, io, wk.cost_rows, t);
+        if (policy) compact_place_kernel<MS, true, 0><<<grid_rows, 256, img, s>>>(a.ds, a.st, io, wk.cost_rows, t, m);
+        else compact_place_kernel<MS, false, 0><<<grid_rows, 256, img, s>>>(a.ds, a.st, io, wk.cost_rows, t, m);
     }
 #undef MARLSC_PLACE_L
   }
   MARLSC_CUDA(cudaGetLastError());
   if (wk.marks) MARLSC_CUDA(cudaEventRecord(wk.marks[1], s));
-  compact_alloc_kernel<NCH, FS><<<grid_envs, kCompactWarps * 32, smem, s>>>(a.ds, a.st, io, lay, wk.cost_alloc, t);
+  if (stats) compact_alloc_kernel<NCH, FS, true><<<grid_envs, kCompactWarps * 32, smem, s>>>(a.ds, a.st, io, lay, wk.cost_alloc, t, m);
+  else compact_alloc_kernel<NCH, FS><<<grid_envs, kCompactWarps * 32, smem, s>>>(a.ds, a.st, io, lay, wk.cost_alloc, t, m);
   MARLSC_CUDA(cudaGetLastError());
   if (wk.marks) MARLSC_CUDA(cudaEventRecord(wk.marks[2], s));
   const int agent_scope = a.ds.scope == MARLSC_SCOPE_AGENT;
   // bulk-copy version when an environment's blocks are 16-byte granular (W S a multiple of 8) and aligned
   const auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
   const size_t feat_smem = (size_t)kFeatStages * (1 + kWindow) * 2 * a.ds.W * a.ds.S + 16 * kFeatStages;
-  if (a.ds.feature_bulk && al16(a.st.inventory) && al16(a.st.demand_hist) && (int)feat_smem <= a.max_smem_optin) {
+  if (!stats && a.ds.feature_bulk && al16(a.st.inventory) && al16(a.st.demand_hist) && (int)feat_smem <= a.max_smem_optin) {
     static int feat_configured[kMaxDevices] = {0};
     int sms = 0;
     MARLSC_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
@@ -1331,9 +1398,12 @@ int launch_split_nch(const LaunchArgs& a, const marlsc_step_io_t& io, const Spli
     const int per_sm = imax_host(1, imin_host((int)(220 * 1024 / feat_smem), 2048 / (32 * a.ds.W)));
     const unsigned grid_feat = (unsigned)std::min<int64_t>(a.st.num_envs, (int64_t)sms * per_sm);
     compact_feature_bulk_kernel<MS><<<grid_feat, 32 * a.ds.W, feat_smem, s>>>(a.ds, a.st, io, wk.cost_rows, wk.cost_alloc, t, agent_scope);
+  } else if (stats) {
+    compact_feature_kernel<MS, true><<<grid_rows, 256, (size_t)8 * 3 * a.ds.S * sizeof(float), s>>>(a.ds, a.st, io, wk.cost_rows, wk.cost_alloc,
+                                                                                                   t, agent_scope, m);
   } else {
     compact_feature_kernel<MS><<<grid_rows, 256, (size_t)8 * 3 * a.ds.S * sizeof(float), s>>>(a.ds, a.st, io, wk.cost_rows, wk.cost_alloc, t,
-                                                                                             agent_scope);
+                                                                                             agent_scope, m);
   }
   MARLSC_CUDA(cudaGetLastError());
   if (wk.marks) MARLSC_CUDA(cudaEventRecord(wk.marks[3], s));

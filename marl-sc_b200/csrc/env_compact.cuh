@@ -75,4 +75,10 @@ int launch_base_stock_compact(const DevSpec& ds, const marlsc_env_state_t& st, c
 int launch_lines_from_orders(const DevSpec& ds, int64_t num_envs, const marlsc_step_io_t& io, int32_t line_stride, uint16_t* lines,
                              int32_t* line_counts, int32_t* overflow, cudaStream_t s);
 
+// Episode metrics (csrc/metrics.cu): after a COMPACT split step, add the step's rewards to episode_return; after a WIDE
+// step, fold its diagnostic outputs (cost_breakdown, d_ordered, d_ship, d_unfulfilled) and rewards into every accumulator.
+int launch_metrics_returns(const marlsc_episode_metrics_t& m, const float* rewards, int64_t num_envs, int W, cudaStream_t s);
+int launch_metrics_fold(const marlsc_episode_metrics_t& m, const marlsc_step_io_t& io, int64_t num_envs, int W, int R, int S,
+                        cudaStream_t s);
+
 }  // namespace marlsc

@@ -31,6 +31,7 @@ struct SplitWork {
   double* cost_alloc;   // [E,W] outbound + penalty cost (K1b)
   double* cost_rows;    // [E,W] holding + inbound cost (K1c)
   cudaEvent_t* marks;   // five events around the four launches when timing is on (marlsc_env_set_timing), else null
+  const marlsc_episode_metrics_t* metrics = nullptr;   // compact split step: episode accumulators (marlsc_env_set_metrics), or null
 };
 
 // Lookup tables straight from global memory (a few KB, read-only, L1 resident) for the kernels without scratch.

@@ -70,6 +70,8 @@ struct marlsc_env {
   cudaStream_t copy_stream = nullptr;        // marlsc_env_rollout_host: H2D copies of the next step
   cudaEvent_t ready[2] = {nullptr, nullptr};  // staging set filled
   cudaEvent_t done[2] = {nullptr, nullptr};   // staging set consumed by its step kernel
+  int metrics_on = 0;                         // marlsc_env_set_metrics: episode accumulators registered
+  marlsc_episode_metrics_t metrics = {};
 };
 
 namespace {
@@ -382,7 +384,26 @@ int marlsc_env_set_generic(marlsc_env_t* env, int32_t on) {
 
 int marlsc_env_set_fused(marlsc_env_t* env, int32_t on) {
   if (!env) return set_error(MARLSC_EINVAL, "null handle");
+  if (on && env->metrics_on && env->layout == MARLSC_LAYOUT_COMPACT)
+    return set_error(MARLSC_EUNSUPPORTED, "the compact fused step kernel does not accumulate episode metrics (marlsc_env_set_metrics)");
   env->force_fused = on ? 1 : 0;                       // compact layout: the single fused kernel instead of the split step
+  return MARLSC_OK;
+}
+
+int marlsc_env_set_metrics(marlsc_env_t* env, const marlsc_episode_metrics_t* m) {
+  if (!env) return set_error(MARLSC_EINVAL, "null handle");
+  if (!m) {
+    env->metrics_on = 0;
+    env->metrics = marlsc_episode_metrics_t{};
+    return MARLSC_OK;
+  }
+  if (!m->holding_cost || !m->penalty_cost || !m->outbound_cost || !m->inbound_cost || !m->ordered_units || !m->shipped_units ||
+      !m->episode_return || !m->demand_units || !m->lost_units)
+    return set_error(MARLSC_EINVAL, "every marlsc_episode_metrics pointer is required");
+  if (env->force_fused && env->layout == MARLSC_LAYOUT_COMPACT)
+    return set_error(MARLSC_EUNSUPPORTED, "the compact fused step kernel does not accumulate episode metrics (marlsc_env_set_fused)");
+  env->metrics = *m;
+  env->metrics_on = 1;
   return MARLSC_OK;
 }
 
@@ -414,6 +435,14 @@ int marlsc_env_reset(marlsc_env_t* env, const marlsc_env_state_t* state, const i
   if (!init_inventory || !obs) return set_error(MARLSC_EINVAL, "init_inventory and obs must not be NULL");
   MARLSC_CUDA(cudaSetDevice(env->device));
   cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (env->metrics_on) {                               // a new episode: its accumulators start from zero
+    const marlsc_episode_metrics_t& m = env->metrics;
+    const size_t rows = sizeof(double) * (size_t)state->num_envs * env->ds.W, envs = sizeof(double) * (size_t)state->num_envs;
+    for (double* p : {m.holding_cost, m.penalty_cost, m.outbound_cost, m.inbound_cost, m.ordered_units, m.shipped_units, m.episode_return})
+      MARLSC_CUDA(cudaMemsetAsync(p, 0, rows, s));
+    MARLSC_CUDA(cudaMemsetAsync(m.demand_units, 0, envs, s));
+    MARLSC_CUDA(cudaMemsetAsync(m.lost_units, 0, envs, s));
+  }
   if (env->layout == MARLSC_LAYOUT_COMPACT) {
     const LaunchArgs lc{env->ds, *state, env->max_smem_optin, true};
     return launch_reset_compact(lc, init_inventory, per_env, obs, s);
@@ -429,7 +458,12 @@ int marlsc_env_reset(marlsc_env_t* env, const marlsc_env_state_t* state, const i
   MARLSC_DISPATCH_G(team, launch_reset_g, spl, la, init_inventory, per_env, obs, s)
 }
 
-int marlsc_env_step(marlsc_env_t* env, const marlsc_env_state_t* state, const marlsc_step_io_t* io, int32_t t, void* stream) {
+}  // extern "C"
+
+namespace {
+
+// marlsc_env_step without the episode-metrics epilogue
+int step_impl(marlsc_env_t* env, const marlsc_env_state_t* state, const marlsc_step_io_t* io, int32_t t, void* stream) {
   int rc = check_state(env, state);
   if (rc) return rc;
   if (!io) return set_error(MARLSC_EINVAL, "null io");
@@ -478,10 +512,12 @@ int marlsc_env_step(marlsc_env_t* env, const marlsc_env_state_t* state, const ma
       rc = ensure_work(env, state->num_envs);
       if (rc) return rc;
       const SplitWork wk{env->d_work, env->d_work + (size_t)env->work_envs * env->ds.W,
-                         (env->timing && io->lines) ? env->marks : nullptr};
+                         (env->timing && io->lines) ? env->marks : nullptr, env->metrics_on ? &env->metrics : nullptr};
       env->timed_launches = (env->timing && io->lines) ? 4 : 0;
       return launch_split_compact(lc, ioc, wk, t, s);
     }
+    if (env->metrics_on)
+      return set_error(MARLSC_EUNSUPPORTED, "episode metrics need the compact split step (not the fused kernel, fewer than 2^32 rows)");
     rc = launch_step_compact(lc, ioc, t, s);
     if (rc) return rc;
     if (env->timing) MARLSC_CUDA(cudaEventRecord(env->marks[n_marks], s));
@@ -522,6 +558,22 @@ int marlsc_env_step(marlsc_env_t* env, const marlsc_env_state_t* state, const ma
     return MARLSC_OK;
   }
   MARLSC_DISPATCH_G(team, launch_step_g, spl, la, *io, t, s)
+}
+
+}  // namespace
+
+extern "C" {
+
+int marlsc_env_step(marlsc_env_t* env, const marlsc_env_state_t* state, const marlsc_step_io_t* io, int32_t t, void* stream) {
+  const bool metrics = env && env->metrics_on && io;
+  if (metrics && env->layout == MARLSC_LAYOUT_WIDE && (!io->cost_breakdown || !io->d_ordered || !io->d_ship || !io->d_unfulfilled))
+    return set_error(MARLSC_EINVAL, "episode metrics on a WIDE handle need io.cost_breakdown, d_ordered, d_ship and d_unfulfilled");
+  const int rc = step_impl(env, state, io, t, stream);
+  if (rc || !metrics) return rc;
+  // after the step's last launch, on its stream
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (env->layout == MARLSC_LAYOUT_COMPACT) return launch_metrics_returns(env->metrics, io->rewards, state->num_envs, env->ds.W, s);
+  return launch_metrics_fold(env->metrics, *io, state->num_envs, env->ds.W, env->ds.R, env->ds.S, s);
 }
 
 }  // extern "C" (host-buffer entry points follow their staging helper)
@@ -597,6 +649,9 @@ int marlsc_env_rollout_host(marlsc_env_t* env, const marlsc_env_state_t* state, 
   if (rc) return rc;
   if (!staging || !host || !rewards_dev) return set_error(MARLSC_EINVAL, "null staging, host descriptors or rewards_dev");
   if (n_steps < 1 || t0 < 0) return set_error(MARLSC_EINVAL, "n_steps must be positive and t0 >= 0");
+  if (env->metrics_on && env->layout == MARLSC_LAYOUT_WIDE)
+    return set_error(MARLSC_EUNSUPPORTED, "episode metrics on a WIDE handle fold the diagnostic outputs, which the caller zeroes "
+                                          "before every step: use marlsc_env_step");
   MARLSC_CUDA(cudaSetDevice(env->device));
   if (!env->copy_stream) {
     MARLSC_CUDA(cudaStreamCreateWithFlags(&env->copy_stream, cudaStreamNonBlocking));

@@ -30,6 +30,18 @@ def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
     return None if t is None else t.data_ptr()
 
 
+# marlsc_episode_metrics (include/marlsc_b200.h), in field order: [E,W] accumulators, then the [E] ones
+METRICS_PER_ROW = ("holding_cost", "penalty_cost", "outbound_cost", "inbound_cost", "ordered_units", "shipped_units",
+                   "episode_return")
+METRICS_PER_ENV = ("demand_units", "lost_units")
+COST_METRICS = ("holding_cost", "penalty_cost", "outbound_cost", "inbound_cost")
+
+
+def fill_rate(demand_units: torch.Tensor, lost_units: torch.Tensor) -> torch.Tensor:
+    """Unit fill rate 1 - lost / demand, and 1 where nothing was demanded."""
+    return torch.where(demand_units > 0, 1.0 - lost_units / demand_units.clamp(min=1.0), torch.ones_like(demand_units))
+
+
 class DeviceOrders:
     """One step of demand resident on the device (CSR, see marlsc_b200.demand)."""
 
@@ -72,9 +84,11 @@ class BatchedInventoryEnv:
                  region_map: Optional[Sequence[int]] = None, env_seeds: Optional[Sequence[int]] = None,
                  host_samplers: bool = True, diagnostics: bool = False, team_size: int = 0,
                  generic_kernel: bool = False, fused_kernel: bool = False, device_demand: bool = False, demand_seed: int = 0,
-                 max_orders_per_env: Optional[int] = None, layout: Optional[str] = None):
+                 max_orders_per_env: Optional[int] = None, layout: Optional[str] = None, episode_metrics: bool = False):
         if num_envs < 1:
             raise ValueError("num_envs must be positive")
+        if episode_metrics and fused_kernel and layout == "compact":
+            raise ValueError("episode_metrics needs the compact layout's split step: the fused kernel does not accumulate them")
         if not torch.cuda.is_available():
             raise RuntimeError("BatchedInventoryEnv needs a CUDA device: this path has no CPU implementation")
         meta = env_meta or {}
@@ -165,7 +179,7 @@ class BatchedInventoryEnv:
                                           torch.zeros(1, dtype=torch.int16, device=dev),
                                           torch.zeros(16, dtype=torch.uint8, device=dev), 0)
         self.diag: Dict[str, torch.Tensor] = {}
-        if diagnostics:
+        if diagnostics or (episode_metrics and self.layout == "wide"):    # a wide handle folds its metrics from these
             R = self.n_regions
             self.diag = dict(
                 cost_breakdown=torch.zeros((E, W, 4), dtype=torch.float32, device=dev),
@@ -175,6 +189,13 @@ class BatchedInventoryEnv:
                 unfulfilled=torch.zeros((E, R, S), dtype=torch.int32, device=dev),
                 lost_orders=torch.zeros((E, R), dtype=torch.int32, device=dev),
                 lost_sales=torch.zeros((E, W, S), dtype=torch.float32, device=dev))
+        # per-episode accumulators (marlsc_env_set_metrics): zeroed by reset, added to by every step
+        self._metrics: Dict[str, torch.Tensor] = {}
+        if episode_metrics:
+            self._metrics = {k: torch.zeros((E, W), dtype=torch.float64, device=dev) for k in METRICS_PER_ROW}
+            self._metrics.update({k: torch.zeros(E, dtype=torch.float64, device=dev) for k in METRICS_PER_ENV})
+            self._metrics_c = _capi.EpisodeMetricsC(*[self._metrics[k].data_ptr() for k in METRICS_PER_ROW + METRICS_PER_ENV])
+            _capi.check(L.marlsc_env_set_metrics(self._h, C.byref(self._metrics_c)))
         self.timestep = 0
         self._seed, self._episode = seed, 0  # reproducible device-side initial stock (see _initial_inventory)
         self._frame = None                   # empirical demand: the packed frame on the device (marlsc_b200.data)
@@ -337,6 +358,24 @@ class BatchedInventoryEnv:
     def demand_overflowed(self) -> bool:
         """True when some environment drew more orders than max_orders_per_env (the surplus was dropped)."""
         return bool(self._dd is not None and int(self._dd["overflow"].item()) != 0)
+
+    # ------------------------------------------------------------------ per-episode metrics
+    @property
+    def has_episode_metrics(self) -> bool:
+        return bool(self._metrics)
+
+    def episode_metrics(self) -> Dict[str, torch.Tensor]:
+        """What the steps since the last reset added up to (reference: collect_step_info, multi_env.py:330-362, summed over
+        the episode), float64 on the device: ``holding_cost``, ``penalty_cost``, ``outbound_cost``, ``inbound_cost``
+        (unscaled), ``ordered_units``, ``shipped_units``, ``episode_return`` and ``total_cost`` per warehouse [E,W];
+        ``demand_units``, ``lost_units`` and the unit ``fill_rate`` (1 where nothing was demanded) per environment [E].
+        The accumulators themselves, not copies: the next step or reset changes them. Needs ``episode_metrics=True``."""
+        if not self._metrics:
+            raise ValueError("construct the environment with episode_metrics=True")
+        m = dict(self._metrics)
+        m["total_cost"] = sum(m[k] for k in COST_METRICS)
+        m["fill_rate"] = fill_rate(m["demand_units"], m["lost_units"])
+        return m
 
     # ------------------------------------------------------------------ heuristic policies (K5)
     def base_stock_actions(self, level: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
