@@ -398,8 +398,11 @@ int marlsc_standardize(float* x, int64_t n, void* workspace, void* stream);
  * src/algorithms/models/rlmodules/base.py:412-457; IPPO model sizes config_files/algorithms/ippo.yaml):
  *   out[n, :] = W2 act(W1 x[n, :] + b1) + b2,   activation 0 = ReLU, 1 = tanh, float32 throughout.
  * x [n_rows, in_dim], w1 [hidden, in_dim], b1 [hidden], w2 [out_dim, hidden], b2 [out_dim] (torch.nn.Linear layouts),
- * out [n_rows, out_dim], all on the device, contiguous. in_dim <= 64, out_dim <= 3 (action means of a 2-3 SKU network, or
- * the value); anything else: MARLSC_EUNSUPPORTED, use the library GEMMs. The hidden activations stay in registers. */
+ * out [n_rows, out_dim], all on the device, contiguous. in_dim <= 128, out_dim <= 16 (action means of a 2-3 SKU network or
+ * the value; the joint head of a centralised (CPPO) policy: W x local width inputs, W x S outputs); anything else:
+ * MARLSC_EUNSUPPORTED, use the library GEMMs. The hidden activations stay in registers. in_dim <= 64 with out_dim <= 3 runs
+ * the narrow kernel; wider heads a second form whose shared memory holds hidden x (in_dim padded to 16 / 32 / 64 / 128 +
+ * out_dim padded to 4 / 8 / 16 + 4) floats, MARLSC_EUNSUPPORTED past the device's per-block limit. */
 int marlsc_mlp1_forward(const float* x, int64_t n_rows, int32_t in_dim, const float* w1, const float* b1, int32_t hidden,
                         const float* w2, const float* b2, int32_t out_dim, int32_t activation, float* out, void* stream);
 
@@ -410,13 +413,15 @@ int marlsc_mlp1_forward(const float* x, int64_t n_rows, int32_t in_dim, const fl
 int marlsc_linear_in_forward(const float* x, int64_t n_rows, int32_t in_dim, const float* w, const float* b, int32_t hidden,
                              int32_t activation, float* out, void* stream);
 
-/* K7b - output layer of a deeper MLP head during rollouts: out[n, :] = W a[n, :] + b for out_dim <= 4 (the last
+/* K7b - output layer of a deeper MLP head during rollouts: out[n, :] = W a[n, :] + b for out_dim <= 16 (the last
  * nn.Linear of the reference's "mlp" networks, rlmodules/base.py:412-457, e.g. MAPPO's actor [14, 256, 256, 2] and
  * critic [56, 64, 64, 1], config_files/algorithms/mappo.yaml:43-55), where a = h, or - with pre_bias != NULL -
  * a = relu(h + pre_bias): h is then the RAW product of the hidden layer before, whose bias [in_dim] and ReLU are applied
  * on the way in (saves the separate epilogue pass the library GEMM runs over the activations). h [n_rows, in_dim]
  * (in_dim a multiple of 4, <= 2048), w [out_dim, in_dim], b [out_dim], out [n_rows, out_dim], float32, device,
- * contiguous, h / w / pre_bias 16-byte aligned. One pass over h at the HBM rate. */
+ * contiguous, h / w / pre_bias 16-byte aligned. One pass over h at the HBM rate. out_dim 5 to 16 (the joint action means
+ * of a centralised policy's deeper head) runs a second form that pads the outputs to 8 or 16; anything past 16 outputs is
+ * MARLSC_EUNSUPPORTED. */
 int marlsc_linear_out_forward(const float* h, int64_t n_rows, int32_t in_dim, const float* pre_bias, const float* w, const float* b,
                               int32_t out_dim, float* out, void* stream);
 

@@ -116,6 +116,126 @@ int launch_mlp1(const float* x, long long N, int D, const float* w1, const float
   return MARLSC_OK;
 }
 
+// The same head with a wide input or output: the joint head of a centralised policy reads the global state (W x local
+// width, up to 128 floats) and writes the joint action (W x S, up to 16 means). NOP: output count rounded up to 4 / 8 /
+// 16 (the padding weights are zero, the padding sums are not stored). Shared-memory record of hidden unit j: DP floats
+// of W1[j,:], then b1[j], then W2[0..NOP-1, j], padded to whole float4s. The record is consumed a float4 at a time, so
+// only x (ROWS x DP floats) and the ROWS x NOP sums stay in registers. Units in ascending order per output as in K7;
+// within a unit the inputs are summed in four interleaved partial sums.
+template <int DP, int ROWS, int ACT, int NOP>
+__global__ void __launch_bounds__(128)
+mlp1_wide_forward_kernel(const float* __restrict__ x, long long N, int D, const float* __restrict__ w1, const float* __restrict__ b1,
+                         int H, const float* __restrict__ w2, const float* __restrict__ b2, int O, float* __restrict__ out) {
+  extern __shared__ float4 s_rec[];
+  constexpr int P = DP + NOP + 4;
+  float* const s = reinterpret_cast<float*>(s_rec);
+  for (int i = threadIdx.x; i < H * P; i += blockDim.x) {
+    const int j = i / P, c = i - j * P;
+    float v = 0.0f;
+    if (c < D) v = w1[(long long)j * D + c];
+    else if (c == DP) v = b1[j];
+    else if (c > DP && c - DP - 1 < O) v = w2[(long long)(c - DP - 1) * H + j];
+    s[i] = v;
+  }
+  __syncthreads();
+  float bias[NOP];
+#pragma unroll
+  for (int k = 0; k < NOP; ++k) bias[k] = k < O ? b2[k] : 0.0f;
+  const long long stride = (long long)gridDim.x * blockDim.x * ROWS;
+  for (long long row0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * ROWS; row0 < N; row0 += stride) {
+    float xr[ROWS][DP];
+#pragma unroll
+    for (int r = 0; r < ROWS; ++r)
+#pragma unroll
+      for (int d = 0; d < DP; ++d) xr[r][d] = (d < D && row0 + r < N) ? x[(row0 + r) * D + d] : 0.0f;
+    float acc[ROWS][NOP];
+#pragma unroll
+    for (int r = 0; r < ROWS; ++r)
+#pragma unroll
+      for (int k = 0; k < NOP; ++k) acc[r][k] = bias[k];
+#pragma unroll 2
+    for (int j = 0; j < H; ++j) {
+      const float4* const rec = s_rec + j * (P / 4);
+      const float4 t0 = rec[DP / 4];                  // b1[j], W2[0..2, j]
+      // four partial sums per row (input quads q % 4): a 128-input dot product is not one 128-deep FMA chain
+      float hp[ROWS][4], h[ROWS];
+#pragma unroll
+      for (int r = 0; r < ROWS; ++r) {
+        hp[r][0] = t0.x;
+        hp[r][1] = hp[r][2] = hp[r][3] = 0.0f;
+      }
+#pragma unroll
+      for (int q = 0; q < DP / 4; ++q) {
+        const float4 t = rec[q];
+#pragma unroll
+        for (int r = 0; r < ROWS; ++r) {
+          float& a = hp[r][q & 3];
+          a = fmaf(xr[r][4 * q], t.x, a);
+          a = fmaf(xr[r][4 * q + 1], t.y, a);
+          a = fmaf(xr[r][4 * q + 2], t.z, a);
+          a = fmaf(xr[r][4 * q + 3], t.w, a);
+        }
+      }
+#pragma unroll
+      for (int r = 0; r < ROWS; ++r) {
+        h[r] = (hp[r][0] + hp[r][1]) + (hp[r][2] + hp[r][3]);
+        h[r] = ACT == 0 ? fmaxf(h[r], 0.0f) : tanhf(h[r]);
+        acc[r][0] = fmaf(h[r], t0.y, acc[r][0]);
+        acc[r][1] = fmaf(h[r], t0.z, acc[r][1]);
+        acc[r][2] = fmaf(h[r], t0.w, acc[r][2]);
+      }
+#pragma unroll
+      for (int q = 1; q < (NOP + 4) / 4; ++q) {       // W2[4q-1 .. 4q+2, j]
+        const float4 t = rec[DP / 4 + q];
+        const float tw[4] = {t.x, t.y, t.z, t.w};
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          if (4 * q - 1 + c >= NOP) continue;
+#pragma unroll
+          for (int r = 0; r < ROWS; ++r) acc[r][4 * q - 1 + c] = fmaf(h[r], tw[c], acc[r][4 * q - 1 + c]);
+        }
+      }
+    }
+#pragma unroll
+    for (int r = 0; r < ROWS; ++r)
+      if (row0 + r < N) {
+#pragma unroll
+        for (int k = 0; k < NOP; ++k)
+          if (k < O) out[(row0 + r) * O + k] = acc[r][k];
+      }
+  }
+}
+
+template <int DP, int ROWS>
+int launch_mlp1_wide(const float* x, long long N, int D, const float* w1, const float* b1, int H, const float* w2, const float* b2,
+                     int O, int act, float* out, cudaStream_t s) {
+  const int nop = O <= 4 ? 4 : (O <= 8 ? 8 : 16);
+  const size_t smem = (size_t)H * (DP + nop + 4) * sizeof(float);
+  int dev = 0, sms = 0, optin = 0;
+  MARLSC_CUDA(cudaGetDevice(&dev));
+  MARLSC_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  MARLSC_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+  if ((int)smem > optin) return set_error(MARLSC_EUNSUPPORTED, "mlp1_forward: the hidden layer's weights do not fit shared memory");
+  const long long want = (N + 128LL * ROWS - 1) / (128LL * ROWS);
+  const unsigned grid = (unsigned)(want < (long long)sms * 8 ? (want > 0 ? want : 1) : (long long)sms * 8);
+#define MARLSC_MLP1W(A, K)                                                                                                 \
+  {                                                                                                                        \
+    if (smem > 48 * 1024)                                                                                                  \
+      MARLSC_CUDA(cudaFuncSetAttribute((const void*)mlp1_wide_forward_kernel<DP, ROWS, A, K>,                              \
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                           \
+    mlp1_wide_forward_kernel<DP, ROWS, A, K><<<grid, 128, smem, s>>>(x, N, D, w1, b1, H, w2, b2, O, out);                  \
+  }
+  if (act == 0) {
+    if (nop == 4) MARLSC_MLP1W(0, 4) else if (nop == 8) MARLSC_MLP1W(0, 8) else MARLSC_MLP1W(0, 16)
+  } else {
+    if (nop == 4) MARLSC_MLP1W(1, 4) else if (nop == 8) MARLSC_MLP1W(1, 8) else MARLSC_MLP1W(1, 16)
+  }
+#undef MARLSC_MLP1W
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  MARLSC_CUDA(cudaGetLastError());
+  return MARLSC_OK;
+}
+
 // Output layer of a deeper head: out[n, :] = W h[n, :] + b with a handful of outputs (action means of a small network, the
 // value). The library GEMM path treats this as a [N x H] x [H x 2] product and reads the 805 MB of hidden activations at a
 // third of the HBM rate, then adds the bias in a second pass; here a warp takes a row as 16-byte words (one coalesced
@@ -165,6 +285,56 @@ linear_out_kernel(const float* __restrict__ h, long long N, int H, const float* 
     if (lane == 0) {
 #pragma unroll
       for (int k = 0; k < NO; ++k) out[row * NO + k] = acc[k] + b[k];
+    }
+  }
+}
+
+// The same output layer with 5 to 16 outputs (the joint action means of a centralised policy's deeper head). NOP: the
+// output count rounded up to 8 or 16; the weight rows past O are zero in shared memory and their sums are not stored.
+template <int NOP, bool PRE>
+__global__ void __launch_bounds__(256)
+linear_out_wide_kernel(const float* __restrict__ h, long long N, int H, const float* __restrict__ pre_bias, const float* __restrict__ w,
+                       const float* __restrict__ b, int O, float* __restrict__ out) {
+  extern __shared__ float4 s_w4[];                    // [NOP][H / 4], then (PRE) the producing layer's bias [H / 4]
+  const int H4 = H >> 2;
+  for (int i = threadIdx.x; i < NOP * H4; i += blockDim.x)
+    s_w4[i] = i < O * H4 ? reinterpret_cast<const float4*>(w)[i] : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+  if (PRE)
+    for (int i = threadIdx.x; i < H4; i += blockDim.x) s_w4[NOP * H4 + i] = reinterpret_cast<const float4*>(pre_bias)[i];
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
+  for (long long row = warp; row < N; row += n_warps) {
+    const float4* const hr = reinterpret_cast<const float4*>(h) + row * H4;
+    float acc[NOP];
+#pragma unroll
+    for (int k = 0; k < NOP; ++k) acc[k] = 0.0f;
+    for (int c = lane; c < H4; c += 32) {
+      float4 v = hr[c];
+      if (PRE) {
+        const float4 pb = s_w4[NOP * H4 + c];
+        v.x = fmaxf(v.x + pb.x, 0.0f);
+        v.y = fmaxf(v.y + pb.y, 0.0f);
+        v.z = fmaxf(v.z + pb.z, 0.0f);
+        v.w = fmaxf(v.w + pb.w, 0.0f);
+      }
+#pragma unroll
+      for (int k = 0; k < NOP; ++k) {
+        const float4 q = s_w4[k * H4 + c];
+        acc[k] = fmaf(v.x, q.x, acc[k]);
+        acc[k] = fmaf(v.y, q.y, acc[k]);
+        acc[k] = fmaf(v.z, q.z, acc[k]);
+        acc[k] = fmaf(v.w, q.w, acc[k]);
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < NOP; ++k)
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], o);
+    if (lane == 0) {
+#pragma unroll
+      for (int k = 0; k < NOP; ++k)
+        if (k < O) out[row * O + k] = acc[k] + b[k];
     }
   }
 }
@@ -274,29 +444,54 @@ using namespace marlsc;
 extern "C" int marlsc_mlp1_forward(const float* x, int64_t n_rows, int32_t in_dim, const float* w1, const float* b1, int32_t hidden,
                                    const float* w2, const float* b2, int32_t out_dim, int32_t activation, float* out, void* stream) {
   if (!x || !w1 || !b1 || !w2 || !b2 || !out) return set_error(MARLSC_EINVAL, "mlp1_forward: null pointer");
-  if (n_rows < 0 || in_dim < 1 || in_dim > 64 || hidden < 1 || out_dim < 1 || out_dim > 3 || (activation != 0 && activation != 1))
-    return set_error(MARLSC_EUNSUPPORTED, "mlp1_forward: in_dim <= 64, out_dim <= 3, activation 0 (ReLU) or 1 (tanh)");
+  if (n_rows < 0 || in_dim < 1 || in_dim > 128 || hidden < 1 || out_dim < 1 || out_dim > 16 || (activation != 0 && activation != 1))
+    return set_error(MARLSC_EUNSUPPORTED, "mlp1_forward: in_dim <= 128, out_dim <= 16, activation 0 (ReLU) or 1 (tanh)");
   if (n_rows == 0) return MARLSC_OK;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (in_dim <= 16) return launch_mlp1<16, 4>(x, n_rows, in_dim, w1, b1, hidden, w2, b2, out_dim, activation, out, s);
-  if (in_dim <= 32) return launch_mlp1<32, 2>(x, n_rows, in_dim, w1, b1, hidden, w2, b2, out_dim, activation, out, s);
-  return launch_mlp1<64, 1>(x, n_rows, in_dim, w1, b1, hidden, w2, b2, out_dim, activation, out, s);
+  if (in_dim <= 64 && out_dim <= 3) {
+    if (in_dim <= 16) return launch_mlp1<16, 4>(x, n_rows, in_dim, w1, b1, hidden, w2, b2, out_dim, activation, out, s);
+    if (in_dim <= 32) return launch_mlp1<32, 2>(x, n_rows, in_dim, w1, b1, hidden, w2, b2, out_dim, activation, out, s);
+    return launch_mlp1<64, 1>(x, n_rows, in_dim, w1, b1, hidden, w2, b2, out_dim, activation, out, s);
+  }
+  if (in_dim <= 16) return launch_mlp1_wide<16, 4>(x, n_rows, in_dim, w1, b1, hidden, w2, b2, out_dim, activation, out, s);
+  if (in_dim <= 32) return launch_mlp1_wide<32, 2>(x, n_rows, in_dim, w1, b1, hidden, w2, b2, out_dim, activation, out, s);
+  if (in_dim <= 64) return launch_mlp1_wide<64, 1>(x, n_rows, in_dim, w1, b1, hidden, w2, b2, out_dim, activation, out, s);
+  return launch_mlp1_wide<128, 1>(x, n_rows, in_dim, w1, b1, hidden, w2, b2, out_dim, activation, out, s);
 }
 
 extern "C" int marlsc_linear_out_forward(const float* h, int64_t n_rows, int32_t in_dim, const float* pre_bias, const float* w,
                                          const float* b, int32_t out_dim, float* out, void* stream) {
   if (!h || !w || !b || !out) return set_error(MARLSC_EINVAL, "linear_out_forward: null pointer");
-  if (n_rows < 0 || in_dim < 4 || (in_dim & 3) || in_dim > 2048 || out_dim < 1 || out_dim > 4 ||
+  if (n_rows < 0 || in_dim < 4 || (in_dim & 3) || in_dim > 2048 || out_dim < 1 || out_dim > 16 ||
       ((reinterpret_cast<uintptr_t>(h) | reinterpret_cast<uintptr_t>(w) | reinterpret_cast<uintptr_t>(pre_bias)) & 15u))
-    return set_error(MARLSC_EUNSUPPORTED, "linear_out_forward: in_dim a multiple of 4 (<= 2048), out_dim <= 4, 16-byte aligned h, w, pre_bias");
+    return set_error(MARLSC_EUNSUPPORTED, "linear_out_forward: in_dim a multiple of 4 (<= 2048), out_dim <= 16, 16-byte aligned h, w, pre_bias");
   if (n_rows == 0) return MARLSC_OK;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   int dev = 0, sms = 0;
   MARLSC_CUDA(cudaGetDevice(&dev));
   MARLSC_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  const size_t smem = (size_t)(out_dim + (pre_bias ? 1 : 0)) * in_dim * sizeof(float);
   const long long want = (n_rows + 7) / 8;
   const unsigned grid = (unsigned)(want < (long long)sms * 8 ? want : (long long)sms * 8);
+  if (out_dim > 4) {
+    // up to 17 x 2048 floats: past the default 48 KB of dynamic shared memory
+    const size_t smem = (size_t)((out_dim <= 8 ? 8 : 16) + (pre_bias ? 1 : 0)) * in_dim * sizeof(float);
+#define MARLSC_LOUTW(K, PRE)                                                                                              \
+  {                                                                                                                       \
+    if (smem > 48 * 1024)                                                                                                 \
+      MARLSC_CUDA(cudaFuncSetAttribute((const void*)linear_out_wide_kernel<K, PRE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    linear_out_wide_kernel<K, PRE><<<grid, 256, smem, s>>>(h, n_rows, in_dim, pre_bias, w, b, out_dim, out);              \
+  }
+    if (out_dim <= 8) {
+      if (pre_bias) MARLSC_LOUTW(8, true) else MARLSC_LOUTW(8, false)
+    } else {
+      if (pre_bias) MARLSC_LOUTW(16, true) else MARLSC_LOUTW(16, false)
+    }
+#undef MARLSC_LOUTW
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    MARLSC_CUDA(cudaGetLastError());
+    return MARLSC_OK;
+  }
+  const size_t smem = (size_t)(out_dim + (pre_bias ? 1 : 0)) * in_dim * sizeof(float);
 #define MARLSC_LOUT(K)                                                                                      \
   if (pre_bias) linear_out_kernel<K, true><<<grid, 256, smem, s>>>(h, n_rows, in_dim, pre_bias, w, b, out);  \
   else linear_out_kernel<K, false><<<grid, 256, smem, s>>>(h, n_rows, in_dim, pre_bias, w, b, out);

@@ -8,17 +8,20 @@ Environments never interact, so a multi-GPU run shards them by rank with no comm
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import Callable, Optional
+from typing import Callable, Optional, Union
 
 import torch
 
 from ..envs import BatchedInventoryEnv, DeviceOrders
 from .gae import compute_gae, standardize_, standardize_columns_
-from .policy import ActorCritic
+from .policy import ActorCritic, CentralizedActorCritic
 
 
 @dataclass
 class Rollout:
+    """Shapes for an ``ActorCritic``; with a ``CentralizedActorCritic`` the agent axis goes: actions and mean_old are
+    [T, E, W*S], logp / rewards (summed over the warehouses) / values / advantages / targets are [T(+1), E] and
+    log_std_old is [1, W*S]."""
     obs: torch.Tensor        # [T+1, E, W, D]
     actions: torch.Tensor    # [T, E, W, S] RAW (unclipped) samples - what ``logp`` refers to; the env saw clamp(-1, 1)
     logp: torch.Tensor       # [T, E, W]
@@ -39,26 +42,39 @@ def shard_envs(total_envs: int, rank: int, world_size: int) -> range:
 
 
 class RolloutCollector:
-    def __init__(self, env: BatchedInventoryEnv, policy: ActorCritic, horizon: int, gamma: float = 0.99,
-                 lam: float = 0.95, demand_fn: Optional[Callable[[int], DeviceOrders]] = None,
+    """Collects T steps of E environments under an ``ActorCritic`` (one sample per agent) or a
+    ``CentralizedActorCritic`` (CPPO: one sample per environment - the joint action, the summed reward, one value)."""
+
+    def __init__(self, env: BatchedInventoryEnv, policy: Union[ActorCritic, CentralizedActorCritic], horizon: int,
+                 gamma: float = 0.99, lam: float = 0.95, demand_fn: Optional[Callable[[int], DeviceOrders]] = None,
                  standardize_advantages: bool = True, seed: int = 0, keep_dist_inputs: bool = False,
                  obs_filter=None):
         self.env, self.policy, self.T = env, policy, int(horizon)
         self.gamma, self.lam = float(gamma), float(lam)
         self.demand_fn = demand_fn            # step index -> DeviceOrders; None = env host samplers
         self.standardize = standardize_advantages
-        self.obs_filter = obs_filter          # running MeanStdFilter (obs_normalization == "meanstd"), applied in place
+        # running MeanStdFilter (obs_normalization == "meanstd"), applied in place: per local column shared by the agents,
+        # or, for the centralised policy, per global column over the [E, W*D] view
+        self.obs_filter = obs_filter
         E, W, S, D, dev = env.num_envs, env.n_warehouses, env.n_skus, env.obs_dim, env.device
         T = self.T
+        central = isinstance(policy, CentralizedActorCritic)
+        if central and obs_filter is not None and obs_filter.mean.numel() != W * D:
+            raise ValueError(f"the centralised policy's observation filter normalises the global state: MeanStdFilter({W * D})")
+        self._flt_shape = (E, W * D) if central else (E, W, D)
+        agent = () if central else (W,)       # per-agent axis of the per-sample buffers
+        act = (W * S,) if central else (W, S)
         self.obs = torch.empty((T + 1, E, W, D), device=dev)
-        self.actions = torch.empty((T, E, W, S), device=dev)
-        self.mean_old = torch.empty((T, E, W, S), device=dev) if keep_dist_inputs else None   # use_kl_loss needs it
-        self.logp = torch.empty((T, E, W), device=dev)
-        self.rewards = torch.empty((T, E, W), device=dev)
-        self.values = torch.empty((T + 1, E, W), device=dev)
-        self.cut_values = torch.zeros((T, E, W), device=dev)
-        self.adv = torch.empty((T, E, W), device=dev)
-        self.targets = torch.empty((T, E, W), device=dev)
+        self.actions = torch.empty((T, E, *act), device=dev)
+        self.mean_old = torch.empty((T, E, *act), device=dev) if keep_dist_inputs else None   # use_kl_loss needs it
+        self.logp = torch.empty((T, E, *agent), device=dev)
+        self.rewards = torch.empty((T, E, *agent), device=dev)
+        # the step writes [E, W] rewards; the centralised policy's reward is their sum (CentralizedEnvWrapper.step)
+        self._step_rewards = torch.empty((E, W), device=dev) if central else None
+        self.values = torch.empty((T + 1, E, *agent), device=dev)
+        self.cut_values = torch.zeros((T, E, *agent), device=dev)
+        self.adv = torch.empty((T, E, *agent), device=dev)
+        self.targets = torch.empty((T, E, *agent), device=dev)
         self.gen = torch.Generator(device=dev)
         self.gen.manual_seed(seed)
         self._need_reset = True
@@ -72,7 +88,7 @@ class RolloutCollector:
         if self._need_reset:
             env.reset(obs_out=self.obs[0])
             if flt is not None:
-                flt(self.obs[0])
+                flt(self.obs[0].view(self._flt_shape))
             self._need_reset = False
         else:
             self.obs[0].copy_(self.obs[T])
@@ -86,9 +102,12 @@ class RolloutCollector:
             if self.mean_old is not None:
                 self.mean_old[t] = mean
             orders = self.demand_fn(self.total_steps) if self.demand_fn is not None else None
-            _, _, truncated = env.step(act.contiguous(), orders=orders, obs_out=self.obs[t + 1], rewards_out=self.rewards[t])
+            rew = self.rewards[t] if self._step_rewards is None else self._step_rewards
+            _, _, truncated = env.step(act.contiguous(), orders=orders, obs_out=self.obs[t + 1], rewards_out=rew)
+            if self._step_rewards is not None:
+                torch.sum(rew, dim=1, out=self.rewards[t])
             if flt is not None:
-                flt(self.obs[t + 1])
+                flt(self.obs[t + 1].view(self._flt_shape))
             self.total_steps += 1
             if truncated:
                 # the final observation bootstraps the value target (RLlib appends it to the episode); the
@@ -98,7 +117,7 @@ class RolloutCollector:
                 self.cut_values[t] = pol.value(self.obs[t + 1])
                 env.reset(obs_out=self.obs[t + 1])
                 if flt is not None:
-                    flt(self.obs[t + 1])
+                    flt(self.obs[t + 1].view(self._flt_shape))
         self.values[T] = pol.value(self.obs[T])
         cut = torch.tensor(cut_host, dtype=torch.uint8, device=env.device)
         compute_gae(self.rewards, self.values, self.gamma, self.lam, cut if any_cut else None,

@@ -13,7 +13,7 @@ import torch
 
 from ..envs import BatchedInventoryEnv
 from ..envs.batched_env import COST_METRICS, METRICS_PER_ENV, METRICS_PER_ROW, fill_rate
-from .policy import ActorCritic
+from .policy import ActorCritic, CentralizedActorCritic
 
 
 @dataclass
@@ -51,7 +51,7 @@ class EpisodeMetrics:
         return out
 
 
-Actor = Union[ActorCritic, torch.Tensor, np.ndarray, Callable[[torch.Tensor], torch.Tensor]]
+Actor = Union[ActorCritic, CentralizedActorCritic, torch.Tensor, np.ndarray, Callable[[torch.Tensor], torch.Tensor]]
 
 
 def _resolve_actor(env: BatchedInventoryEnv, actor: Actor):
@@ -62,6 +62,11 @@ def _resolve_actor(env: BatchedInventoryEnv, actor: Actor):
             raise ValueError(f"the ActorCritic maps {actor.local_obs_dim}-wide observations to {actor.action_dim} actions; the "
                              f"environment has {env.obs_dim} and {S}")
         return "actor_critic", actor
+    if isinstance(actor, CentralizedActorCritic):
+        if (actor.n_warehouses, actor.action_dim, actor.local_obs_dim) != (W, S, env.obs_dim):
+            raise ValueError(f"the CentralizedActorCritic is built for {actor.n_warehouses} warehouses x {actor.action_dim} SKUs "
+                             f"with {actor.local_obs_dim}-wide local observations; the environment has {W} x {S} and {env.obs_dim}")
+        return "centralized", actor
     if isinstance(actor, (torch.Tensor, np.ndarray)):
         if tuple(actor.shape) not in ((W, S), (E, W, S)):
             raise ValueError(f"a base-stock level must have shape {(W, S)} or {(E, W, S)}, got {tuple(actor.shape)}")
@@ -70,7 +75,7 @@ def _resolve_actor(env: BatchedInventoryEnv, actor: Actor):
         return "base_stock", torch.as_tensor(actor, dtype=torch.float32, device=env.device).contiguous()
     if callable(actor):
         return "callable", actor
-    raise ValueError("actor must be an ActorCritic, a base-stock level [W,S] / [E,W,S] or a callable obs -> actions")
+    raise ValueError("actor must be an ActorCritic, a CentralizedActorCritic, a base-stock level [W,S] / [E,W,S] or a callable obs -> actions")
 
 
 @torch.no_grad()
@@ -80,7 +85,8 @@ def evaluate(env: BatchedInventoryEnv, actor: Actor, num_episodes: int, orders_f
 
     ``actor`` is an ``ActorCritic`` (its mean action clipped to [-1, 1], the reference's ``explore=False`` path,
     src/algorithms/base.py:98-265, on the observations passed through ``obs_filter`` when given - a copy, the env's
-    buffer stays raw), a base-stock level [W,S] or [E,W,S] (evaluated inside the step on the compact layout, by the
+    buffer stays raw), a ``CentralizedActorCritic`` (the same with the joint mean action [E, W*S] viewed as [E, W, S]; its
+    filter normalises the [E, W*D] global state), a base-stock level [W,S] or [E,W,S] (evaluated inside the step on the compact layout, by the
     policy kernel otherwise), or a callable ``obs [E,W,obs_dim] -> actions [E,W,S]``. Demand comes from
     ``orders_fn(t)``, else from whatever the environment is set up with (device sampler, empirical frame, host samplers).
     Each episode starts with ``env.reset()``."""
@@ -105,6 +111,10 @@ def evaluate(env: BatchedInventoryEnv, actor: Actor, num_episodes: int, orders_f
             elif kind == "actor_critic":
                 x = obs if obs_filter is None else obs_filter(obs.clone())
                 a = pol.action_mean(x).clamp(-1.0, 1.0)
+            elif kind == "centralized":
+                # the joint mean action [E, W*S], warehouse-major; a CPPO filter normalises the [E, W*D] global state
+                x = obs if obs_filter is None else obs_filter(obs.clone().view(obs.shape[0], -1)).view(obs.shape)
+                a = pol.action_mean(x).clamp(-1.0, 1.0).view(obs.shape[0], env.n_warehouses, env.n_skus)
             else:
                 a = pol(obs)
             obs, _, done = env.step(a.contiguous(), orders=orders)

@@ -14,6 +14,8 @@ W policies still run as one kernel per layer.
 The centralised critic never materialises the W-times duplicated ``[local_i | global]`` vector: its first
 layer is split into a local and a global block, ``W1 [local|global]^T = Wl local_i^T + Wg global^T``,
 and the global term is computed once per environment.
+
+CPPO (src/algorithms/cppo.py) is :class:`CentralizedActorCritic`: one policy over the global state and the joint action.
 """
 from __future__ import annotations
 
@@ -76,15 +78,17 @@ def stacked_mlp(n: int, in_dim: int, hidden: Sequence[int], out_dim: int, activa
     return nn.Sequential(*layers)
 
 
-def _fused_mlp1(mods, h: torch.Tensor) -> Optional[torch.Tensor]:
-    """K7 (``marlsc_mlp1_forward``, csrc/mlp_forward.cu): a ``Linear -> ReLU|Tanh -> Linear`` head with at most 64 inputs and
-    3 outputs (the IPPO actor / critic of the small networks) in one kernel that keeps the hidden activations in
-    registers. Returns None when the network or the tensors do not qualify."""
+def _fused_mlp1(mods, h: torch.Tensor, max_in: int = 64, max_out: int = 3) -> Optional[torch.Tensor]:
+    """K7 (``marlsc_mlp1_forward``, csrc/mlp_forward.cu): a ``Linear -> ReLU|Tanh -> Linear`` head with at most ``max_in``
+    inputs and ``max_out`` outputs (by default 64 and 3: the IPPO actor / critic of the small networks; the kernel takes up
+    to 128 and 16) in one kernel that keeps the hidden activations in registers. Returns None when the network or the
+    tensors do not qualify."""
     if len(mods) != 3 or not isinstance(mods[0], nn.Linear) or not isinstance(mods[2], nn.Linear):
         return None
     act = 0 if isinstance(mods[1], nn.ReLU) else (1 if isinstance(mods[1], nn.Tanh) else -1)
     l1, l2 = mods[0], mods[2]
-    if (act < 0 or l1.bias is None or l2.bias is None or l1.in_features > 64 or l2.out_features > 3 or h.dtype != torch.float32
+    if (act < 0 or l1.bias is None or l2.bias is None or l1.in_features > max_in or l2.out_features > max_out
+            or h.dtype != torch.float32
             or any(t.dtype != torch.float32 or not t.is_contiguous() for t in (l1.weight, l1.bias, l2.weight, l2.bias))):
         return None
     from .. import _capi
@@ -98,9 +102,10 @@ def _fused_mlp1(mods, h: torch.Tensor) -> Optional[torch.Tensor]:
     return out
 
 
-def _linear_out_ok(m, h: torch.Tensor) -> bool:
-    """Shapes ``marlsc_linear_out_forward`` takes: a multiple of 4 inputs (<= 2048), at most 4 outputs."""
-    return (isinstance(m, nn.Linear) and m.bias is not None and m.out_features <= 4 and m.in_features % 4 == 0
+def _linear_out_ok(m, h: torch.Tensor, max_out: int = 4) -> bool:
+    """Shapes ``marlsc_linear_out_forward`` takes: a multiple of 4 inputs (<= 2048), at most ``max_out`` outputs (by
+    default 4; the kernel takes up to 16)."""
+    return (isinstance(m, nn.Linear) and m.bias is not None and m.out_features <= max_out and m.in_features % 4 == 0
             and 4 <= m.in_features <= 2048 and h.dtype == torch.float32 and m.weight.dtype == torch.float32
             and m.weight.is_contiguous() and m.bias.is_contiguous())
 
@@ -201,7 +206,12 @@ class ActorCritic(nn.Module):
     def from_algorithm_config(cls, algo_config, local_obs_dim: int, n_warehouses: int, action_dim: int) -> "ActorCritic":
         """``local_obs_dim`` must include the one-hot warehouse id when ``parameter_sharing`` is on: the reference
         turns ``include_warehouse_id`` on with it (ippo.py:70, mappo.py:67) - build the env with
-        ``env_meta_from_algorithm_config(algo_config)``."""
+        ``env_meta_from_algorithm_config(algo_config)``. A CPPO config is rejected: its model is
+        :class:`CentralizedActorCritic`."""
+        from ..config.schema import CPPOConfig
+        if isinstance(algo_config, CPPOConfig):
+            raise ValueError("a CPPO config describes one centralised policy over the joint action: build it with "
+                             "CentralizedActorCritic.from_algorithm_config")
         sp = algo_config.algorithm_specific
         net = sp.networks
         return cls(local_obs_dim, n_warehouses, action_dim, actor_hidden=net.actor.config.hidden_sizes,
@@ -266,9 +276,135 @@ class ActorCritic(nn.Module):
         return (self.clamped_log_std() + 1.4189385332046727).sum()
 
 
+# K7 runs a centralised one-hidden-layer head up to this many inputs (the kernel takes 128)
+_CENTRAL_K7_MAX_IN = 128
+
+
+def _mlp1_smem_bytes(in_dim: int, hidden: int, out_dim: int) -> int:
+    """Shared memory K7 needs for a head (csrc/mlp_forward.cu): hidden x (padded inputs + 4) floats for the narrow form
+    (<= 64 inputs, <= 3 outputs), hidden x (padded inputs + padded outputs + 4) for the wide one."""
+    if in_dim <= 64 and out_dim <= 3:
+        dp = 16 if in_dim <= 16 else (32 if in_dim <= 32 else 64)
+        return hidden * (dp + 4) * 4
+    dp = 16 if in_dim <= 16 else (32 if in_dim <= 32 else (64 if in_dim <= 64 else 128))
+    nop = 4 if out_dim <= 4 else (8 if out_dim <= 8 else 16)
+    return hidden * (dp + nop + 4) * 4
+
+
+def _central_forward(seq: nn.Sequential, x: torch.Tensor) -> torch.Tensor:
+    """``seq(x)`` for the :func:`mlp` heads of :class:`CentralizedActorCritic`, x ``[B, W*D]``. Without autograd on a CUDA
+    tensor a one-hidden-layer head runs in K7 (up to ``_CENTRAL_K7_MAX_IN`` inputs and 16 outputs, when its hidden layer's
+    weights fit the device's shared memory); any other head runs its hidden layers through the library GEMMs - the last one
+    as a plain product whose bias and ReLU K7b applies on the way in - and its output layer through K7b (up to 16
+    outputs)."""
+    if torch.is_grad_enabled() or not x.is_cuda or not hasattr(torch, "_addmm_activation"):
+        return seq(x)
+    mods = list(seq)
+    if (len(mods) == 3 and isinstance(mods[0], nn.Linear) and isinstance(mods[2], nn.Linear)
+            and _mlp1_smem_bytes(mods[0].in_features, mods[0].out_features, mods[2].out_features)
+            <= torch.cuda.get_device_properties(x.device).shared_memory_per_block_optin):
+        fused = _fused_mlp1(mods, x, max_in=_CENTRAL_K7_MAX_IN, max_out=16)
+        if fused is not None:
+            return fused
+    return _central_layers(mods, x)
+
+
+def _central_layers(mods, x: torch.Tensor) -> torch.Tensor:
+    """The layer-by-layer rollout forward of :func:`_central_forward`: library GEMMs for the hidden layers (the last one a
+    plain product whose bias and ReLU K7b applies on the way in), K7b for the output layer."""
+    h, i, last = x, 0, mods[-1]
+    while i < len(mods) - 1:
+        m = mods[i]
+        if isinstance(m, nn.Linear) and m.bias is not None and isinstance(mods[i + 1], nn.ReLU):
+            if i + 2 == len(mods) - 1 and _linear_out_ok(last, h, max_out=16) and m.bias.is_contiguous():
+                return _linear_out(torch.mm(h, m.weight.t()), last, pre_bias=m.bias)
+            h = torch._addmm_activation(m.bias, h, m.weight.t())
+            i += 2
+        else:
+            h = m(h)
+            i += 1
+    return _linear_out(h, last) if _linear_out_ok(last, h, max_out=16) else last(h)
+
+
+class CentralizedActorCritic(nn.Module):
+    """CPPO's model (reference: src/algorithms/cppo.py, RLlib single-agent PPO on ``CentralizedEnvWrapper``): one actor
+    MLP from the global state ``obs.reshape(B, W*D)`` to the joint action means ``[W*S]``, a free ``log_std [W*S]`` clamped
+    from below, and one critic MLP from the global state to the value.
+
+    The joint action is warehouse-major: entry ``w*S + s`` is warehouse w, SKU s (``CentralizedEnvWrapper._split_action``),
+    so ``[..., W*S]`` viewed as ``[..., W, S]`` is what the batched env takes. The interface is ActorCritic's, for the
+    collector, the learner and ``evaluate()``, with one policy and one log-prob and value per environment."""
+
+    n_policies = 1
+
+    def __init__(self, local_obs_dim: int, n_warehouses: int, action_dim: int, actor_hidden: Sequence[int] = (256,),
+                 critic_hidden: Sequence[int] = (256,), activation: str = "relu", logstd_init: float = 0.0,
+                 logstd_floor: float = -2.0):
+        super().__init__()
+        self.local_obs_dim, self.n_warehouses, self.action_dim = local_obs_dim, n_warehouses, action_dim
+        self.global_obs_dim = n_warehouses * local_obs_dim
+        self.joint_action_dim = n_warehouses * action_dim
+        self.logstd_floor = float(logstd_floor)
+        self.actor = mlp(self.global_obs_dim, actor_hidden, self.joint_action_dim, activation)
+        self.log_std = nn.Parameter(torch.full((self.joint_action_dim,), float(logstd_init)))
+        self.critic = mlp(self.global_obs_dim, critic_hidden, 1, activation)
+
+    @classmethod
+    def from_algorithm_config(cls, algo_config, local_obs_dim: int, n_warehouses: int,
+                              action_dim: int) -> "CentralizedActorCritic":
+        """From a CPPO config (``config_files/algorithms/cppo.yaml``); ``action_dim`` is the SKU count per warehouse. The
+        env carries no warehouse id (``env_meta_from_algorithm_config`` of a CPPO config)."""
+        from ..config.schema import CPPOConfig
+        if not isinstance(algo_config, CPPOConfig):
+            raise ValueError("CentralizedActorCritic is CPPO's model: IPPO and MAPPO configs build an ActorCritic")
+        sp = algo_config.algorithm_specific
+        net = sp.networks
+        return cls(local_obs_dim, n_warehouses, action_dim, actor_hidden=net.actor.config.hidden_sizes,
+                   critic_hidden=net.critic.config.hidden_sizes, activation=net.actor.config.activation,
+                   logstd_init=sp.logstd_init, logstd_floor=sp.logstd_floor)
+
+    def _head(self, seq: nn.Sequential, obs: torch.Tensor) -> torch.Tensor:
+        if tuple(obs.shape[-2:]) != (self.n_warehouses, self.local_obs_dim):
+            raise ValueError(f"obs must be [..., {self.n_warehouses}, {self.local_obs_dim}], got {tuple(obs.shape)}")
+        lead = obs.shape[:-2]
+        out = _central_forward(seq, obs.reshape(-1, self.global_obs_dim))
+        return out.reshape(*lead, out.shape[-1])
+
+    # obs: [B, W, D] local observations, flattened over W to the global state
+    def action_mean(self, obs: torch.Tensor) -> torch.Tensor:
+        """Joint action means [B, W*S]."""
+        return self._head(self.actor, obs)
+
+    def value(self, obs: torch.Tensor) -> torch.Tensor:
+        """[B]."""
+        return self._head(self.critic, obs).squeeze(-1)
+
+    def act(self, obs: torch.Tensor, generator: Optional[torch.Generator] = None, deterministic: bool = False,
+            return_raw: bool = False):
+        """As ``ActorCritic.act``: ``(clipped [B, W, S], logp [B], value [B])``, or with ``return_raw=True``
+        ``(clipped [B, W, S], raw [B, W*S], logp [B], value [B], mean [B, W*S])``."""
+        mean = self.action_mean(obs)
+        if deterministic:
+            raw = mean
+        else:
+            raw = mean + self.std() * torch.randn(mean.shape, device=mean.device, dtype=mean.dtype, generator=generator)
+        logp = self.log_prob(mean, raw)
+        clipped = raw.clamp(-1.0, 1.0).view(*mean.shape[:-1], self.n_warehouses, self.action_dim)
+        if return_raw:
+            return clipped, raw, logp, self.value(obs), mean
+        return clipped, logp, self.value(obs)
+
+    # the diagonal Gaussian over the joint action: the same functions as ActorCritic's single shared policy
+    clamped_log_std = ActorCritic.clamped_log_std
+    std = ActorCritic.std
+    log_prob = ActorCritic.log_prob
+    entropy = ActorCritic.entropy
+
+
 def env_meta_from_algorithm_config(algo_config) -> dict:
     """The ``env_meta`` keys the reference's algorithm wrappers derive from the algorithm config
-    (ippo.py:68-73, 121-142): parameter sharing switches the one-hot warehouse id on."""
+    (ippo.py:68-73, 121-142): parameter sharing switches the one-hot warehouse id on. CPPO has no parameter sharing, so
+    no warehouse id."""
     sp = algo_config.algorithm_specific
     meta = {"obs_normalization": getattr(sp, "obs_normalization", "off")}
     if getattr(sp, "parameter_sharing", False):

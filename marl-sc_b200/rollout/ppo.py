@@ -9,14 +9,14 @@ num_minibatches``, ``shuffle_batch_per_epoch=True``, ``use_kl_loss``, ``grad_cli
 ippo.py:106-115, hysteretic weighting src/algorithms/learners/hysteretic_learner.py:39-42."""
 from __future__ import annotations
 
-from typing import Dict, List, Optional
+from typing import Dict, List, Optional, Union
 
 import torch
 import torch.distributed as dist
 
 from .. import _capi
 from .collector import Rollout
-from .policy import ActorCritic
+from .policy import ActorCritic, CentralizedActorCritic
 
 
 class _FusedPPOObjective(torch.autograd.Function):
@@ -142,7 +142,7 @@ class GradBuckets:
 
 
 class PPOLearner:
-    def __init__(self, policy: ActorCritic, lr: float = 5e-4, clip_param: float = 0.2, vf_clip_param: float = 10.0,
+    def __init__(self, policy: Union[ActorCritic, CentralizedActorCritic], lr: float = 5e-4, clip_param: float = 0.2, vf_clip_param: float = 10.0,
                  vf_loss_coeff: float = 1.0, entropy_coeff: float = 0.01, grad_clip: Optional[float] = None,
                  hysteretic_beta: Optional[float] = None, fused_loss: Optional[bool] = None, use_kl_loss: bool = False,
                  kl_coeff: float = 0.2, kl_target: float = 0.01, num_epochs: int = 1, num_minibatches: int = 1,
@@ -150,6 +150,10 @@ class PPOLearner:
         self.policy = policy
         # K6 on CUDA parameters unless asked otherwise; loss_reference() keeps the plain PyTorch form
         self.fused = next(policy.parameters()).is_cuda if fused_loss is None else bool(fused_loss)
+        if self.fused and policy.log_std.shape[-1] > 512:
+            # a centralised policy's joint action (W*S) can outgrow K6's shared-memory tables
+            raise ValueError(f"the fused PPO loss (K6) takes at most 512 action dimensions per policy, this policy has "
+                             f"{policy.log_std.shape[-1]}: pass fused_loss=False for the PyTorch objective")
         self.opt = torch.optim.Adam(policy.parameters(), lr=lr)
         self.clip, self.vf_clip, self.vf_coeff, self.ent_coeff = clip_param, vf_clip_param, vf_loss_coeff, entropy_coeff
         self.grad_clip, self.beta = grad_clip, hysteretic_beta
@@ -163,7 +167,7 @@ class PPOLearner:
         self.gen.manual_seed(seed)
 
     @classmethod
-    def from_algorithm_config(cls, policy: ActorCritic, algo_config, **kw) -> "PPOLearner":
+    def from_algorithm_config(cls, policy: Union[ActorCritic, CentralizedActorCritic], algo_config, **kw) -> "PPOLearner":
         sp, sh = algo_config.algorithm_specific, algo_config.shared
         lr = sh.learning_rate if isinstance(sh.learning_rate, (int, float)) else sh.learning_rate[0][1]
         return cls(policy, lr=lr, clip_param=sp.clip_param, vf_clip_param=sp.vf_clip_param, vf_loss_coeff=sp.vf_loss_coeff,
