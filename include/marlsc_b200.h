@@ -228,22 +228,24 @@ int32_t marlsc_env_team_size(const marlsc_env_t* env);
 /* The library holds a lean and a generic instantiation of the step kernel and picks the lean one when
  * the configuration allows it; on != 0 forces the generic one (used by the parity tests). */
 int marlsc_env_set_generic(marlsc_env_t* env, int32_t on);
-/* Lean launches of teams of 8+ lanes run the step as four kernels (place / allocate / features / rewards, see
- * csrc/env_split.cuh); on != 0 keeps them in the single fused kernel (used for comparisons and by the tests). */
+/* WIDE only. Lean launches of teams of 8+ lanes run the step as four kernels (place / allocate / features /
+ * rewards, see csrc/env_split.cuh); on != 0 keeps them in the single fused kernel (used for comparisons and by the
+ * tests). A COMPACT handle has one step: there on != 0 returns MARLSC_EUNSUPPORTED (force MARLSC_LAYOUT_WIDE first)
+ * and on == 0 is accepted. */
 int marlsc_env_set_fused(marlsc_env_t* env, int32_t on);
 /* State layout of this handle (MARLSC_LAYOUT_*): COMPACT when the configuration qualifies, else WIDE. */
 int32_t marlsc_env_layout(const marlsc_env_t* env);
 /* Force a layout before the state is allocated / first reset: MARLSC_LAYOUT_WIDE is always possible (needed for the
- * diagnostic outputs, explicit team sizes and the generic / fused test switches); MARLSC_LAYOUT_COMPACT fails with
- * MARLSC_EUNSUPPORTED when the configuration does not qualify. */
+ * diagnostic outputs, explicit team sizes and the generic / fused test switches, which are WIDE only);
+ * MARLSC_LAYOUT_COMPACT fails with MARLSC_EUNSUPPORTED when the configuration does not qualify. */
 int marlsc_env_set_layout(marlsc_env_t* env, int32_t layout);
 /* Rounds per environment of the library-owned line buffer a COMPACT handle converts dense orders into (default 128;
  * a stream that needs more sets an overflow flag that fails the NEXT call on the handle). */
 int marlsc_env_set_line_stride(marlsc_env_t* env, int32_t rounds);
 /* Measurement aid: with on != 0 every marlsc_env_step records CUDA events on its stream around each kernel it
  * launches. marlsc_env_last_timing waits for the last timed step and writes the per-launch durations in
- * milliseconds (split step: place, allocate, features, rewards; fused step: one entry); returns how many, or a
- * negative error code. */
+ * milliseconds (split step: place, allocate, features, rewards; WIDE fused step: one entry); returns how many, or a
+ * negative error code. A COMPACT step is timed when it is given lines (marlsc_step_io.lines), not with dense orders. */
 int marlsc_env_set_timing(marlsc_env_t* env, int32_t on);
 int marlsc_env_last_timing(marlsc_env_t* env, float* ms, int32_t capacity);
 
@@ -317,8 +319,7 @@ typedef struct marlsc_episode_metrics {
  * or m == NULL to stop accumulating. While set, marlsc_env_reset zeroes them on its stream (cudaMemsetAsync) and every
  * step the handle runs (marlsc_env_step, marlsc_env_step_host, marlsc_env_rollout_host) adds to them, for the
  * num_envs of the state it is given. Observations, rewards and state are the same as without metrics.
- *   COMPACT: the split step's kernels accumulate as they go, plus one small launch that adds the rewards. The fused
- *            kernel (marlsc_env_set_fused) has no metrics: the combination is MARLSC_EUNSUPPORTED.
+ *   COMPACT: the step's kernels accumulate as they go, plus one small launch that adds the rewards.
  *   WIDE:    the step's diagnostic outputs are folded into the accumulators by one extra launch, so marlsc_step_io must
  *            carry cost_breakdown, d_ordered, d_ship and d_unfulfilled (else MARLSC_EINVAL); that selects the generic
  *            step kernel. d_ship and d_unfulfilled accumulate, so the caller zeroes them before every step, which

@@ -1,6 +1,5 @@
 // env_alloc.cu - launcher of the one-warp allocation kernel of the split step (env_alloc.cuh).
 #include <atomic>
-#include <cstdlib>
 
 #include "env_alloc.cuh"
 
@@ -51,9 +50,7 @@ int launch_t(const LaunchArgs& a, const marlsc_step_io_t& io, double* cost_alloc
 }  // namespace
 
 int launch_alloc_warp(int spl, const LaunchArgs& a, const marlsc_step_io_t& io, double* cost_alloc, int t, cudaStream_t s, bool prepare_only) {
-  // MARLSC_ALLOC_CHUNKED=1 keeps the chunked allocate_orders kernel (A/B comparisons only)
-  static const bool chunked = std::getenv("MARLSC_ALLOC_CHUNKED") != nullptr;
-  if (chunked || io.order_qty_bytes != 1) return 0;
+  if (io.order_qty_bytes != 1) return 0;
   switch (spl) {
     case 1: return launch_t<1>(a, io, cost_alloc, t, s, prepare_only);
     case 4: return launch_t<4>(a, io, cost_alloc, t, s, prepare_only);

@@ -1,5 +1,5 @@
-// env_compact.cu - fused environment step, reset, base-stock policy and order -> line conversion over the compact
-// state layout (see env_compact.cuh for the design notes).
+// env_compact.cu - environment step (K1a' place, K1b' allocate, K1c' features, K1d rewards), reset, base-stock policy
+// and order -> line conversion over the compact state layout (see env_compact.cuh for the design notes).
 //
 // Reference semantics restated here (paths under the reference repo):
 //   step order ................. src/environment/envs/multi_env.py:253-366
@@ -17,13 +17,10 @@
 #define MARLSC_ALLOC_CTAS 4
 #endif
 namespace marlsc {
-static inline int imin_host(int a, int b) { return a < b ? a : b; }
-static inline int imax_host(int a, int b) { return a > b ? a : b; }
 namespace {
 
 constexpr unsigned FULL = 0xffffffffu;
 constexpr int kSlots = kCompactMaxS / 32;   // SKU slots per lane
-constexpr int kPlaneBatch = 9;              // ring planes of a row in flight per lane (times kSlots cells)
 
 __device__ __forceinline__ uint32_t sm_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ uint32_t ld_s_u8(uint32_t a) { uint32_t v; asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
@@ -40,8 +37,6 @@ __device__ __forceinline__ void red_s_add_f64(uint32_t a, double v) {   // share
   } while (old != seen);
 }
 __device__ __forceinline__ void red_g_add(uint32_t* p, uint32_t v) { asm volatile("red.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
-__device__ __forceinline__ uint32_t ld_nc_u16(const uint16_t* p) { uint32_t v; asm volatile("ld.global.nc.u16 %0, [%1];" : "=r"(v) : "l"(p)); return v; }
-__device__ __forceinline__ uint32_t ld_cg_u16(const uint16_t* p) { uint32_t v; asm volatile("ld.global.cg.u16 %0, [%1];" : "=r"(v) : "l"(p)); return v; }
 __device__ __forceinline__ void prefetch_l2_bulk(const void* p, uint32_t bytes) {
   asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
 }
@@ -194,349 +189,17 @@ __device__ __forceinline__ float nrm(float x, const float* __restrict__ mean, co
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// K1 (compact): one warp per environment; in the allocation a lane owns the SKUs its stream's map word names. The row loops walk pointers (one add per row or
-// plane, cells at constant offsets): the first version of this kernel spent 80 % of its 39 k warp instructions per
-// env-step on index arithmetic.
+// The step as three row / environment kernels and the reward kernel (K1a' .. K1d), cut along the data dependencies: the
+// two streaming parts run as short-lived warps, one per (environment, warehouse) row with every load of the row in flight
+// at once, and only the allocation keeps an environment's stock in shared memory. The same step as one fused kernel kept
+// the stock there from the first row to the last, which held it to 32 warps per SM, and at that residency every one of
+// its ~30 dependent memory round trips per env-step showed (ncu: 13 warps per issue slot waiting on the long scoreboard,
+// 35-40 % issue utilisation, 25-30 % of DRAM bandwidth; 2.7 to 3.9 ms per step at 65,536 large environments against
+// 1.73 ms split, DESIGN.md section 4).
 // ---------------------------------------------------------------------------------------------------------------
+
 // SKU slot k of a lane is valid: always below FS (= S / 32, compile time), for lanes below the remainder at FS, never above
 #define VALID(k) ((k) < FS || ((k) == FS && tail))
-
-template <int NCH, bool MS, int FS>
-__global__ void __launch_bounds__(kCompactWarps * 32, 4)
-env_step_compact_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__ marlsc_env_state_t st,
-                        const __grid_constant__ marlsc_step_io_t io, int t, int prefetch) {
-  extern __shared__ __align__(16) unsigned char smem[];
-  __shared__ int s_poff[kCompactMaxL];                // 32-bit word offset of pipeline slot k's plane inside a warehouse row of the ring
-  const int W = sp.W, S = sp.S, R = sp.R, L = sp.L, WS = W * S;
-  const CompactSmem lay = compact_smem(W, S, R, NCH, sp.pen_uniform);
-  if (threadIdx.x < kCompactMaxL) s_poff[threadIdx.x] = (int)((unsigned)(t + 1 + threadIdx.x) % (unsigned)L) * (S >> 2);
-  {  // per-CTA tables: availability -> priority-order permutation, priority rows, home warehouse of a region
-    const int n_perm = (R * NCH * 32) >> 1, n_prio = (R * 16) >> 2, n_home = (R + 3) >> 2;
-    for (int i = threadIdx.x; i < n_perm + n_prio + n_home; i += blockDim.x) {
-      if (i < n_perm) reinterpret_cast<uint32_t*>(smem + lay.t_perm)[i] = reinterpret_cast<const uint32_t*>(sp.perm5)[i];
-      else if (i < n_perm + n_prio) reinterpret_cast<uint32_t*>(smem + lay.t_prio)[i - n_perm] = reinterpret_cast<const uint32_t*>(sp.prio16)[i - n_perm];
-      else reinterpret_cast<uint32_t*>(smem + lay.t_home)[i - n_perm - n_prio] = reinterpret_cast<const uint32_t*>(sp.home_wh)[i - n_perm - n_prio];
-    }
-  }
-  __syncthreads();
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  const int64_t e = (int64_t)blockIdx.x * kCompactWarps + wid;
-  if (e >= st.num_envs) return;                       // whole warps leave together; everything below is warp-local
-
-  // this environment's lines: read first, everything the allocation loads hangs on these two values
-  const int64_t round0 = io.line_counts ? e * (int64_t)io.line_stride : (int64_t)io.line_offsets[e];
-  const int n_rounds = io.line_counts ? io.line_counts[e] : io.line_offsets[e + 1] - (int)round0;
-  if (lane == 0 && n_rounds > 0) prefetch_l2_bulk(io.lines + round0 * 32, (uint32_t)n_rounds * 64u);   // in flight during phase 1
-  // ... and this environment's state blocks on their way into L2 (one bulk prefetch each, no registers or shared
-  // memory held): the row loops below then wait for L2, not DRAM
-  if (prefetch) {
-    if (lane == 1) prefetch_l2_bulk(static_cast<const uint8_t*>(st.ring_qty) + e * (int64_t)WS * L, (uint32_t)(WS * L));
-    if (lane == 2 && !io.action_qty) prefetch_l2_bulk(io.actions + e * WS, (uint32_t)(WS * 4));
-    if (lane == 3) prefetch_l2_bulk(static_cast<const uint16_t*>(st.inventory) + e * WS, (uint32_t)(WS * 2));
-    if (lane == 4 && io.action_qty) prefetch_l2_bulk(io.action_qty + e * WS, (uint32_t)WS);
-  }
-
-  unsigned char* const wbase = smem + lay.t_bytes + (size_t)wid * lay.warp_bytes;
-  uint16_t* const s_inv = reinterpret_cast<uint16_t*>(wbase + lay.inv);
-  uint32_t* const s_shipq = reinterpret_cast<uint32_t*>(wbase + lay.shipq);
-  uint32_t* const s_lostU = reinterpret_cast<uint32_t*>(wbase + lay.lostU);
-  double* const s_lostP = reinterpret_cast<double*>(wbase + lay.lostP);
-  const bool pen_uniform = sp.pen_uniform != 0;
-  for (int i = lane; i < W * R; i += 32) s_shipq[i] = 0u;
-  for (int i = lane; i < R; i += 32) {
-    s_lostU[i] = 0u;
-    if (!pen_uniform) s_lostP[i] = 0.0;
-  }
-
-  const bool need_hist = sp.need_hist != 0;
-  const int pa = t % L;                               // plane of the orders arriving now
-  const bool by_row = sp.row_rates_uniform != 0;
-  const bool tail = lane < S - 32 * FS;               // this lane owns a SKU in the partly filled slot FS
-  // per-lane bases (this lane's first cell); rows advance them by their strides
-  uint16_t* const g_inv = pinned(static_cast<uint16_t*>(st.inventory) + e * WS + lane);
-  uint8_t* const g_ring = pinned(static_cast<uint8_t*>(st.ring_qty) + e * (int64_t)WS * L + lane);
-  uint16_t* const g_hist = need_hist ? pinned(static_cast<uint16_t*>(st.demand_hist) + e * (int64_t)kWindow * WS + lane) : nullptr;
-  uint16_t* const hist_now = need_hist ? g_hist + (t % kWindow) * WS : nullptr;
-  float* const g_obs = pinned(io.obs + e * (int64_t)W * sp.obs_dim + sp.id_off + lane);
-  const float* const mean_l = MS ? sp.obs_mean + lane : nullptr;
-  const float* const istd_l = MS ? sp.obs_std + lane : nullptr;
-  const int obs_dim = sp.obs_dim, off_pipe = sp.off_pipe, LS = L * S;
-
-  // ---- phase 1: per warehouse row - orders in, arrivals in (multi_env.py:287-292), pipeline block of the observation
-  // (multi_env.py:941-968). In this phase lane q owns the four CONSECUTIVE SKUs 4q .. 4q+3 of a row, so a row's cells
-  // and ring planes arrive as a handful of vector loads (one 32-bit load per plane: the nine planes of a row in flight
-  // cost nine registers; byte loads by strided lanes cost 36 and were what kept this kernel waiting on memory).
-  // Slot k of the pipeline block is plane (t + 1 + k) % L for every cell. Slots 0 .. L-2 are the planes after the
-  // arrival plane, copied as they stand - four shuffles per plane turn the lane-contiguous bytes into 128-byte
-  // coalesced float stores; this step only adds the order a cell places now, which lands in slot lead-1 (the byte there
-  // is 0: the plane was cleared when it last arrived, and only this cell's order of exactly that lead writes it) and is
-  // patched into the row right after the copy, while its sectors are still in L2 (patching a whole phase later made L2
-  // re-fetch every patched sector: +37 KB of DRAM traffic per env-step). Slot L-1 is the arrival plane itself, which
-  // after this step only holds the new orders of lead L.
-  int rowQ = 0, rowPos = 0;                           // lane w keeps row w's ordered units / ordered cells
-  double rowInb = 0.0;                                // ... or its inbound cost when the rates vary over the row
-  {
-    const bool mine = 4 * lane < S;                   // S % 4 == 0: a lane's four cells exist together
-    const int c4 = mine ? lane : 0;
-    const float4* __restrict__ act4 = io.action_qty ? nullptr : reinterpret_cast<const float4*>(io.actions + e * WS) + c4;
-    const uint32_t* __restrict__ aq4 = io.action_qty ? reinterpret_cast<const uint32_t*>(io.action_qty + e * WS) + c4 : nullptr;
-    const uint32_t* __restrict__ lead4 = reinterpret_cast<const uint32_t*>(sp.lead_u8) + c4;
-    uint2* inv4 = reinterpret_cast<uint2*>(static_cast<uint16_t*>(st.inventory) + e * WS) + c4;
-    uint32_t* row4 = reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(st.ring_qty) + e * (int64_t)WS * L) + c4;
-    uint2* hz4 = need_hist ? reinterpret_cast<uint2*>(hist_now - lane) + c4 : nullptr;
-    float* __restrict__ out = g_obs + off_pipe;       // lane l's element of a 32-wide store group
-    float* __restrict__ outc = g_obs - lane + off_pipe + 4 * c4;   // this lane's own four cells
-    uint32_t a_sinv = sm_addr(s_inv) + 8u * c4;
-    const int S4 = S >> 2, LS4 = LS >> 2, pa4 = pa * S4;
-    int mx[4];                                        // order maxima are whole numbers <= 255 in this layout
-#pragma unroll
-    for (int j = 0; j < 4; ++j) mx[j] = mine ? (int)sp.action_max[4 * lane + j] : 0;
-    const int sub = lane & 3, src0 = lane >> 2;       // where lane l's element of store group j lives: lane 8j + l/4, byte l%4
-#pragma unroll 1
-    for (int w = 0; w < W; ++w) {
-      // every load of the row first: own cells, then the planes of the first batch
-      float4 a4 = make_float4(0.f, 0.f, 0.f, 0.f);
-      uint32_t aqw = 0u, arr4 = 0u, le4 = 0x01010101u;
-      uint2 iv = make_uint2(0u, 0u);
-      if (mine) {
-        if (aq4) aqw = *aq4; else a4 = *act4;
-        iv = *inv4;
-        arr4 = row4[pa4];
-        le4 = *lead4;
-      }
-      int q[4], le[4];
-      float* dst = out;
-      int moff = off_pipe;
-#pragma unroll 1
-      for (int k0 = 0; k0 < L; k0 += kPlaneBatch) {
-        uint32_t x[kPlaneBatch];
-#pragma unroll
-        for (int kk = 0; kk < kPlaneBatch; ++kk) {
-          const bool live = k0 + kk < L - 1;
-          x[kk] = (mine && live) ? row4[s_poff[live ? k0 + kk : 0]] : 0u;
-        }
-        if (k0 == 0) {                                // the row's own cells: order quantity, stock, ring, history plane
-          const float af[4] = {a4.x, a4.y, a4.z, a4.w};
-          const uint32_t ivv[4] = {iv.x & 0xffffu, iv.x >> 16, iv.y & 0xffffu, iv.y >> 16};
-          uint32_t ni[4], newarr = 0u;
-          int nQ = 0, nPos = 0;
-          double inb = 0.0;
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            le[j] = (int)((le4 >> (8 * j)) & 0xffu);
-            q[j] = 0;
-            if (mine) q[j] = aq4 ? imin((int)((aqw >> (8 * j)) & 0xffu), mx[j]) : rescale_action<kCapsLean>(sp, af[j], (double)mx[j], 0, 0);
-            ni[j] = ivv[j] + ((arr4 >> (8 * j)) & 0xffu);
-            if (le[j] == L) newarr |= (uint32_t)q[j] << (8 * j);
-            nQ += q[j];
-            nPos += q[j] > 0 ? 1 : 0;
-            if (!by_row && q[j] > 0) {
-              const int i = w * S + 4 * lane + j;
-              inb += sp.in_fixed[i] + ((double)q[j] * sp.skw[4 * lane + j]) * sp.in_var[i];
-            }
-          }
-          if (mine) {
-            asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(a_sinv), "r"(ni[0] | (ni[1] << 16)), "r"(ni[2] | (ni[3] << 16)) : "memory");
-            row4[pa4] = newarr;                       // arrivals consumed, lead-L orders in
-            uint8_t* rowb = reinterpret_cast<uint8_t*>(row4);
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-              if (q[j] > 0 && le[j] < L) {
-                int p2 = pa + le[j];
-                p2 -= p2 >= L ? L : 0;
-                rowb[p2 * S + j] = (uint8_t)q[j];
-              }
-            if (need_hist) *hz4 = make_uint2(0u, 0u);
-          }
-          if (by_row) {
-            nQ = __reduce_add_sync(FULL, nQ);
-            nPos = __reduce_add_sync(FULL, nPos);
-            if (lane == w) {
-              rowQ = nQ;
-              rowPos = nPos;
-            }
-          } else {
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) inb += __shfl_xor_sync(FULL, inb, o);
-            if (lane == w) rowInb = inb;
-          }
-        }
-#pragma unroll
-        for (int kk = 0; kk < kPlaneBatch; ++kk) {
-          if (k0 + kk < L) {                          // slot L-1 (x == 0): the arrival plane
-#pragma unroll
-            for (int j = 0; j < kSlots; ++j) {
-              const uint32_t v = __shfl_sync(FULL, x[kk], 8 * j + src0);
-              if (VALID(j)) dst[32 * j] = nrm<MS>((float)((v >> (8 * sub)) & 0xffu), mean_l, istd_l, moff + 32 * j);
-            }
-            dst += S;
-            moff += S;
-          }
-        }
-      }
-      if (mine) {
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-          if (q[j] > 0) {                             // the new order's slot of the pipeline block
-            const int po = (le[j] - 1) * S + j;
-            outc[po] = nrm<MS>((float)q[j], mean_l - lane, istd_l - lane, off_pipe + 4 * lane + po);
-          }
-      }
-      if (aq4) aq4 += S4; else act4 += S4;
-      lead4 += S4;
-      inv4 += S4;
-      row4 += LS4;
-      hz4 += S4;
-      out += obs_dim;
-      outc += obs_dim;
-      a_sinv += 2u * S;
-    }
-  }
-  __syncwarp();                                       // stock staged, history plane cleared
-
-  // ---- phase 2: greedy allocation of this step's lines (demand_allocator.py:150-208) -----------------------------
-  {
-    LineStream ls;
-    ls.init(io.lines, round0, n_rounds, lane);
-    uint32_t avlo, avhi;
-    owner_masks(ls.map, sm_addr(s_inv), W, S, avlo, avhi);
-    allocation_chains<NCH>(sp, ls, sm_addr(smem + lay.t_perm), sm_addr(smem + lay.t_prio), sm_addr(smem + lay.t_home),
-                           sm_addr(s_inv), sm_addr(s_shipq), sm_addr(s_lostU), sm_addr(s_lostP), avlo, avhi,
-                           need_hist ? reinterpret_cast<uint32_t*>(hist_now - lane) : nullptr);
-  }
-  __syncwarp();
-
-  // Outbound cost and lost-sales penalty of every warehouse (reward_calculator.py:134-142). Lanes take regions (two per
-  // lane cover R <= 64). Per region the lost volume's cost is either spread over the warehouses in proportion to what
-  // they shipped there (shipment handler, lost_sales_handler.py:113-148: a rate per shipped unit, one division per
-  // region) or goes to the closest warehouse (closest handler, and the shipment handler's fallback when nothing was
-  // shipped). Then warehouse by warehouse the lanes' partial sums meet in a shuffle reduction; lane w keeps row w's.
-  double costA = 0.0;
-  {
-    const double pen0 = sp.pen_rate[0];
-    double rate[2], lump[2];
-    int close_w[2];
-#pragma unroll
-    for (int qq = 0; qq < 2; ++qq) {
-      const int r = lane + 32 * qq;
-      rate[qq] = lump[qq] = 0.0;
-      close_w[qq] = -1;
-      if (r < R) {
-        const uint32_t lu = s_lostU[r];
-        if (lu > 0u) {
-          const double lpn = pen_uniform ? (double)lu * pen0 : s_lostP[r];
-          uint32_t shipped_r = 0u;
-          if (sp.lost_type == MARLSC_LOST_SHIPMENT)
-            for (int w = 0; w < W; ++w) shipped_r += s_shipq[w * R + r];
-          if (shipped_r > 0u) {
-            rate[qq] = lpn / (double)shipped_r;
-          } else {
-            lump[qq] = lpn;
-            close_w[qq] = sp.closest[r];
-          }
-        }
-      }
-    }
-    for (int w = 0; w < W; ++w) {
-      double c = 0.0;
-#pragma unroll
-      for (int qq = 0; qq < 2; ++qq) {
-        const int r = lane + 32 * qq;
-        if (r < R) {
-          const uint32_t sq = s_shipq[w * R + r];
-          if (sq > 0u) c += (double)sq * (sp.out_var[w * R + r] + rate[qq]);
-          if (close_w[qq] == w) c += lump[qq];
-        }
-      }
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(FULL, c, o);
-      if (lane == w) costA = c;
-    }
-  }
-
-  // ---- phase 3: per warehouse row - stock out, rolling mean, the remaining observation blocks, holding cost ------
-  const int hist_n = imin(t + 1, kWindow);
-  double costR = 0.0;
-  {
-    // mean over the window = integer sum / n, rounded to float32 like NumPy's (multi_env.py:785-787): the product with
-    // the double reciprocal is within 2^-52 of the quotient, far from every float32 rounding boundary of a quotient
-    // of integers below 2^24 by n <= 5, so rounding it gives the correctly rounded float32 quotient
-    const double rcp_n = 1.0 / (double)hist_n;
-    uint32_t a_sinv = sm_addr(s_inv) + 2u * lane;
-    uint16_t* inv = g_inv;
-    const uint16_t* hnow = hist_now;
-    const uint16_t* hold_p[kWindow - 1];
-#pragma unroll
-    for (int back = 1; back < kWindow; ++back) hold_p[back - 1] = need_hist ? g_hist + pmod(t - back, kWindow) * WS : nullptr;
-    float* out = g_obs;
-    const int off_inv = sp.off_inv, off_dh = sp.off_dh, off_rm = sp.off_rm;
-    const bool inv_agg = (sp.feat & MARLSC_F_INVENTORY_AGG) != 0;
-#pragma unroll 1
-    for (int w = 0; w < W; ++w) {
-      int vI[kSlots], vdh[kSlots], hv[kSlots][kWindow - 1];
-#pragma unroll
-      for (int k = 0; k < kSlots; ++k) {              // loads first
-        vI[k] = VALID(k) ? (int)ld_s_u16(a_sinv + 64u * k) : 0;
-        vdh[k] = VALID(k) && need_hist ? (int)ld_cg_u16(hnow + 32 * k) : 0;   // accumulated with fire-and-forget adds above
-#pragma unroll
-        for (int back = 1; back < kWindow; ++back)
-          hv[k][back - 1] = VALID(k) && need_hist && back < hist_n ? (int)hold_p[back - 1][32 * k] : 0;
-      }
-      int nI = 0;
-      double hold = 0.0;
-#pragma unroll
-      for (int k = 0; k < kSlots; ++k)
-        if (VALID(k)) {
-          inv[32 * k] = (uint16_t)vI[k];              // multi_env.py:307 (never negative)
-          nI += vI[k];
-          if (!by_row) hold += (double)vI[k] * sp.hold_rate[lane + 32 * k];
-          out[off_inv + 32 * k] = nrm<MS>((float)vI[k], mean_l, istd_l, off_inv + 32 * k);
-          if (off_dh >= 0) out[off_dh + 32 * k] = nrm<MS>((float)vdh[k], mean_l, istd_l, off_dh + 32 * k);
-          if (off_rm >= 0) {
-            const int hsum = (hv[k][0] + hv[k][1]) + (hv[k][2] + hv[k][3]) + vdh[k];
-            out[off_rm + 32 * k] = nrm<MS>((float)((double)hsum * rcp_n), mean_l, istd_l, off_rm + 32 * k);
-          }
-        }
-      nI = __reduce_add_sync(FULL, nI);
-      if (lane == 0 && inv_agg) out[off_inv + S] = nrm<MS>((float)nI, mean_l, istd_l, off_inv + S);
-      if (sp.id_off && lane < W) out[-sp.id_off] = lane == w ? 1.0f : 0.0f;   // obs_w[lane]: out already points at element id_off + lane
-      if (by_row) {
-        if (lane == w) {
-          const int base = w * S;
-          costR = (double)nI * sp.hold_rate[0] + ((double)rowPos * sp.in_fixed[base] + ((double)rowQ * sp.skw[0]) * sp.in_var[base]);
-        }
-      } else {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) hold += __shfl_xor_sync(FULL, hold, o);
-        if (lane == w) costR = hold + rowInb;
-      }
-      a_sinv += 2u * S;
-      inv += S;
-      hnow += S;
-#pragma unroll
-      for (int back = 1; back < kWindow; ++back) hold_p[back - 1] += S;
-      out += obs_dim;
-    }
-  }
-
-  // ---- rewards (multi_env.py:316-327) ----------------------------------------------------------------------------
-  double rew = lane < W ? -((costR + costA) * sp.scale) : 0.0;
-  if (sp.scope == MARLSC_SCOPE_TEAM) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) rew += __shfl_xor_sync(FULL, rew, o);
-  }
-  if (lane < W) io.rewards[e * W + lane] = (float)rew;
-  if (io.truncated && lane == 0) io.truncated[e] = (uint8_t)(t + 1 >= sp.episode_length);
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// The same step as three row / environment kernels + the reward kernel (K1a' .. K1d). The fused kernel above keeps an
-// environment's stock in shared memory from the first row to the last, which holds it to 32 warps per SM, and at that
-// residency every one of its ~30 dependent memory round trips per env-step shows (ncu: 13 warps per issue slot waiting on
-// the long scoreboard, 35-40 % issue utilisation, 25-30 % of DRAM bandwidth). Cut along the data dependencies, the two
-// streaming parts run as short-lived warps, one per (environment, warehouse) row with every load of the row in flight at
-// once, and only the allocation keeps the shared-memory scratch.
-// ---------------------------------------------------------------------------------------------------------------
 
 // K1a': one warp per (environment, warehouse) row - order quantities, arrivals, the row of the ring rewritten with the
 // new orders in, history plane cleared, pipeline block of the observation row; the row's inbound cost goes to cost_rows.
@@ -765,7 +428,11 @@ compact_alloc_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
 #pragma unroll
     for (int k = 0; k < kSlots; ++k)
       if (VALID(k)) g_inv[w0 * S + 32 * k] = s_inv[w0 * S + lane + 32 * k];
-  // outbound cost and lost-sales penalty per warehouse (see the fused kernel)
+  // Outbound cost and lost-sales penalty of every warehouse (reward_calculator.py:134-142). Lanes take regions (two per
+  // lane cover R <= 64). Per region the lost volume's cost is either spread over the warehouses in proportion to what
+  // they shipped there (shipment handler, lost_sales_handler.py:113-148: a rate per shipped unit, one division per
+  // region) or goes to the closest warehouse (closest handler, and the shipment handler's fallback when nothing was
+  // shipped). Then warehouse by warehouse the lanes' partial sums meet in a shuffle reduction.
   const double pen0 = sp.pen_rate[0];
   double rate[2], lump[2];
   int close_w[2];
@@ -902,7 +569,10 @@ compact_feature_kernel(const __grid_constant__ DevSpec sp, const __grid_constant
     }
   }
   float* const img = reinterpret_cast<float*>(smem) + (threadIdx.x >> 5) * (3 * S);
-  const double rcp_n = 1.0 / (double)hist_n;          // see the fused kernel: rounds to the correctly rounded float32 quotient
+  // mean over the window = integer sum / n, rounded to float32 like NumPy's (multi_env.py:785-787): the product with the
+  // double reciprocal is within 2^-52 of the quotient, far from every float32 rounding boundary of a quotient of integers
+  // below 2^24 by n <= 5, so rounding it gives the correctly rounded float32 quotient
+  const double rcp_n = 1.0 / (double)hist_n;
   const bool by_row = sp.row_rates_uniform != 0;
   int nI = 0;
   double hold = 0.0;
@@ -969,151 +639,6 @@ compact_feature_kernel(const __grid_constant__ DevSpec sp, const __grid_constant
 #pragma unroll
     for (int k = 0; k < kSlots; ++k)                  // S <= 32 kSlots: four predicated stores, no loop scaffolding
       if (32 * k + lane < S) out[offs[b] + 32 * k] = nrm<MS>(src[32 * k], mean_l, istd_l, 32 * k);
-  }
-}
-
-// K1c' with the bulk-copy engine (opt-in: MARLSC_FEATURE_BULK=1; measured slower, see below): persistent CTAs, one warp
-// per warehouse row. A single thread asks the copy engine for an environment's stock block ([W,S] uint16) and its five
-// history planes ([5,W,S] uint16, contiguous) - two cp.async.bulk requests (SASS UBLKCP.S.G), 12 W S bytes, completion
-// counted on an mbarrier - a few environments ahead of the one the warps are reading out of shared memory; a second set
-// of mbarriers hands the stages back, so no warp waits for another. The blocks are 16-byte granular when W S is a
-// multiple of 8 (the launcher checks). Same arithmetic as above, bit-identical results (the parity tests run both).
-// Measured at 65,536 large environments (one B200): 0.37 ms with four stages and a CTA barrier per environment,
-// 0.48-0.55 ms in this form, against 0.34 ms for the register version above; the copy pipeline alone (no read-out) runs
-// in 0.15 ms, the read-out without its observation stores adds 0.16 ms and the stores another 0.17 ms - the three do
-// not overlap the way the 40 independent short-lived warps per SM of the register version do, so that one stays.
-constexpr int kFeatStages = 5;
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_load(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src), "r"(bytes),
-               "r"(bar)
-               : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done;
-  asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.b32 %0, 1, 0, p;\n\t}"
-               : "=r"(done)
-               : "r"(bar), "r"(parity)
-               : "memory");
-  return done != 0u;
-}
-
-template <bool MS>
-__global__ void __launch_bounds__(512)
-compact_feature_bulk_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__ marlsc_env_state_t st,
-                            const __grid_constant__ marlsc_step_io_t io, double* __restrict__ cost_rows,
-                            const double* __restrict__ cost_alloc, int t, int write_rewards) {
-  extern __shared__ __align__(16) unsigned char smem[];           // kFeatStages x (stock | 5 history planes), then the mbarriers
-  const int W = sp.W, S = sp.S, WS = W * S;
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;         // blockDim.x = 32 W: warp w owns row w
-  const bool need_hist = sp.need_hist != 0;
-  const uint32_t stock_bytes = 2u * (uint32_t)WS, hist_bytes = need_hist ? (uint32_t)kWindow * stock_bytes : 0u;
-  const uint32_t stage_bytes = (1u + (uint32_t)kWindow) * stock_bytes;
-  const uint32_t a_smem = sm_addr(smem), a_full = a_smem + (uint32_t)kFeatStages * stage_bytes, a_empty = a_full + 8u * kFeatStages;
-  if (threadIdx.x == 0) {
-#pragma unroll
-    for (int i = 0; i < kFeatStages; ++i) {
-      mbar_init(a_full + 8u * i, 1u);
-      mbar_init(a_empty + 8u * i, (uint32_t)W);       // one arrival per warp that has read the stage out
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
-  const int64_t n_env = st.num_envs, stride = gridDim.x;
-  const uint16_t* const g_inv = static_cast<const uint16_t*>(st.inventory);
-  const uint16_t* const g_hist = static_cast<const uint16_t*>(st.demand_hist);
-  const auto request = [&](int64_t e, int stage) {    // thread 0: the two blocks of environment e into a stage
-    const uint32_t bar = a_full + 8u * stage, dst = a_smem + (uint32_t)stage * stage_bytes;
-    mbar_expect_tx(bar, stock_bytes + hist_bytes);
-    bulk_load(dst, g_inv + e * WS, stock_bytes, bar);
-    if (need_hist) bulk_load(dst + stock_bytes, g_hist + e * (int64_t)kWindow * WS, hist_bytes, bar);
-  };
-  // Trip i reads stage i % kFeatStages. Thread 0 requests trip i + kFeatStages - 2 at the start of trip i: that stage
-  // was read out in trip i - 2, so the other warps had a whole trip to leave it (no warp waits for another here; the
-  // warps of a CTA drift up to two environments apart).
-  constexpr int kAhead = kFeatStages - 2;
-  if (threadIdx.x == 0)
-    for (int k = 0; k < kAhead; ++k)
-      if (blockIdx.x + k * stride < n_env) request(blockIdx.x + k * stride, k);
-  const int hist_n = imin(t + 1, kWindow);
-  const double rcp_n = 1.0 / (double)hist_n;          // see the fused kernel: rounds to the correctly rounded float32 quotient
-  const bool by_row = sp.row_rates_uniform != 0;
-  const int p_now = t % kWindow;
-  int it = 0;
-  for (int64_t e = blockIdx.x; e < n_env; e += stride, ++it) {
-    const int stage = it % kFeatStages;
-    if (threadIdx.x == 0) {
-      const int64_t e_next = e + (int64_t)kAhead * stride;
-      if (e_next < n_env) {
-        const int st_next = (it + kAhead) % kFeatStages;
-        if (it >= 2) {                                // its previous tenant: trip it - 2
-          const uint32_t par = (uint32_t)((it - 2) / kFeatStages) & 1u;
-          while (!mbar_try_wait(a_empty + 8u * st_next, par)) {}
-        }
-        request(e_next, st_next);
-      }
-    }
-    const int64_t row = e * W + w;
-    double cost_in = 0.0, cost_al = 0.0;              // on their way while the stage lands
-    if (lane == 0) {
-      cost_in = cost_rows[row];
-      if (write_rewards) cost_al = cost_alloc[row];
-    }
-    const uint32_t parity = (uint32_t)(it / kFeatStages) & 1u;
-    while (!mbar_try_wait(a_full + 8u * stage, parity)) {}
-    const uint16_t* const s_inv = reinterpret_cast<const uint16_t*>(smem + (size_t)stage * stage_bytes) + w * S;
-    const uint16_t* const s_hist = s_inv + WS;        // plane p of this row: s_hist + p WS
-    float* const obs_w = io.obs + (size_t)row * sp.obs_dim;
-    float* const out = obs_w + sp.id_off;
-    int nI = 0;
-    double hold = 0.0;
-    for (int i = lane; i < S; i += 32) {
-      const uint32_t v = s_inv[i];
-      nI += (int)v;
-      if (!by_row) hold += (double)v * sp.hold_rate[i];
-      if (sp.off_inv >= 0) out[sp.off_inv + i] = nrm<MS>((float)v, sp.obs_mean, sp.obs_std, sp.off_inv + i);
-      if (need_hist) {
-        const uint32_t d = s_hist[p_now * WS + i];
-        uint32_t hs = d;
-#pragma unroll
-        for (int back = 1; back < kWindow; ++back)
-          if (back < hist_n) hs += s_hist[pmod(t - back, kWindow) * WS + i];
-        if (sp.off_dh >= 0) out[sp.off_dh + i] = nrm<MS>((float)d, sp.obs_mean, sp.obs_std, sp.off_dh + i);
-        if (sp.off_rm >= 0) out[sp.off_rm + i] = nrm<MS>((float)((double)hs * rcp_n), sp.obs_mean, sp.obs_std, sp.off_rm + i);
-      }
-    }
-    nI = __reduce_add_sync(FULL, nI);
-    double cost;
-    if (by_row) {
-      cost = (double)nI * sp.hold_rate[0];
-    } else {
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) hold += __shfl_xor_sync(FULL, hold, o);
-      cost = hold;
-    }
-    __syncwarp();
-    if (lane == 0) {
-      asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(a_empty + 8u * stage) : "memory");   // this warp has left the stage
-      cost += cost_in;                                // + the inbound cost K1a' left there
-      if (write_rewards) {                            // agent scope (multi_env.py:316-327): no reward kernel needed
-        io.rewards[row] = (float)(-((cost + cost_al) * sp.scale));
-        if (io.truncated && w == 0) io.truncated[e] = (uint8_t)(t + 1 >= sp.episode_length);
-      } else {
-        cost_rows[row] = cost;
-      }
-      if (sp.feat & MARLSC_F_INVENTORY_AGG) {
-        float x = (float)nI;
-        if (MS) x = f_mul(f_sub(x, sp.obs_mean[sp.off_inv + S]), sp.obs_std[sp.off_inv + S]);
-        obs_w[sp.id_off + sp.off_inv + S] = x;
-      }
-    }
-    if (sp.id_off && lane < W) obs_w[lane] = lane == w ? 1.0f : 0.0f;
   }
 }
 
@@ -1299,31 +824,6 @@ lines_from_orders_kernel(const __grid_constant__ DevSpec sp, long long E, const 
 }
 
 template <int NCH, bool MS, int FS>
-int launch_step_nch(const LaunchArgs& a, const marlsc_step_io_t& io, int t, cudaStream_t s) {
-  const CompactSmem lay = compact_smem(a.ds.W, a.ds.S, a.ds.R, NCH, a.ds.pen_uniform);
-  const size_t smem = (size_t)lay.t_bytes + (size_t)kCompactWarps * lay.warp_bytes;
-  if ((int)smem > a.max_smem_optin)
-    return set_error(MARLSC_EUNSUPPORTED, "compact step: shared-memory scratch of " + std::to_string(smem) + " bytes per CTA does not fit");
-  static int configured_for[kMaxDevices] = {0};       // per device: the attributes belong to the device's context
-  int dev = 0;
-  MARLSC_CUDA(cudaGetDevice(&dev));
-  if (dev >= kMaxDevices || configured_for[dev] < (int)smem) {
-    MARLSC_CUDA(cudaFuncSetAttribute((const void*)env_step_compact_kernel<NCH, MS, FS>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                     (int)cudaSharedmemCarveoutMaxShared));
-    MARLSC_CUDA(cudaFuncSetAttribute((const void*)env_step_compact_kernel<NCH, MS, FS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (dev < kMaxDevices) configured_for[dev] = (int)smem;
-  }
-  const unsigned grid = (unsigned)((a.st.num_envs + kCompactWarps - 1) / kCompactWarps);
-  // bulk L2 prefetches of an environment's state blocks need 16-byte aligned addresses and sizes
-  const auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
-  const int prefetch = a.ds.compact_prefetch && al16(a.st.ring_qty) && al16(a.st.inventory) && al16(io.actions) && al16(io.action_qty);
-  env_step_compact_kernel<NCH, MS, FS><<<grid, kCompactWarps * 32, smem, s>>>(a.ds, a.st, io, t, prefetch);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  MARLSC_CUDA(cudaGetLastError());
-  return MARLSC_OK;
-}
-
-template <int NCH, bool MS, int FS>
 int launch_split_nch(const LaunchArgs& a, const marlsc_step_io_t& io, const SplitWork& wk, int t, cudaStream_t s) {
   const CompactSmem lay = compact_smem(a.ds.W, a.ds.S, a.ds.R, NCH, a.ds.pen_uniform);
   const size_t smem = (size_t)lay.t_bytes + (size_t)kCompactWarps * lay.warp_bytes;
@@ -1382,23 +882,7 @@ int launch_split_nch(const LaunchArgs& a, const marlsc_step_io_t& io, const Spli
   MARLSC_CUDA(cudaGetLastError());
   if (wk.marks) MARLSC_CUDA(cudaEventRecord(wk.marks[2], s));
   const int agent_scope = a.ds.scope == MARLSC_SCOPE_AGENT;
-  // bulk-copy version when an environment's blocks are 16-byte granular (W S a multiple of 8) and aligned
-  const auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
-  const size_t feat_smem = (size_t)kFeatStages * (1 + kWindow) * 2 * a.ds.W * a.ds.S + 16 * kFeatStages;
-  if (!stats && a.ds.feature_bulk && al16(a.st.inventory) && al16(a.st.demand_hist) && (int)feat_smem <= a.max_smem_optin) {
-    static int feat_configured[kMaxDevices] = {0};
-    int sms = 0;
-    MARLSC_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    if (dev >= kMaxDevices || feat_configured[dev] < (int)feat_smem) {
-      MARLSC_CUDA(cudaFuncSetAttribute((const void*)compact_feature_bulk_kernel<MS>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                       (int)cudaSharedmemCarveoutMaxShared));
-      MARLSC_CUDA(cudaFuncSetAttribute((const void*)compact_feature_bulk_kernel<MS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)feat_smem));
-      if (dev < kMaxDevices) feat_configured[dev] = (int)feat_smem;
-    }
-    const int per_sm = imax_host(1, imin_host((int)(220 * 1024 / feat_smem), 2048 / (32 * a.ds.W)));
-    const unsigned grid_feat = (unsigned)std::min<int64_t>(a.st.num_envs, (int64_t)sms * per_sm);
-    compact_feature_bulk_kernel<MS><<<grid_feat, 32 * a.ds.W, feat_smem, s>>>(a.ds, a.st, io, wk.cost_rows, wk.cost_alloc, t, agent_scope);
-  } else if (stats) {
+  if (stats) {
     compact_feature_kernel<MS, true><<<grid_rows, 256, (size_t)8 * 3 * a.ds.S * sizeof(float), s>>>(a.ds, a.st, io, wk.cost_rows, wk.cost_alloc,
                                                                                                    t, agent_scope, m);
   } else {
@@ -1427,28 +911,7 @@ int launch_split_fs(const LaunchArgs& a, const marlsc_step_io_t& io, const Split
   }
 }
 
-template <int NCH, bool MS>
-int launch_step_fs(const LaunchArgs& a, const marlsc_step_io_t& io, int t, cudaStream_t s) {
-  switch (a.ds.S / 32) {                              // compact layouts have 32 < S <= 128
-    case 1: return launch_step_nch<NCH, MS, 1>(a, io, t, s);
-    case 2: return launch_step_nch<NCH, MS, 2>(a, io, t, s);
-    case 3: return launch_step_nch<NCH, MS, 3>(a, io, t, s);
-    default: return launch_step_nch<NCH, MS, 4>(a, io, t, s);
-  }
-}
-
 }  // namespace
-
-int launch_step_compact(const LaunchArgs& a, const marlsc_step_io_t& io, int t, cudaStream_t s) {
-  const bool ms = a.ds.norm == MARLSC_NORM_MEANSTD;
-  switch (a.ds.perm5_chunks) {
-    case 1: return ms ? launch_step_fs<1, true>(a, io, t, s) : launch_step_fs<1, false>(a, io, t, s);
-    case 2: return ms ? launch_step_fs<2, true>(a, io, t, s) : launch_step_fs<2, false>(a, io, t, s);
-    case 3: return ms ? launch_step_fs<3, true>(a, io, t, s) : launch_step_fs<3, false>(a, io, t, s);
-    case 4: return ms ? launch_step_fs<4, true>(a, io, t, s) : launch_step_fs<4, false>(a, io, t, s);
-    default: return set_error(MARLSC_EUNSUPPORTED, "compact step needs W <= 16");
-  }
-}
 
 int launch_split_compact(const LaunchArgs& a, const marlsc_step_io_t& io, const SplitWork& wk, int t, cudaStream_t s) {
   const bool ms = a.ds.norm == MARLSC_NORM_MEANSTD;

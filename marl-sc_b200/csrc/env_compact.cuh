@@ -1,9 +1,11 @@
-// env_compact.cuh - the environment step of the common configurations as ONE fused kernel over the compact state
-// layout (MARLSC_LAYOUT_COMPACT): a warp advances one environment by one timestep.
+// env_compact.cuh - the environment step of the common configurations over the compact state layout
+// (MARLSC_LAYOUT_COMPACT), in env_compact.cu: K1a' places the orders and writes the pipeline block with one warp per
+// (environment, warehouse) row, K1b' allocates the step's demand with one warp per environment, K1c' writes the remaining
+// observation blocks and row costs with one warp per row, and K1d sums team rewards.
 //
-// What changed against the split step (env_split.cuh) and why (ncu, profiles/r1_k1_split_65536envs.summary.txt: the three
-// kernels issued 27 k warp instructions per env-step - 70 % of the row kernels' were address arithmetic of the per-cell
-// ring gather - and moved 154 KB per env-step, 44 KB of it the int32 ring):
+// What changed against the WIDE layout's split step (env_split.cuh) and why (ncu, profiles/r1_k1_split_65536envs.summary.txt:
+// the three kernels issued 27 k warp instructions per env-step - 70 % of the row kernels' were address arithmetic of the
+// per-cell ring gather - and moved 154 KB per env-step, 44 KB of it the int32 ring):
 //
 //   * state in the width the values need - on-hand stock and home-demand history uint16, in-transit ring uint8 - and the
 //     ring indexed by ARRIVAL time: an order placed at t with (fixed) lead l goes to plane (t + l) % L of its warehouse
@@ -13,11 +15,9 @@
 //   * demand as sparse "lines" (marlsc_step_io.lines): the non-zero (order, SKU) cells, pre-sorted into 32 streams by
 //     SKU % 32. Lane l walks stream l - no pass over 80 %-zero dense rows, no shuffles, 2 bytes per line instead of
 //     S + 2 bytes per order.
-//   * the lane that owns SKU s owns every cell (w, s): stock [W,S] lives in shared memory for the step, a SKU's
+//   * in the allocation the lane that owns SKU s owns every cell (w, s): stock [W,S] lives in shared memory, a SKU's
 //     availability over the warehouses in two registers, and a trip of the allocation loop is one shipment from the
 //     cheapest warehouse that has the SKU (same chains as env_alloc.cuh; demand_allocator.py:150-208).
-//   * rewards come out of the same kernel: no cost workspaces, no reward launch, inventory and the home-demand plane
-//     cross HBM once.
 //
 // Semantics are the reference's (multi_env.py:253-366), results equal the wide kernels' (integers exact; float64 cost
 // sums in a different order).
@@ -32,7 +32,7 @@ constexpr int kCompactMaxR = 64;          // region id field of a line
 constexpr int kCompactMaxW = 16;          // availability masks
 constexpr int kCompactMaxL = 16;
 
-// shared memory of the step kernel: [perm5 | prio16 | home_wh | warp 0 | warp 1 | ...], byte offsets
+// shared memory of the allocation kernel (K1b'): [perm5 | prio16 | home_wh | warp 0 | warp 1 | ...], byte offsets
 struct CompactSmem {
   int t_perm, t_prio, t_home, t_bytes;          // per CTA
   int inv, shipq, lostU, lostP, avail, ring, warp_bytes;     // per warp, from the warp's base
@@ -66,7 +66,6 @@ __host__ __device__ inline uint32_t identity_map_word(int lane, int S) {
   return m;
 }
 
-int launch_step_compact(const LaunchArgs& a, const marlsc_step_io_t& io, int t, cudaStream_t s);
 struct SplitWork;
 int launch_split_compact(const LaunchArgs& a, const marlsc_step_io_t& io, const SplitWork& wk, int t, cudaStream_t s);
 int launch_reset_compact(const LaunchArgs& a, const int32_t* init, int per_env, float* obs, cudaStream_t s);

@@ -120,10 +120,7 @@ struct DevSpec {
   const uint8_t* prio16;       // [R,16] warehouses in priority order
   const uint8_t* home_wh;      // [R] the warehouse whose home region r is; 255 none, 254 several (see home_mask)
   int perm5_chunks;
-  unsigned long long home_bits; // bit r: region r (< 64) is some warehouse's home region
-  int compact_ok;              // the configuration fits the compact state layout and its fused kernel
-  int compact_prefetch;        // the per-environment state blocks are 16-byte granular: bulk L2 prefetches are legal
-  int feature_bulk;            // K1c' may fetch an environment's stock / history blocks with cp.async.bulk (W S % 8 == 0)
+  int compact_ok;              // the configuration fits the compact state layout
   int row_rates_uniform;       // holding / weight / inbound rates do not vary over the SKUs of a warehouse
   const float* obs_mean;
   const float* obs_std;        // holds 1/std (precomputed on the host in float32)

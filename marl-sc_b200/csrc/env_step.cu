@@ -4,7 +4,6 @@
 
 #include <atomic>
 #include <cstdio>
-#include <cstdlib>
 #include <new>
 #include <string>
 
@@ -54,7 +53,7 @@ struct marlsc_env {
   void* d_blob = nullptr;  // one allocation holding every device table
   int max_smem_optin = 0;
   int force_generic = 0;   // tests: always run the generic instantiation
-  int force_fused = 0;     // tests / comparisons: lean launches stay in the fused kernel
+  int force_fused = 0;     // WIDE layout, tests / comparisons: lean launches stay in the fused kernel
   double* d_work = nullptr;    // split step: [2, work_envs, W] cost partials
   int64_t work_envs = 0;
   int timing = 0;              // marlsc_env_set_timing: events around the launches of a step
@@ -166,7 +165,7 @@ bool split_ok(const marlsc_env* env) {
   return ((g == 8 || g == 16) && (k == 1 || k == 4)) || (g == 32 && (k == 1 || k == 4 || k == 8 || k == 16)) || g == 64;
 }
 
-// Configurations the compact layout and its fused kernel cover (include/marlsc_b200.h, MARLSC_LAYOUT_COMPACT).
+// Configurations the compact layout covers (include/marlsc_b200.h, MARLSC_LAYOUT_COMPACT).
 bool compact_eligible(const DevSpec& ds, const HostTables& tb) {
   const uint32_t caps = required_caps(ds, tb, nullptr) & ~C_REGMAP;    // the region map is applied when lines are built
   if (caps & ~kCapsLean) return false;
@@ -303,10 +302,6 @@ int marlsc_env_create(const marlsc_env_spec_t* spec, int device, marlsc_env_t** 
   env->ds.prio16 = t.prio16.empty() ? nullptr : b + o_p16;
   env->ds.home_wh = b + o_hw;
   env->ds.compact_ok = compact_eligible(env->ds, env->tb) ? 1 : 0;
-  // cp.async.bulk.prefetch.L2 wants 16-byte aligned addresses and sizes: true for every environment's block when the
-  // smallest one (W*S bytes of uint8 quantities) is a multiple of 16 (MARLSC_NO_PREFETCH=1 switches them off for A/B runs)
-  env->ds.compact_prefetch = ((env->ds.W * env->ds.S) % 16 == 0 && !std::getenv("MARLSC_NO_PREFETCH")) ? 1 : 0;
-  env->ds.feature_bulk = ((env->ds.W * env->ds.S) % 8 == 0 && std::getenv("MARLSC_FEATURE_BULK")) ? 1 : 0;   // opt-in: measured slower
   env->layout = env->ds.compact_ok ? MARLSC_LAYOUT_COMPACT : MARLSC_LAYOUT_WIDE;
   *out = env;
   return MARLSC_OK;
@@ -384,9 +379,9 @@ int marlsc_env_set_generic(marlsc_env_t* env, int32_t on) {
 
 int marlsc_env_set_fused(marlsc_env_t* env, int32_t on) {
   if (!env) return set_error(MARLSC_EINVAL, "null handle");
-  if (on && env->metrics_on && env->layout == MARLSC_LAYOUT_COMPACT)
-    return set_error(MARLSC_EUNSUPPORTED, "the compact fused step kernel does not accumulate episode metrics (marlsc_env_set_metrics)");
-  env->force_fused = on ? 1 : 0;                       // compact layout: the single fused kernel instead of the split step
+  if (on && env->layout == MARLSC_LAYOUT_COMPACT)
+    return set_error(MARLSC_EUNSUPPORTED, "the compact layout has one step (no fused kernel): force MARLSC_LAYOUT_WIDE first");
+  env->force_fused = on ? 1 : 0;
   return MARLSC_OK;
 }
 
@@ -400,8 +395,6 @@ int marlsc_env_set_metrics(marlsc_env_t* env, const marlsc_episode_metrics_t* m)
   if (!m->holding_cost || !m->penalty_cost || !m->outbound_cost || !m->inbound_cost || !m->ordered_units || !m->shipped_units ||
       !m->episode_return || !m->demand_units || !m->lost_units)
     return set_error(MARLSC_EINVAL, "every marlsc_episode_metrics pointer is required");
-  if (env->force_fused && env->layout == MARLSC_LAYOUT_COMPACT)
-    return set_error(MARLSC_EUNSUPPORTED, "the compact fused step kernel does not accumulate episode metrics (marlsc_env_set_fused)");
   env->metrics = *m;
   env->metrics_on = 1;
   return MARLSC_OK;
@@ -469,8 +462,8 @@ int step_impl(marlsc_env_t* env, const marlsc_env_state_t* state, const marlsc_s
   if (!io) return set_error(MARLSC_EINVAL, "null io");
   if ((!io->actions && !io->action_qty && !io->base_stock_level) || !io->rewards || !io->obs)
     return set_error(MARLSC_EINVAL, "io.actions (or io.action_qty / io.base_stock_level), io.rewards and io.obs must not be NULL");
-  if (io->base_stock_level && !io->actions && !io->action_qty && (env->layout != MARLSC_LAYOUT_COMPACT || env->force_fused))
-    return set_error(MARLSC_EINVAL, "io.base_stock_level needs a handle with the COMPACT layout running the split step");
+  if (io->base_stock_level && !io->actions && !io->action_qty && env->layout != MARLSC_LAYOUT_COMPACT)
+    return set_error(MARLSC_EINVAL, "io.base_stock_level needs a handle with the COMPACT layout");
   if (io->lines) {
     if (env->layout != MARLSC_LAYOUT_COMPACT) return set_error(MARLSC_EINVAL, "io.lines needs a handle with the COMPACT layout");
     if (!io->line_offsets && !io->line_counts) return set_error(MARLSC_EINVAL, "io.lines needs io.line_offsets or io.line_counts");
@@ -491,10 +484,11 @@ int step_impl(marlsc_env_t* env, const marlsc_env_state_t* state, const marlsc_s
     if (io->order_qty_bytes == 2 && !io->lines) return set_error(MARLSC_EUNSUPPORTED, "two-byte order quantities need MARLSC_LAYOUT_WIDE");
     if (io->cost_breakdown || io->d_ordered || io->d_ship || io->d_ship_count || io->d_unfulfilled || io->d_lost_orders || io->d_lost_sales)
       return set_error(MARLSC_EUNSUPPORTED, "the diagnostic outputs need MARLSC_LAYOUT_WIDE (marlsc_env_set_layout before the first reset)");
+    // the row kernels index (environment, warehouse) rows with 32 bits
+    if (state->num_envs * (int64_t)env->ds.W >= (int64_t)0xffffffffLL)
+      return set_error(MARLSC_EUNSUPPORTED, "the compact step needs num_envs * W < 2^32 - 1; force MARLSC_LAYOUT_WIDE or split the batch");
     const LaunchArgs lc{env->ds, *state, env->max_smem_optin, true};
     marlsc_step_io_t ioc = *io;
-    if (env->timing) MARLSC_CUDA(cudaEventRecord(env->marks[0], s));
-    int n_marks = 1;
     if (!io->lines) {                                  // dense orders: build the lines in the library's buffer first
       rc = ensure_lines(env, state->num_envs);
       if (rc) return rc;
@@ -504,25 +498,15 @@ int step_impl(marlsc_env_t* env, const marlsc_env_state_t* state, const marlsc_s
       ioc.line_offsets = nullptr;
       ioc.line_counts = env->d_line_counts;
       ioc.line_stride = env->line_stride;
-      if (env->timing) MARLSC_CUDA(cudaEventRecord(env->marks[n_marks], s));
-      ++n_marks;
     }
-    if (!env->force_fused && state->num_envs * (int64_t)env->ds.W < (int64_t)0xffffffffLL) {
-      // the step as row / environment kernels (K1a' place, K1b' allocate, K1c' features, K1d rewards)
-      rc = ensure_work(env, state->num_envs);
-      if (rc) return rc;
-      const SplitWork wk{env->d_work, env->d_work + (size_t)env->work_envs * env->ds.W,
-                         (env->timing && io->lines) ? env->marks : nullptr, env->metrics_on ? &env->metrics : nullptr};
-      env->timed_launches = (env->timing && io->lines) ? 4 : 0;
-      return launch_split_compact(lc, ioc, wk, t, s);
-    }
-    if (env->metrics_on)
-      return set_error(MARLSC_EUNSUPPORTED, "episode metrics need the compact split step (not the fused kernel, fewer than 2^32 rows)");
-    rc = launch_step_compact(lc, ioc, t, s);
+    // the step as row / environment kernels (K1a' place, K1b' allocate, K1c' features, K1d rewards); timed when the caller
+    // gave lines
+    rc = ensure_work(env, state->num_envs);
     if (rc) return rc;
-    if (env->timing) MARLSC_CUDA(cudaEventRecord(env->marks[n_marks], s));
-    env->timed_launches = env->timing ? n_marks : 0;
-    return MARLSC_OK;
+    const SplitWork wk{env->d_work, env->d_work + (size_t)env->work_envs * env->ds.W,
+                       (env->timing && io->lines) ? env->marks : nullptr, env->metrics_on ? &env->metrics : nullptr};
+    env->timed_launches = (env->timing && io->lines) ? 4 : 0;
+    return launch_split_compact(lc, ioc, wk, t, s);
   }
   const bool lean = !env->force_generic && (required_caps(env->ds, env->tb, io) & ~kCapsLean) == 0;
   const LaunchArgs la{env->ds, *state, env->max_smem_optin, lean};

@@ -147,9 +147,6 @@ inline std::string build_devspec(const marlsc_env_spec_t& sp, DevSpec& ds, HostT
       }
   }
   tb.home_wh.assign(R, 255);
-  ds.home_bits = 0ull;
-  for (int w = 0; w < W; ++w)
-    if (tb.home[w] < 64) ds.home_bits |= 1ull << tb.home[w];
   for (int w = 0; w < W; ++w) {
     uint8_t& h = tb.home_wh[tb.home[w]];
     h = h == 255 ? (uint8_t)w : (uint8_t)254;

@@ -1,5 +1,5 @@
-"""BatchedInventoryEnv - E independent inventory environments advanced by one fused CUDA kernel per
-timestep (csrc/env_step.cu). Tensor-in / tensor-out counterpart of the reference's
+"""BatchedInventoryEnv - E independent inventory environments advanced by the CUDA step kernels once per
+timestep (csrc/env_step.cu, csrc/env_compact.cu). Tensor-in / tensor-out counterpart of the reference's
 ``InventoryEnvironment`` (src/environment/envs/multi_env.py:38-366); the dict-based single-env API of
 the reference is provided on top of it by ``marlsc_b200.envs.InventoryEnvironment``.
 
@@ -87,8 +87,8 @@ class BatchedInventoryEnv:
                  max_orders_per_env: Optional[int] = None, layout: Optional[str] = None, episode_metrics: bool = False):
         if num_envs < 1:
             raise ValueError("num_envs must be positive")
-        if episode_metrics and fused_kernel and layout == "compact":
-            raise ValueError("episode_metrics needs the compact layout's split step: the fused kernel does not accumulate them")
+        if fused_kernel and layout == "compact":
+            raise ValueError("fused_kernel=True needs the wide layout: the compact layout has one step and no fused kernel")
         if not torch.cuda.is_available():
             raise RuntimeError("BatchedInventoryEnv needs a CUDA device: this path has no CPU implementation")
         meta = env_meta or {}
@@ -127,13 +127,12 @@ class BatchedInventoryEnv:
         with torch.cuda.device(self.device):
             _capi.check(L.marlsc_env_create(C.byref(self._spec_c), self.device.index, C.byref(handle)))
         self._h = handle
-        # State layout (include/marlsc_b200.h): "compact" (narrow state, one fused kernel, sparse demand lines) when the
+        # State layout (include/marlsc_b200.h): "compact" (narrow state, its own step kernels, sparse demand lines) when the
         # configuration qualifies and nothing asks for the general kernels; "wide" otherwise.
         if layout not in (None, "wide", "compact"):
             raise ValueError("layout must be None, 'wide' or 'compact'")
         compact = L.marlsc_env_layout(self._h) == _capi.LAYOUT_COMPACT
-        wants_wide = (bool(diagnostics or team_size or generic_kernel or (fused_kernel and layout != "compact"))
-                      or self._stock_bound() >= 32768)
+        wants_wide = bool(diagnostics or team_size or generic_kernel or fused_kernel) or self._stock_bound() >= 32768
         if layout == "compact":
             if wants_wide:
                 raise ValueError("layout='compact' excludes diagnostics / team_size / generic_kernel and needs "
@@ -146,7 +145,7 @@ class BatchedInventoryEnv:
             _capi.check(L.marlsc_env_set_team_size(self._h, team_size))
         if generic_kernel:      # tests: bypass the lean instantiation of the step kernel
             _capi.check(L.marlsc_env_set_generic(self._h, 1))
-        if fused_kernel:        # comparisons: keep lean launches in the single fused kernel instead of the split step
+        if fused_kernel:        # comparisons (wide layout): keep lean launches in the single fused kernel instead of the split step
             _capi.check(L.marlsc_env_set_fused(self._h, 1))
         self.obs_dim = int(L.marlsc_env_obs_dim(self._h))            # local_obs_dim of the reference
         self.global_obs_dim = self.n_warehouses * self.obs_dim

@@ -282,22 +282,26 @@ def test_evaluate_base_stock_known_answer_and_actor_critic():
     b.close()
 
 
-def test_metrics_refuse_unsupported_combinations():
-    """The compact fused kernel does not accumulate metrics (either order of the two switches), and a WIDE step with
-    metrics needs the diagnostic outputs."""
+def test_compact_refuses_fused_and_wide_metrics_need_diagnostics():
+    """The compact layout has no fused kernel (with or without metrics), and a WIDE step with metrics needs the diagnostic
+    outputs."""
     from marlsc_b200 import _capi
     from marlsc_b200.demand import pack_orders
     from marlsc_b200.envs import BatchedInventoryEnv
     cfg = _large_cfg()
-    with pytest.raises(ValueError, match="fused"):
-        BatchedInventoryEnv(cfg, 8, device="cuda:0", host_samplers=False, layout="compact", fused_kernel=True, episode_metrics=True)
+    for metrics in (False, True):
+        with pytest.raises(ValueError, match="fused"):
+            BatchedInventoryEnv(cfg, 8, device="cuda:0", host_samplers=False, layout="compact", fused_kernel=True,
+                                episode_metrics=metrics)
     L = _capi.lib()
-    env = BatchedInventoryEnv(cfg, 8, device="cuda:0", host_samplers=False, layout="compact", fused_kernel=True)
     bufs = [torch.zeros(80, dtype=torch.float64, device="cuda:0") for _ in range(9)]
     m = _capi.EpisodeMetricsC(*[t.data_ptr() for t in bufs])
-    assert L.marlsc_env_set_metrics(env._h, C.byref(m)) == -4           # MARLSC_EUNSUPPORTED
+    env = BatchedInventoryEnv(cfg, 8, device="cuda:0", host_samplers=False, layout="compact")
+    assert L.marlsc_env_set_fused(env._h, 1) == -4                      # MARLSC_EUNSUPPORTED
+    assert L.marlsc_env_set_fused(env._h, 0) == 0
     env.close()
     env = BatchedInventoryEnv(cfg, 8, device="cuda:0", host_samplers=False, episode_metrics=True)
+    assert env.layout == "compact"
     assert L.marlsc_env_set_fused(env._h, 1) == -4
     partial = _capi.EpisodeMetricsC(*[t.data_ptr() for t in bufs[:8]])
     assert L.marlsc_env_set_metrics(env._h, C.byref(partial)) == -1     # MARLSC_EINVAL: a pointer is missing

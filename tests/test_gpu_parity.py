@@ -44,22 +44,17 @@ def test_cuda_matches_reference_auto_team(name):
     _run(Golden(name))
 
 
-@pytest.mark.parametrize("mode", ["auto", "compact_fused", "split", "fused", "generic"])
+@pytest.mark.parametrize("mode", ["auto", "split", "fused", "generic"])
 @pytest.mark.parametrize("name", NAMES)
 def test_cuda_without_diagnostics(name, mode):
-    """No diagnostic outputs. ``auto``: the compact layout and its fused kernel where the configuration qualifies (the
-    large networks), else the wide lean path; ``split``: the wide layout's lean path - the four-kernel split step for
-    teams of 8+ lanes, else the lean fused kernel; ``fused`` keeps lean launches in the wide fused kernel; ``generic``
-    forces the generic instantiation."""
-    if mode == "compact_fused":
-        if not name.startswith("large_network"):
-            pytest.skip("configuration does not qualify for the compact layout")
-        used = _run(Golden(name), diagnostics=False, fused=True, layout="compact")
-    else:
-        used = _run(Golden(name), diagnostics=False, generic=mode == "generic", fused=mode == "fused",
-                    layout="wide" if mode == "split" else None)
+    """No diagnostic outputs. ``auto``: the compact layout and its step where the configuration qualifies (the large
+    networks), else the wide lean path; ``split``: the wide layout's lean path - the four-kernel split step for teams of
+    8+ lanes, else the lean fused kernel; ``fused`` keeps lean launches in the wide fused kernel; ``generic`` forces the
+    generic instantiation."""
+    used = _run(Golden(name), diagnostics=False, generic=mode == "generic", fused=mode == "fused",
+                layout="wide" if mode == "split" else None)
     if name.startswith("large_network"):
-        assert used == ("compact" if mode in ("auto", "compact_fused") else "wide")
+        assert used == ("compact" if mode == "auto" else "wide")
 
 
 @pytest.mark.parametrize("team", [1, 2, 4, 8, 16, 32])
@@ -1013,13 +1008,11 @@ def test_poisson_inversion_survives_the_largest_uniform():
     (6, 64, 12, "shipment", True, 20, 4, "norm_id_team"),   # fixed mean/std normalisation, one-hot id, team reward, home-demand block
     (10, 100, 50, "shipment", True, 30, 6, "region_map"),   # 50 raw regions mapped onto 10 included ones (preprocessor.py:382-441)
 ])
-@pytest.mark.parametrize("fused", [False, True])
-def test_compact_step_vs_oracle(W, S, R, lost, pen_uniform, max_orders, lead_hi, variant, fused):
-    """The compact layout's kernels (csrc/env_compact.cu: the split step K1a'-K1d, and with ``fused`` the single fused
-    kernel) against the oracle: scarce stock (most lines are split or
-    lost), environments without orders, all-zero orders, a batch that does not fill the last CTA, a mid-run reset, ring
-    wrap-around, and every way of feeding it (lines packed on the host, dense rows converted on the device, integer
-    quantity actions, a region map)."""
+def test_compact_step_vs_oracle(W, S, R, lost, pen_uniform, max_orders, lead_hi, variant):
+    """The compact layout's kernels (csrc/env_compact.cu: the step K1a'-K1d) against the oracle: scarce stock (most lines
+    are split or lost), environments without orders, all-zero orders, a batch that does not fill the last CTA, a mid-run
+    reset, ring wrap-around, and every way of feeding it (lines packed on the host, dense rows converted on the device,
+    integer quantity actions, a region map)."""
     from marlsc_b200.config import environment_config_from_dict
     from marlsc_b200.demand import pack_orders
     from marlsc_b200.envs import BatchedInventoryEnv, DeviceOrders
@@ -1039,7 +1032,7 @@ def test_compact_step_vs_oracle(W, S, R, lost, pen_uniform, max_orders, lead_hi,
         okw = dict(obs_normalization="meanstd_custom", obs_stats=stats, include_warehouse_id=True)
     E, T = 11, 2 * lead_hi + 7
     env = BatchedInventoryEnv(cfg, E, device="cuda:0", host_samplers=False, env_meta=meta, region_map=region_map,
-                              layout="compact", fused_kernel=fused)
+                              layout="compact")
     assert env.layout == "compact"
     oracles = [OracleEnv(env_dict, **okw) for _ in range(E)]
     maxq = np.asarray(env_dict["action_space"]["params"]["max_order_quantities"])
@@ -1090,31 +1083,6 @@ def test_compact_step_vs_oracle(W, S, R, lost, pen_uniform, max_orders, lead_hi,
             lost_any = lost_any or out["lost_orders"].sum() > 0
     assert lost_any, "workload was meant to lose sales"
     env.close()
-
-
-def test_feature_kernel_bulk_copy_variant_is_bit_identical(monkeypatch):
-    """K1c' has an opt-in variant that fetches an environment's stock and history blocks with cp.async.bulk + mbarriers
-    (MARLSC_FEATURE_BULK=1, csrc/env_compact.cu compact_feature_bulk_kernel; measured slower, kept for audit): same
-    observations, rewards and state as the default register version, including a batch that does not fill the grid."""
-    from marlsc_b200.config import environment_config_from_dict
-    from marlsc_b200.envs import BatchedInventoryEnv
-    rng = np.random.default_rng(11)
-    cfg = environment_config_from_dict(dict(_lean_env_dict(rng, 10, 100, 50, "shipment", True, 6, demand_home=True), allow_region_mismatch=True))
-    E = 777
-    a = BatchedInventoryEnv(cfg, E, device="cuda:0", host_samplers=False, device_demand=True, demand_seed=9, layout="compact")
-    monkeypatch.setenv("MARLSC_FEATURE_BULK", "1")
-    b = BatchedInventoryEnv(cfg, E, device="cuda:0", host_samplers=False, device_demand=True, demand_seed=9, layout="compact")
-    monkeypatch.delenv("MARLSC_FEATURE_BULK")
-    assert torch.equal(a.reset(), b.reset())
-    gen = torch.Generator(device="cuda:0").manual_seed(1)
-    for t in range(12):
-        act = torch.rand((E, 10, 100), device="cuda:0", generator=gen) * 2 - 1
-        oa, ra, _ = a.step(act)
-        ob, rb, _ = b.step(act)
-        assert torch.equal(oa, ob) and torch.equal(ra, rb), t
-        assert torch.equal(a.inventory, b.inventory) and torch.equal(a.demand_hist, b.demand_hist)
-    a.close()
-    b.close()
 
 
 def test_lines_from_orders_matches_host_packer():

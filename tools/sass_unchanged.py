@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Check that every kernel of an older build of libmarlsc_b200.so compiles to the same machine code in a newer one.
 
-    python tools/sass_unchanged.py OLD.so NEW.so
+    python tools/sass_unchanged.py [--ignore-param-offsets] OLD.so NEW.so
 
 Runs ``cuobjdump -sass`` and ``cuobjdump -res-usage`` on both libraries (no GPU needed), demangles the kernel names
 and identifies a kernel by its qualified name and template arguments (parameter lists are left out: a kernel may gain
@@ -11,6 +11,11 @@ of the old one (``k<false>`` for ``k``). Every kernel of the old build must exis
 instruction text and the same registers, stack, static shared memory and local memory (a template kernel instantiated in several translation units has one
 copy per unit: the copies are compared as a set); kernels only the new build has are listed. Exit status 0 when nothing
 changed, 1 otherwise.
+
+``--ignore-param-offsets`` compares the instructions with every kernel-parameter operand ``c[0x0][...0x...]`` reduced
+to ``c[0x0][...*]`` and without the ``/* 0x... */`` encodings (which hold those offsets). Use it when a change moves
+kernel parameters, for example a smaller struct passed by value: opcodes, registers, predicates, branch targets and
+resource usage are still compared exactly.
 """
 from __future__ import annotations
 
@@ -75,14 +80,20 @@ def drop_trailing_false(key: str) -> str:
     return key
 
 
-def _normalise(line: str) -> str:
+_PARAM = re.compile(r"c\[0x0\]\[([^\]]*?)0x[0-9a-f]+\]")   # a constant-bank-0 operand: kernel parameters and launch constants
+_ENCODING = re.compile(r"/\* 0x[0-9a-f]+ \*/")
+
+
+def _normalise(line: str, ignore_param_offsets: bool = False) -> str:
+    if ignore_param_offsets:
+        line = _ENCODING.sub("", _PARAM.sub(r"c[0x0][\1*]", line))
     return re.sub(r"\s+", " ", line).strip()
 
 
 Kernel = Tuple[Tuple[str, ...], str]                    # (instruction lines, "REG:n STACK:n SHARED:n LOCAL:n") of one copy
 
 
-def read_library(path: str) -> Dict[str, List[Kernel]]:
+def read_library(path: str, ignore_param_offsets: bool = False) -> Dict[str, List[Kernel]]:
     """kernel key -> its copies, sorted"""
     exe = _cuobjdump()
     sass = _run([exe, "-sass", path]).splitlines()
@@ -94,7 +105,9 @@ def read_library(path: str) -> Dict[str, List[Kernel]]:
             bodies.append((m.group(1), []))
             continue
         if bodies and line.strip().startswith("/*") and "*/" in line:
-            bodies[-1][1].append(_normalise(line))
+            text = _normalise(line, ignore_param_offsets)
+            if text:                                     # the second half of an encoding is a line of its own
+                bodies[-1][1].append(text)
     regs: Dict[str, List[str]] = {}
     for line, nxt in zip(res, res[1:] + [""]):          # "Function <name>:" then its resource line
         m = _RES.match(line)
@@ -147,8 +160,10 @@ def main() -> int:
     ap.add_argument("old", help="libmarlsc_b200.so of the older build")
     ap.add_argument("new", help="libmarlsc_b200.so of the newer build")
     ap.add_argument("--verbose", action="store_true", help="list every unchanged kernel")
+    ap.add_argument("--ignore-param-offsets", action="store_true",
+                    help="do not compare the offsets of kernel-parameter operands (and the encodings that hold them)")
     a = ap.parse_args()
-    old, new = read_library(a.old), read_library(a.new)
+    old, new = read_library(a.old, a.ignore_param_offsets), read_library(a.new, a.ignore_param_offsets)
     report, problems, added = compare(old, new)
     if a.verbose:
         print("\n".join(report))
