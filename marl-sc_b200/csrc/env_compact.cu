@@ -36,12 +36,14 @@ __device__ __forceinline__ void red_s_add_f64(uint32_t a, double v) {   // share
     asm volatile("atom.shared.cas.b64 %0, [%1], %2, %3;" : "=l"(old) : "r"(a), "l"(seen), "l"(want) : "memory");
   } while (old != seen);
 }
-__device__ __forceinline__ void red_g_add(uint32_t* p, uint32_t v) { asm volatile("red.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
 __device__ __forceinline__ void prefetch_l2_bulk(const void* p, uint32_t bytes) {
   asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
 }
 
 __device__ __forceinline__ uint32_t ld_nc_u32(const uint32_t* p) { uint32_t v; asm volatile("ld.global.nc.u32 %0, [%1];" : "=r"(v) : "l"(p)); return v; }
+__device__ __forceinline__ void ld_nc_u32_if(uint32_t& v, const uint32_t* p, bool c) {   // v = *p when c, else v stays
+  asm volatile("{ .reg .pred q; setp.ne.u32 q, %2, 0; @q ld.global.nc.u32 %0, [%1]; }" : "+r"(v) : "l"(p), "r"((uint32_t)c));
+}
 
 // A lane's line stream (marlsc_step_io.lines): two consecutive entries per 32-bit word, words of one round pair side
 // by side for the 32 lanes. The first word of a lane is its SKU map (byte k = the SKU its slot k stands for, 255 = none;
@@ -64,25 +66,27 @@ struct LineStream {
     at = 160u;
   }
   __device__ __forceinline__ uint32_t next() const { return cur & 0xffffu; }   // 0: the stream has ended
-  __device__ __forceinline__ void pop() {
+  __device__ __forceinline__ void pop() {         // selects rather than a branch: nearly every trip some lane of the warp refills
     cur >>= 16;
-    if (cur == 0u) {
-      cur = w1;
-      w1 = w2;
-      w2 = w3;
-      w3 = at < n ? ld_nc_u32(base + at) : 0u;
-      at += 32u;
-    }
+    const bool adv = cur == 0u;
+    cur = adv ? w1 : cur;
+    w1 = adv ? w2 : w1;
+    w2 = adv ? w3 : w2;
+    w3 = adv ? 0u : w3;
+    ld_nc_u32_if(w3, base + at, adv && at < n);
+    at += adv ? 32u : 0u;
   }
 };
 
-// The SKU a lane's slot stands for (byte `slot` of its map word).
+// Byte `slot` of a map word.
 __device__ __forceinline__ uint32_t map_sku(uint32_t map, uint32_t slot) { return __byte_perm(map, 0u, 0x4440u + slot); }
 
 // Availability masks of a lane's SKUs from the staged stock [W,S] uint16 at shared address a_inv: bit w + 16 (k & 1) of
-// (k & 2 ? avhi : avlo) says warehouse w holds the SKU of slot k. Map bytes that name no SKU (255, or anything >= S in a
-// malformed stream) are pointed at SKU S-1 with an empty mask: their lines, if any, count as lost and touch no memory
-// outside the stock image.
+// (k & 2 ? avhi : avlo) says warehouse w holds the SKU of slot k. The map word is rewritten to byte k = 2 x the SKU of
+// slot k (the byte offset of its cell in a stock row; S <= 128). Map bytes that name no SKU (255, or anything >= S in a
+// malformed stream) are pointed at SKU S-1 with an empty mask: their lines, if any, count as lost and leave the stock
+// alone (the home demand of such lines lands on SKU S-1, whose owner is another lane: the result is undefined, as for
+// any stream that breaks the one-owner rule of marlsc_step_io.lines).
 __device__ __forceinline__ void owner_masks(uint32_t& map, uint32_t a_inv, int W, int S, uint32_t& avlo, uint32_t& avhi) {
   avlo = avhi = 0u;
   uint32_t fixed = 0u;
@@ -91,7 +95,7 @@ __device__ __forceinline__ void owner_masks(uint32_t& map, uint32_t a_inv, int W
     uint32_t sku = (map >> (8 * k)) & 0xffu;
     const bool named = sku < (uint32_t)S;
     if (!named) sku = (uint32_t)S - 1u;
-    fixed |= sku << (8 * k);
+    fixed |= (2u * sku) << (8 * k);
     uint32_t m = 0u;
     const uint32_t a = a_inv + 2u * sku;
     for (int w = 0; w < W; ++w) m |= (ld_s_u16(a + (uint32_t)w * 2u * (uint32_t)S) != 0u ? 1u : 0u) << w;
@@ -112,44 +116,50 @@ __device__ __forceinline__ void put(const DevSpec& sp, bool ms, float* __restric
 // the lane's current line is done, take the next entry of its stream; then one shipment from the cheapest warehouse that
 // holds the SKU, or the lost-sales bookkeeping when none does. Lanes only meet in the exit vote. Stock [W,S] uint16,
 // shipped units [W,R] and lost units [R] live in shared memory, a lane's availability masks in two registers. The cells
-// of the SKUs named by the lane's map belong to this lane alone for the duration of the chains.
-template <int NCH>
-__device__ __forceinline__ void allocation_chains(const DevSpec& sp, LineStream& ls, uint32_t a_perm, uint32_t a_prio, uint32_t a_home,
-                                                  uint32_t a_inv, uint32_t a_shipq, uint32_t a_lostU, uint32_t a_lostP, uint32_t& avlo,
-                                                  uint32_t& avhi, uint32_t* hist32) {
-  const uint32_t S = sp.S, S2 = 2u * S, R4 = 4u * sp.R, map = ls.map;
-  const bool pen_uniform = sp.pen_uniform != 0;
-  uint32_t rem = 0u, r = 0u, sl = 0u, sku2 = 0u, cand = 0u;   // units left of the current line, its region, SKU slot, 2 x SKU, candidate bits
+// of the SKUs named by the lane's map belong to this lane alone for the duration of the chains, and so do the cells
+// (w, s) of this step's home-region demand plane [W,S] uint16 that follows the stock image: plain loads and stores.
+// Everything a trip needs of its line is worked out once when the line is taken: the shared addresses of the SKU's
+// stock cell in warehouse 0, of the region's entry in row 0 of the shipped-unit table and of the region's record
+// (compact_region_bytes). From those a shipment is one multiply-add by a row stride (a launch constant) per table.
+// PEN_UNIFORM: every SKU carries the same lost-sales penalty rate, so lost units are enough (else an fp64
+// shared-memory add per lost line).
+constexpr uint32_t kHomeNone = 0xffffu, kHomeSeveral = 0xfffeu;   // home-table entries besides a plane offset
+
+template <int NCH, bool PEN_UNIFORM>
+__device__ __forceinline__ void allocation_chains(const DevSpec& sp, const CompactSmem& lay, LineStream& ls, uint32_t a_reg0,
+                                                  uint32_t a_inv, uint32_t a_shipq, uint32_t a_lostP, uint32_t& avlo,
+                                                  uint32_t& avhi) {
+  constexpr uint32_t kPrio = NCH * 64, kHome = NCH * 64 + 16;     // offsets inside a region record
+  const uint32_t map = ls.map;
+  // the current line: units left, candidate warehouses (priority order), 16 x its SKU slot (the slot's first bit in
+  // avhi:avlo), stock cell in warehouse 0, shipped units of the region at warehouse 0, the region's record
+  uint32_t rem = 0u, cand = 0u, sl16 = 0u, a_cell = 0u, a_sq = 0u, a_reg = 0u;
   while (true) {
     const uint32_t n0 = ls.next();
     if (rem == 0u && n0 != 0u) {
       ls.pop();
       rem = n0 & 0xffu;
-      r = (n0 >> 8) & 0x3fu;
-      sl = n0 >> 14;
-      sku2 = 2u * map_sku(map, sl);
+      const uint32_t r = (n0 >> 8) & 0x3fu;
+      sl16 = (n0 >> 10) & 0x30u;
+      a_cell = a_inv + map_sku(map, n0 >> 14);
+      a_sq = a_shipq + 4u * r;
+      a_reg = a_reg0 + r * (uint32_t)compact_region_bytes(NCH);
       // which warehouses hold the SKU (bit w), then the same bits in the region's priority order
-      const uint32_t am = ((sl & 2u ? avhi : avlo) >> (16u * (sl & 1u))) & 0xffffu;
-      const uint32_t pm = a_perm + r * (NCH * 64u);
-      cand = ld_s_u16(pm + 2u * (am & 31u));
-      if (NCH > 1) cand |= ld_s_u16(pm + 64u + 2u * ((am >> 5) & 31u));
-      if (NCH > 2) cand |= ld_s_u16(pm + 128u + 2u * ((am >> 10) & 31u));
-      if (NCH > 3) cand |= ld_s_u16(pm + 192u + 2u * ((am >> 15) & 31u));
-      if (hist32) {                                   // home-region demand of this step (multi_env.py:763-768)
-        const uint32_t hw = ld_s_u8(a_home + r);
-        if (hw != 255u) {
-          const uint32_t s = sku2 >> 1;
-          if (hw != 254u) {                           // two uint16 cells share a word: add into the cell's half, nobody waits
-            const uint32_t c = hw * S + s;
-            red_g_add(hist32 + (c >> 1), rem << (16u * (c & 1u)));
-          } else {
-            uint32_t hm = sp.home_mask[r];
-            while (hm) {
-              const uint32_t c = (uint32_t)lowest_bit(hm) * S + s;
-              hm &= hm - 1;
-              red_g_add(hist32 + (c >> 1), rem << (16u * (c & 1u)));
-            }
-          }
+      const uint32_t am = ((sl16 & 32u ? avhi : avlo) >> (sl16 & 16u)) & 0xffffu;
+      cand = ld_s_u16(a_reg + 2u * (am & 31u));
+      if (NCH > 1) cand |= ld_s_u16(a_reg + 64u + 2u * ((am >> 5) & 31u));
+      if (NCH > 2) cand |= ld_s_u16(a_reg + 128u + 2u * ((am >> 10) & 31u));
+      if (NCH > 3) cand |= ld_s_u16(a_reg + 192u + 2u * ((am >> 15) & 31u));
+      // home-region demand of this step (multi_env.py:763-768): the entry is the offset of the home warehouse's history
+      // cell from the stock cell
+      const uint32_t ho = ld_s_u16(a_reg + kHome);
+      if (ho < kHomeSeveral) {
+        st_s_u16(a_cell + ho, ld_s_u16(a_cell + ho) + rem);
+      } else if (ho == kHomeSeveral) {
+        const uint32_t h0 = (uint32_t)(lay.hist - lay.inv);
+        for (uint32_t hm = sp.home_mask[r]; hm; hm &= hm - 1) {
+          const uint32_t c = a_cell + h0 + (uint32_t)lowest_bit(hm) * (uint32_t)lay.inv_row;
+          st_s_u16(c, ld_s_u16(c) + rem);
         }
       }
     }
@@ -157,23 +167,22 @@ __device__ __forceinline__ void allocation_chains(const DevSpec& sp, LineStream&
       if (cand != 0u) {                               // ship from the cheapest warehouse that has the SKU
         const uint32_t v = (uint32_t)lowest_bit(cand);
         cand &= cand - 1;
-        const uint32_t w = ld_s_u8(a_prio + r * 16u + v);
-        const uint32_t cell = a_inv + w * S2 + sku2;
+        const uint32_t w = ld_s_u8(a_reg + kPrio + v);
+        const uint32_t cell = a_cell + w * (uint32_t)lay.inv_row;
         const uint32_t a = ld_s_u16(cell);            // the cells of a SKU belong to this lane
         const uint32_t f = rem < a ? rem : a;
         st_s_u16(cell, a - f);
-        red_s_add(a_shipq + w * R4 + 4u * r, f);
+        red_s_add(a_sq + w * (uint32_t)lay.shipq_row, f);
         rem -= f;
         if (a == f) {                                 // emptied
-          const uint32_t clr = ~(1u << (w + 16u * (sl & 1u)));
-          if (sl & 2u) avhi &= clr; else avlo &= clr;
+          const uint32_t b = w + sl16;
+          if (b & 32u) avhi &= ~(1u << (b & 31u)); else avlo &= ~(1u << (b & 31u));
         }
       }
       if (rem != 0u && cand == 0u) {
-        // no warehouse can supply the rest: lost (demand_allocator.py:205-208); units are enough when every SKU
-        // carries the same penalty rate
-        red_s_add(a_lostU + 4u * r, rem);
-        if (!pen_uniform) red_s_add_f64(a_lostP + 8u * r, (double)rem * sp.pen_rate[sku2 >> 1]);
+        // no warehouse can supply the rest: lost (demand_allocator.py:205-208)
+        red_s_add(a_sq + (uint32_t)lay.lost_off, rem);
+        if (!PEN_UNIFORM) red_s_add_f64(a_lostP + 2u * (a_sq - a_shipq), (double)rem * sp.pen_rate[(a_cell - a_inv) >> 1]);
         rem = 0u;
       }
     }
@@ -202,7 +211,7 @@ __device__ __forceinline__ float nrm(float x, const float* __restrict__ mean, co
 #define VALID(k) ((k) < FS || ((k) == FS && tail))
 
 // K1a': one warp per (environment, warehouse) row - order quantities, arrivals, the row of the ring rewritten with the
-// new orders in, history plane cleared, pipeline block of the observation row; the row's inbound cost goes to cost_rows.
+// new orders in, pipeline block of the observation row; the row's inbound cost goes to cost_rows.
 // Loads: lane q reads the four consecutive cells 4q .. 4q+3 of the row and of each of its L ring planes (vector loads,
 // all in flight at once). The row's L x S bytes are then laid out in shared memory in pipeline-slot order (slot k =
 // plane (t + 1 + k) % L, multi_env.py:941-968; slot L-1 is the arrival plane, emptied), the new orders are dropped into
@@ -236,7 +245,6 @@ compact_place_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
   const int LS4 = L * S4;
   int po0 = (pa + 1) * S4;
   po0 = po0 == LS4 ? 0 : po0;
-  const bool need_hist = sp.need_hist != 0;
   uint32_t* const row4 = reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(st.ring_qty) + (e * WS + (int64_t)w * S) * L) + c4;
   // every load of the row first
   float4 a4 = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -313,8 +321,6 @@ compact_place_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
   }
   if (mine) {
     *inv4 = make_uint2(ni[0] | (ni[1] << 16), ni[2] | (ni[3] << 16));
-    if (need_hist)
-      reinterpret_cast<uint2*>(static_cast<uint16_t*>(st.demand_hist) + e * (int64_t)kWindow * WS + (t % kWindow) * WS + w * S)[c4] = make_uint2(0u, 0u);
   }
   if (by_row) {
     nQ = __reduce_add_sync(FULL, nQ);
@@ -368,12 +374,24 @@ compact_alloc_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
                      double* __restrict__ cost_alloc, int t, const __grid_constant__ marlsc_episode_metrics_t m) {
   extern __shared__ __align__(16) unsigned char smem[];
   const int W = sp.W, S = sp.S, R = sp.R, WS = W * S;
+  const bool need_hist = sp.need_hist != 0;
   {
-    const int n_perm = (R * NCH * 32) >> 1, n_prio = (R * 16) >> 2, n_home = (R + 3) >> 2;
-    for (int i = threadIdx.x; i < n_perm + n_prio + n_home; i += blockDim.x) {
-      if (i < n_perm) reinterpret_cast<uint32_t*>(smem + lay.t_perm)[i] = reinterpret_cast<const uint32_t*>(sp.perm5)[i];
-      else if (i < n_perm + n_prio) reinterpret_cast<uint32_t*>(smem + lay.t_prio)[i - n_perm] = reinterpret_cast<const uint32_t*>(sp.prio16)[i - n_perm];
-      else reinterpret_cast<uint32_t*>(smem + lay.t_home)[i - n_perm - n_prio] = reinterpret_cast<const uint32_t*>(sp.home_wh)[i - n_perm - n_prio];
+    // region records, word by word: perm5 chunks, prio16 row, home entry = the offset of the home warehouse's history
+    // cell from the stock cell of the same SKU in warehouse 0 (allocation_chains), kHomeSeveral (home_mask) or
+    // kHomeNone (all kHomeNone without a history plane)
+    constexpr int kWords = compact_region_bytes(NCH) / 4, kPerm = NCH * 16;
+    for (int i = threadIdx.x; i < R * kWords; i += blockDim.x) {
+      const int r = i / kWords, j = i - r * kWords;
+      uint32_t v;
+      if (j < kPerm) {
+        v = reinterpret_cast<const uint32_t*>(sp.perm5)[r * kPerm + j];
+      } else if (j < kPerm + 4) {
+        v = reinterpret_cast<const uint32_t*>(sp.prio16)[r * 4 + j - kPerm];
+      } else {
+        const uint32_t hw = sp.home_wh[r];
+        v = !need_hist || hw == 255u ? kHomeNone : hw == 254u ? kHomeSeveral : (uint32_t)(lay.hist - lay.inv) + hw * (uint32_t)lay.inv_row;
+      }
+      reinterpret_cast<uint32_t*>(smem)[i] = v;
     }
   }
   __syncthreads();
@@ -397,6 +415,9 @@ compact_alloc_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
     s_lostU[i] = 0u;
     if (!pen_uniform) s_lostP[i] = 0.0;
   }
+  uint2* const s_hist = reinterpret_cast<uint2*>(wbase + lay.hist);   // this step's home-region demand, four cells per word pair
+  if (need_hist)
+    for (int i = lane; i < WS / 4; i += 32) s_hist[i] = make_uint2(0u, 0u);
   // stock in: five rows in flight per lane
   uint16_t* const g_inv = pinned(static_cast<uint16_t*>(st.inventory) + e * WS + lane);
   for (int w0 = 0; w0 < W; w0 += 5) {
@@ -414,20 +435,25 @@ compact_alloc_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
   __syncwarp();
   uint32_t avlo, avhi;                                // which warehouses hold the SKUs this lane's streams name
   owner_masks(ls.map, sm_addr(s_inv), W, S, avlo, avhi);
-  const bool need_hist = sp.need_hist != 0;
-  uint32_t* const hist32 = need_hist ? reinterpret_cast<uint32_t*>(static_cast<uint16_t*>(st.demand_hist) + e * (int64_t)kWindow * WS + (t % kWindow) * WS) : nullptr;
   {
     // every shared address the chains use is one of two bases plus a launch constant (the layout is a kernel parameter)
     const uint32_t a_cta = sm_addr(smem), a_warp = a_cta + (uint32_t)lay.t_bytes + (uint32_t)wid * (uint32_t)lay.warp_bytes;
-    allocation_chains<NCH>(sp, ls, a_cta + (uint32_t)lay.t_perm, a_cta + (uint32_t)lay.t_prio, a_cta + (uint32_t)lay.t_home,
-                           a_warp + (uint32_t)lay.inv, a_warp + (uint32_t)lay.shipq, a_warp + (uint32_t)lay.lostU,
-                           a_warp + (uint32_t)lay.lostP, avlo, avhi, hist32);
+    if (pen_uniform)
+      allocation_chains<NCH, true>(sp, lay, ls, a_cta, a_warp + (uint32_t)lay.inv, a_warp + (uint32_t)lay.shipq, a_warp + (uint32_t)lay.lostP,
+                                   avlo, avhi);
+    else
+      allocation_chains<NCH, false>(sp, lay, ls, a_cta, a_warp + (uint32_t)lay.inv, a_warp + (uint32_t)lay.shipq, a_warp + (uint32_t)lay.lostP,
+                                    avlo, avhi);
   }
   __syncwarp();
   for (int w0 = 0; w0 < W; ++w0)                       // stock out (multi_env.py:307; never negative)
 #pragma unroll
     for (int k = 0; k < kSlots; ++k)
       if (VALID(k)) g_inv[w0 * S + 32 * k] = s_inv[w0 * S + lane + 32 * k];
+  if (need_hist) {                                    // every cell of this step's history plane (K1c' reads it)
+    uint2* const g_hist = reinterpret_cast<uint2*>(static_cast<uint16_t*>(st.demand_hist) + (e * kWindow + t % kWindow) * (int64_t)WS);
+    for (int i = lane; i < WS / 4; i += 32) g_hist[i] = s_hist[i];
+  }
   // Outbound cost and lost-sales penalty of every warehouse (reward_calculator.py:134-142). Lanes take regions (two per
   // lane cover R <= 64). Per region the lost volume's cost is either spread over the warehouses in proportion to what
   // they shipped there (shipment handler, lost_sales_handler.py:113-148: a rate per shipped unit, one division per
@@ -561,7 +587,7 @@ compact_feature_kernel(const __grid_constant__ DevSpec sp, const __grid_constant
   if (mine) {                                         // every load of the row first
     iv = *inv4;
     if (need_hist) {
-      // this step's plane was accumulated by K1b' with red.global: read it from L2
+      // this step's plane, written whole by K1b': read once, from L2
       asm volatile("ld.global.cg.v2.u32 {%0, %1}, [%2];" : "=r"(hn.x), "=r"(hn.y) : "l"(reinterpret_cast<const uint2*>(hist + (t % kWindow) * WS) + c4));
 #pragma unroll
       for (int back = 1; back < kWindow; ++back)
@@ -825,7 +851,7 @@ lines_from_orders_kernel(const __grid_constant__ DevSpec sp, long long E, const 
 
 template <int NCH, bool MS, int FS>
 int launch_split_nch(const LaunchArgs& a, const marlsc_step_io_t& io, const SplitWork& wk, int t, cudaStream_t s) {
-  const CompactSmem lay = compact_smem(a.ds.W, a.ds.S, a.ds.R, NCH, a.ds.pen_uniform);
+  const CompactSmem lay = compact_smem(a.ds.W, a.ds.S, a.ds.R, NCH, a.ds.pen_uniform, a.ds.need_hist);
   const size_t smem = (size_t)lay.t_bytes + (size_t)kCompactWarps * lay.warp_bytes;
   if ((int)smem > a.max_smem_optin)
     return set_error(MARLSC_EUNSUPPORTED, "compact step: shared-memory scratch of " + std::to_string(smem) + " bytes per CTA does not fit");

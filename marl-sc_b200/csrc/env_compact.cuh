@@ -32,26 +32,31 @@ constexpr int kCompactMaxR = 64;          // region id field of a line
 constexpr int kCompactMaxW = 16;          // availability masks
 constexpr int kCompactMaxL = 16;
 
-// shared memory of the allocation kernel (K1b'): [perm5 | prio16 | home_wh | warp 0 | warp 1 | ...], byte offsets
+// shared memory of the allocation kernel (K1b'): [region records | warp 0 | warp 1 | ...], byte offsets. The record of
+// region r (compact_region_bytes each) holds everything a line of that region looks up: its perm5 chunks, its prio16 row
+// and its home-table entry (uint16), so that one base address serves all three. Per warp the home-region demand plane
+// [W,S] uint16 of this step (need_hist only) follows the stock [W,S] uint16, and the lost units [R] follow the shipped
+// units [W,R] (they are the table's row W, lost_off bytes on). inv_row and shipq_row are the bytes of one warehouse row
+// of the stock (and history) and of the shipped-unit table: the allocation loop uses them as launch constants.
+__host__ __device__ constexpr int compact_region_bytes(int nch) { return nch * 64 + 20; }
 struct CompactSmem {
-  int t_perm, t_prio, t_home, t_bytes;          // per CTA
-  int inv, shipq, lostU, lostP, avail, ring, warp_bytes;     // per warp, from the warp's base
+  int t_bytes;                                  // per CTA: the region records
+  int inv, hist, shipq, lostU, lostP, warp_bytes;     // per warp, from the warp's base
+  int inv_row, shipq_row, lost_off;
 };
-__host__ __device__ inline CompactSmem compact_smem(int W, int S, int R, int nch, int pen_uniform) {
+__host__ __device__ inline CompactSmem compact_smem(int W, int S, int R, int nch, int pen_uniform, int need_hist) {
   CompactSmem l;
+  l.t_bytes = (R * compact_region_bytes(nch) + 15) & ~15;
   int o = 0;
-  l.t_perm = o; o += (R * nch * 32 * 2 + 15) & ~15;
-  l.t_prio = o; o += R * 16;
-  l.t_home = o; o += (R + 15) & ~15;
-  l.t_bytes = o;
-  o = 0;
   l.lostP = o; o += pen_uniform ? 0 : R * 8;
   l.inv = o; o += (W * S * 2 + 15) & ~15;
+  l.hist = o; o += need_hist ? (W * S * 2 + 15) & ~15 : 0;
   l.shipq = o; o += W * R * 4;
   l.lostU = o; o += R * 4;
-  l.avail = o;                                      // (unused: availability masks live in registers)
-  l.ring = o;                                       // (unused: the line words in flight live in registers)
   l.warp_bytes = (o + 15) & ~15;
+  l.inv_row = S * 2;
+  l.shipq_row = R * 4;
+  l.lost_off = l.lostU - l.shipq;
   return l;
 }
 
