@@ -13,6 +13,8 @@ reference's per-agent ``[local_i | global]`` vector is only materialised on requ
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import pickle
 from typing import Any, Dict, List, Optional, Sequence, Tuple, Union
 
 import numpy as np
@@ -35,6 +37,10 @@ METRICS_PER_ROW = ("holding_cost", "penalty_cost", "outbound_cost", "inbound_cos
                    "episode_return")
 METRICS_PER_ENV = ("demand_units", "lost_units")
 COST_METRICS = ("holding_cost", "penalty_cost", "outbound_cost", "inbound_cost")
+# state_dict(): the device tensors a snapshot copies (None where the layout or configuration has none), and the mutable
+# attributes of a host sampler (its generator; the empirical sampler's window start)
+_SNAPSHOT_TENSORS = ("inventory", "ring_qty", "ring_lead", "demand_hist", "forecast", "obs", "rewards", "truncated")
+_SAMPLER_STATE = ("_rng", "_start_index")
 
 
 def fill_rate(demand_units: torch.Tensor, lost_units: torch.Tensor) -> torch.Tensor:
@@ -375,6 +381,71 @@ class BatchedInventoryEnv:
         m["total_cost"] = sum(m[k] for k in COST_METRICS)
         m["fill_rate"] = fill_rate(m["demand_units"], m["lost_units"])
         return m
+
+    # ------------------------------------------------------------------ snapshot
+    def _fingerprint(self) -> Dict[str, Any]:
+        """What a snapshot must agree on with the environment it is loaded into, in the order it is checked."""
+        h = hashlib.sha256()
+        for k in sorted(self.spec.scalars):
+            h.update(f"{k}={self.spec.scalars[k]!r};".encode())
+        for k in sorted(self.spec.tables):
+            arr = self.spec.tables[k]
+            h.update(f"{k}:{None if arr is None else (arr.dtype.str, arr.shape)};".encode())
+            if arr is not None:
+                h.update(np.ascontiguousarray(arr).tobytes())
+        return dict(num_envs=self.num_envs, layout=self.layout, spec=h.hexdigest(), episode_metrics=bool(self._metrics),
+                    device_demand=self._dd is not None, device_leads=self._dl is not None, host_samplers=bool(self._host_samplers))
+
+    def state_dict(self) -> Dict[str, Any]:
+        """Everything that decides this environment's future, copied to the host: the device state, observations,
+        rewards, truncation flags and episode-metric accumulators, the step / episode / sampler counters, the empirical
+        window starts and, with host samplers, their seed managers and generator states (pickled). ``load_state_dict``
+        of an environment built the same way then continues bit for bit. Waits for the queued work."""
+        host = lambda t: None if t is None else t.detach().to("cpu", copy=True)   # noqa: E731
+        sd: Dict[str, Any] = dict(
+            fingerprint=self._fingerprint(),
+            tensors={k: host(getattr(self, k)) for k in _SNAPSHOT_TENSORS},
+            metrics={k: host(v) for k, v in self._metrics.items()},
+            timestep=self.timestep, episode=self._episode, demand_step=self._demand_step,
+            lead_step=None if self._dl is None else self._dl["step"], frame_start=host(self._frame_start))
+        if self._host_samplers:
+            sampler = lambda s: {k: getattr(s, k) for k in _SAMPLER_STATE if hasattr(s, k)}   # noqa: E731
+            sd["host_samplers"] = pickle.dumps(dict(seed_managers=self.seed_managers,
+                                                    demand=[sampler(s) for s in self.demand_samplers],
+                                                    lead=[sampler(s) for s in self.lead_time_samplers]))
+        return sd
+
+    def load_state_dict(self, sd: Dict[str, Any]) -> None:
+        """Restore a ``state_dict()`` taken from an environment built the same way (number of environments, layout, spec,
+        episode metrics, device demand / lead times and host samplers on or off); ``ValueError`` names the first
+        difference."""
+        mine, theirs = self._fingerprint(), sd["fingerprint"]
+        for k, v in mine.items():
+            if theirs.get(k) != v:
+                raise ValueError(f"environment snapshot does not match this environment: {k} is {theirs.get(k)!r} in the "
+                                 f"snapshot and {v!r} here")
+        for k in _SNAPSHOT_TENSORS:
+            dst, src = getattr(self, k), sd["tensors"][k]
+            if (dst is None) != (src is None):
+                raise ValueError(f"environment snapshot does not match this environment: {k} is present in only one of them")
+            if dst is not None:
+                dst.copy_(src)
+        for k, v in self._metrics.items():
+            v.copy_(sd["metrics"][k])
+        self.timestep, self._episode, self._demand_step = int(sd["timestep"]), int(sd["episode"]), int(sd["demand_step"])
+        if self._dl is not None:
+            self._dl["step"] = int(sd["lead_step"])
+        if self._dd is not None and "lines" in self._dd:
+            self._dd["drawn"] = -1      # lines are keyed by (seed, env, step): the next step draws its own again
+        fs = sd["frame_start"]
+        self._frame_start = None if fs is None else fs.to(self.device)
+        if self._host_samplers:
+            hs = pickle.loads(sd["host_samplers"])
+            self.seed_managers = hs["seed_managers"]
+            for objs, states in ((self.demand_samplers, hs["demand"]), (self.lead_time_samplers, hs["lead"])):
+                for s, st in zip(objs, states):
+                    for k, v in st.items():
+                        setattr(s, k, v)
 
     # ------------------------------------------------------------------ heuristic policies (K5)
     def base_stock_actions(self, level: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:

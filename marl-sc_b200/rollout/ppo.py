@@ -9,7 +9,7 @@ num_minibatches``, ``shuffle_batch_per_epoch=True``, ``use_kl_loss``, ``grad_cli
 ippo.py:106-115, hysteretic weighting src/algorithms/learners/hysteretic_learner.py:39-42."""
 from __future__ import annotations
 
-from typing import Dict, List, Optional, Union
+from typing import Callable, Dict, List, Optional, Sequence, Union
 
 import torch
 import torch.distributed as dist
@@ -17,6 +17,25 @@ import torch.distributed as dist
 from .. import _capi
 from .collector import Rollout
 from .policy import ActorCritic, CentralizedActorCritic
+
+
+def lr_schedule(value: Union[float, Sequence[Sequence[float]]]) -> Callable[[int], float]:
+    """The learning rate as a function of lifetime env steps, for the config's ``learning_rate``: a scalar is constant; a
+    list of ``[timestep, lr]`` points is interpolated linearly between the points and held at the last value after the last
+    point (RLlib's piecewise schedule, which the reference's learner steps with the lifetime count of sampled env steps)."""
+    if isinstance(value, (int, float)):
+        return lambda t: float(value)
+    pts = [(float(t), float(lr)) for t, lr in value]
+
+    def at(t: int) -> float:
+        t = float(t)
+        if t <= pts[0][0]:
+            return pts[0][1]
+        for (t0, v0), (t1, v1) in zip(pts, pts[1:]):
+            if t < t1:
+                return v0 + (t - t0) / (t1 - t0) * (v1 - v0)
+        return pts[-1][1]
+    return at
 
 
 class _FusedPPOObjective(torch.autograd.Function):
@@ -174,6 +193,11 @@ class PPOLearner:
                    entropy_coeff=sp.entropy_coeff, grad_clip=sp.grad_clip, hysteretic_beta=getattr(sp, "hysteretic_beta", None),
                    use_kl_loss=bool(getattr(sp, "use_kl_loss", False)), num_epochs=sh.num_epochs,
                    num_minibatches=sh.num_minibatches, **kw)
+
+    def set_lr(self, lr: float) -> None:
+        """Learning rate of the following updates (a schedule sets it before every update, see ``lr_schedule``)."""
+        for g in self.opt.param_groups:
+            g["lr"] = float(lr)
 
     # ------------------------------------------------------------------ objective
     def loss(self, obs, actions, logp_old, adv, targets, mean_old=None, log_std_old=None) -> Dict[str, torch.Tensor]:
