@@ -113,7 +113,7 @@ typedef struct marlsc_env marlsc_env_t; /* opaque handle */
 
 /*
  * State layouts. WIDE is the general one (every configuration). COMPACT stores the same state in the width the
- * values need and indexes the in-transit ring by arrival time; it exists for the common configurations
+ * values need; it exists for the common configurations
  * (marlsc_env_layout() tells which one a handle uses; marlsc_env_set_layout() can force WIDE before the first reset):
  * fixed lead times, direct action space with order maxima <= 255, unit SKU weights, no outbound fixed costs, static
  * warehouse priority, non-binding split limit, inventory / pipeline / home-demand / rolling-mean feature blocks,
@@ -128,8 +128,9 @@ enum { MARLSC_LAYOUT_WIDE = 0, MARLSC_LAYOUT_COMPACT = 1 };
  * every array is contiguous.
  *                 WIDE                                              COMPACT
  *   inventory    int32 [E,W,S]                                      uint16 [E,W,S]
- *   ring_qty     int32 [E,D,W,S], order placed at step tau lives    uint8 [E,W,L,S], order ARRIVING at step a lives in
- *                in plane tau % D (D = ring_depth)                  plane a % L of its warehouse row (L = max_expected_lead)
+ *   ring_qty     int32 [E,D,W,S], order placed at step tau lives    uint8 [E,L,W,S], order placed at step tau lives in
+ *                in plane tau % D (D = ring_depth)                  plane tau % L (L = max_expected_lead); every cell's
+ *                                                                   quantity, 0 included, is written each step
  *   ring_lead    uint8 [E,D,W,S] actual lead of that order;         unused (NULL)
  *                NULL when lead_mode is FIXED
  *   demand_hist  int32 [E,5,W,S] home-region demand of the last     uint16 [E,5,W,S]

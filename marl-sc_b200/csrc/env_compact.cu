@@ -78,6 +78,10 @@ struct LineStream {
   }
 };
 
+// Each byte of x replaced by its top bit replicated: 0xff or 0 (prmt's sign-replicating selectors; __byte_perm
+// documents only the byte-copying ones).
+__device__ __forceinline__ uint32_t byte_signs(uint32_t x) { uint32_t r; asm("prmt.b32 %0, %1, 0, 0xBA98;" : "=r"(r) : "r"(x)); return r; }
+
 // Byte `slot` of a map word.
 __device__ __forceinline__ uint32_t map_sku(uint32_t map, uint32_t slot) { return __byte_perm(map, 0u, 0x4440u + slot); }
 
@@ -210,14 +214,18 @@ __device__ __forceinline__ float nrm(float x, const float* __restrict__ mean, co
 // SKU slot k of a lane is valid: always below FS (= S / 32, compile time), for lanes below the remainder at FS, never above
 #define VALID(k) ((k) < FS || ((k) == FS && tail))
 
-// K1a': one warp per (environment, warehouse) row - order quantities, arrivals, the row of the ring rewritten with the
-// new orders in, pipeline block of the observation row; the row's inbound cost goes to cost_rows.
-// Loads: lane q reads the four consecutive cells 4q .. 4q+3 of the row and of each of its L ring planes (vector loads,
-// all in flight at once). The row's L x S bytes are then laid out in shared memory in pipeline-slot order (slot k =
-// plane (t + 1 + k) % L, multi_env.py:941-968; slot L-1 is the arrival plane, emptied), the new orders are dropped into
-// their slots there (slot lead-1), and the image goes out twice: back to the ring as whole 32-bit words (the first
-// version stored single bytes: each touched a 32-byte sector of its own, 25 L1 wavefronts per instruction), and to the
-// observation as floats, lane l taking bytes l + 32 j so that every store instruction covers 128 consecutive bytes.
+// K1a': one warp per (environment, warehouse) row - order quantities, arrivals, the new orders into the ring, pipeline
+// block of the observation row; the row's inbound cost goes to cost_rows.
+// The ring is indexed by placement time (marlsc_env_state): at step t plane (t - a) % L holds the orders placed a steps
+// ago, age a = 1 .. L (age L is plane t % L, the one this step overwrites). A cell with lead l receives its order of age
+// l, and pipeline slot k of the observation (what arrives at t + 1 + k, multi_env.py:941-968) is its order of age
+// l - 1 - k, the new one being age 0, or 0 for k >= l.
+// Loads: lane q reads the four consecutive cells 4q .. 4q+3 of the row in each of the L planes (vector loads, all in
+// flight at once). The (age, byte) pairs are then scattered to an image of the pipeline block in shared memory, [L][S] in
+// slot order, that L scratch slots precede: age a of a cell goes to slot l - 1 - a, so the ages that are no longer in
+// transit land in the scratch and slot -1 receives the arrival. Only the new orders go back to the ring - one 32-bit
+// word per lane into plane t % L, a contiguous W x S block per environment - and the image goes to the observation as
+// floats, lane l taking bytes l + 32 j so that every store instruction covers 128 consecutive bytes.
 // POLICY: the base-stock heuristic evaluated in place of given actions (its own instantiation: the extra live values cost
 // the ordinary one a resident CTA per SM)
 // LT: the lead-time horizon L as a compile-time constant (1..16; the plane loops then unroll without predicates: the
@@ -229,7 +237,7 @@ __global__ void __launch_bounds__(256)
 compact_place_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__ marlsc_env_state_t st,
                      const __grid_constant__ marlsc_step_io_t io, double* __restrict__ cost_rows, int t,
                      const __grid_constant__ marlsc_episode_metrics_t m) {
-  extern __shared__ __align__(16) unsigned char smem[];           // [8 warps][L * S] row images
+  extern __shared__ __align__(16) unsigned char smem[];           // [8 warps][2L * S]: L scratch slots, then the L pipeline slots
   constexpr int KMAX = LT ? LT : kCompactMaxL;
   const int W = sp.W, S = sp.S, L = LT ? LT : sp.L, WS = W * S;
   const int lane = threadIdx.x & 31;
@@ -240,68 +248,83 @@ compact_place_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
   const int64_t e = eu;
   const bool mine = 4 * lane < S;
   const int c4 = mine ? lane : 0;
-  const int S4 = S >> 2, pa = t % L;
-  // 32-bit word offset of pipeline slot k's plane inside the ring row: plane (t + 1 + k) % L, walked with one add per slot
-  const int LS4 = L * S4;
-  int po0 = (pa + 1) * S4;
-  po0 = po0 == LS4 ? 0 : po0;
-  uint32_t* const row4 = reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(st.ring_qty) + (e * WS + (int64_t)w * S) * L) + c4;
+  // 32-bit word offsets inside the ring: plane p of the row is p * WS4 words from the row's word in plane 0
+  const int WS4 = WS >> 2, LWS4 = L * WS4, po_new = (t % L) * WS4;
+  uint32_t* const row4 = reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(st.ring_qty) + e * L * WS + (int64_t)w * S) + c4;
   // every load of the row first
   float4 a4 = make_float4(0.f, 0.f, 0.f, 0.f);
-  uint32_t aqw = 0u, arr4 = 0u, le4 = 0x01010101u;
+  uint32_t aqw = 0u, le4 = 0x01010101u;
   uint2 iv = make_uint2(0u, 0u);
   uint2* const inv4 = reinterpret_cast<uint2*>(static_cast<uint16_t*>(st.inventory) + e * WS + w * S) + c4;
-  uint32_t x[KMAX > 1 ? KMAX - 1 : 1];
+  uint32_t x[KMAX];                                   // x[a - 1]: the four cells' orders of age a
   if (mine) {
     if (io.action_qty) aqw = reinterpret_cast<const uint32_t*>(io.action_qty + e * WS + w * S)[c4];
     else if (io.actions) a4 = reinterpret_cast<const float4*>(io.actions + e * WS + w * S)[c4];
     iv = *inv4;
-    arr4 = row4[pa * S4];
     le4 = reinterpret_cast<const uint32_t*>(sp.lead_u8 + w * S)[c4];
-    int po = po0;
+    int po = po_new;
 #pragma unroll
-    for (int k = 0; k < KMAX - 1; ++k)
-      if (k < L - 1) {
-        x[k] = row4[po];
-        po += S4;
-        po = po == LS4 ? 0 : po;
+    for (int a = 1; a <= KMAX; ++a)
+      if (a <= L) {                                   // plane (t - a) % L, walked with one subtraction per age
+        po = (po == 0 ? LWS4 : po) - WS4;
+        x[a - 1] = row4[po];
       }
   }
   constexpr bool policy = POLICY;                     // base-stock heuristic in place of given actions (marlsc_step_io.base_stock_level)
   float4 lv4 = make_float4(0.f, 0.f, 0.f, 0.f);
   if (policy && mine)
     lv4 = reinterpret_cast<const float4*>(io.base_stock_level + (io.base_stock_per_env ? e * WS : 0) + w * S)[c4];
-  const uint32_t img = sm_addr(smem) + (threadIdx.x >> 5) * (uint32_t)(L * S);   // this warp's row image, slot-major
+  const uint32_t img = sm_addr(smem) + (threadIdx.x >> 5) * (uint32_t)(2 * L * S) + (uint32_t)(L * S);   // pipeline slot 0
+  const uint32_t col = img + 4u * (uint32_t)lane;     // the lane's four cells in slot 0
+  uint32_t arr4 = 0u;
   if (mine) {
+    // slots at or past a cell's lead hold nothing: zero the lane's word of every slot, then scatter ages 1 .. L
 #pragma unroll
-    for (int k = 0; k < KMAX - 1; ++k)
-      if (k < L - 1) asm volatile("st.shared.u32 [%0], %1;" ::"r"(img + (uint32_t)(k * S + 4 * lane)), "r"(x[k]) : "memory");
-    asm volatile("st.shared.u32 [%0], %1;" ::"r"(img + (uint32_t)((L - 1) * S + 4 * lane)), "r"(0u) : "memory");
+    for (int k = 0; k < KMAX; ++k)
+      if (k < L) asm volatile("st.shared.u32 [%0], %1;" ::"r"(col + (uint32_t)(k * S)), "r"(0u) : "memory");
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int le = (int)((le4 >> (8 * j)) & 0xffu);
+      uint32_t adr = col + (uint32_t)((le - 2) * S + j);                  // slot le - 1 - a of age a = 1
+#pragma unroll
+      for (int a = 1; a <= KMAX; ++a)
+        if (a <= L) {
+          asm volatile("st.shared.u8 [%0], %1;" ::"r"(adr), "r"(x[a - 1] >> (8 * j)) : "memory");
+          adr -= (uint32_t)S;
+        }
+    }
+    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(arr4) : "r"(col - (uint32_t)S));   // slot -1: the arrivals (age = lead)
   }
   float af[4] = {a4.x, a4.y, a4.z, a4.w};
   const uint32_t ivv[4] = {iv.x & 0xffffu, iv.x >> 16, iv.y & 0xffffu, iv.y >> 16};
   if (policy && mine) {
     // reference make_bs_newsvendor_action_fn (run_baselines.py:188-207): order up to the level given on-hand stock and
-    // everything in transit - every plane of the ring, the arrivals of this step included (the policy acts before them)
+    // everything in transit - ages 1 .. lead, the arrivals of this step included (the policy acts before them). Summed
+    // from the registers, four cells at a time: byte b of (leads | 0x80 per byte) - a keeps its top bit exactly when
+    // lead_b >= a (leads <= 16, no borrow crosses a byte), and the sign-replicating byte permute turns that bit into the
+    // byte's mask. Bytes 0, 2 and 1, 3 add up in 16-bit halves (at most 16 x 255).
+    uint32_t p02 = 0u, p13 = 0u;
+#pragma unroll
+    for (int a = 1; a <= KMAX; ++a)
+      if (a <= L) {
+        const uint32_t v = x[a - 1] & byte_signs((le4 | 0x80808080u) - 0x01010101u * (uint32_t)a);
+        p02 += __byte_perm(v, 0u, 0x4240u);
+        p13 += __byte_perm(v, 0u, 0x4341u);
+      }
+    const uint32_t pend[4] = {p02 & 0xffffu, p13 & 0xffffu, p02 >> 16, p13 >> 16};
     const float lv[4] = {lv4.x, lv4.y, lv4.z, lv4.w};
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-      uint32_t pend = (arr4 >> (8 * j)) & 0xffu;
-#pragma unroll
-      for (int k = 0; k < KMAX - 1; ++k)
-        if (k < L - 1) pend += (x[k] >> (8 * j)) & 0xffu;
       const double mxd = sp.action_max[4 * lane + j];
-      double qd = (double)lv[j] - (double)ivv[j] - (double)pend;
+      double qd = (double)lv[j] - (double)ivv[j] - (double)pend[j];
       qd = qd < 0.0 ? 0.0 : (qd > mxd ? mxd : qd);
       af[j] = (float)(2.0 * qd / mxd - 1.0);
     }
   }
-  uint32_t ni[4];
+  uint32_t ni[4], qw = 0u;
   int nQ = 0, nPos = 0;
   double inb = 0.0;
   const bool by_row = sp.row_rates_uniform != 0;
-  __syncwarp();                                       // a cell's slot may lie in a word another lane has just written? no: own words only,
-                                                      // but the byte stores below must follow this lane's word stores in program order
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
     const int le = (int)((le4 >> (8 * j)) & 0xffu);
@@ -309,8 +332,9 @@ compact_place_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
     if (mine) {
       const int mxj = (int)sp.action_max[4 * lane + j];
       q = io.action_qty ? imin((int)((aqw >> (8 * j)) & 0xffu), mxj) : rescale_action<kCapsLean>(sp, af[j], (double)mxj, 0, 0);
-      if (q > 0) asm volatile("st.shared.u8 [%0], %1;" ::"r"(img + (uint32_t)((le - 1) * S + 4 * lane + j)), "r"(q) : "memory");
+      if (q > 0) asm volatile("st.shared.u8 [%0], %1;" ::"r"(col + (uint32_t)((le - 1) * S + j)), "r"(q) : "memory");   // age 0
     }
+    qw |= (uint32_t)q << (8 * j);
     ni[j] = ivv[j] + ((arr4 >> (8 * j)) & 0xffu);
     nQ += q;
     nPos += q > 0 ? 1 : 0;
@@ -321,6 +345,7 @@ compact_place_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
   }
   if (mine) {
     *inv4 = make_uint2(ni[0] | (ni[1] << 16), ni[2] | (ni[3] << 16));
+    row4[po_new] = qw;                                // every cell, 0 included: the plane held the orders of age L
   }
   if (by_row) {
     nQ = __reduce_add_sync(FULL, nQ);
@@ -339,18 +364,6 @@ compact_place_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__
     }
   }
   __syncwarp();                                       // image complete
-  if (mine) {                                         // the ring row, every plane as whole words
-    int po = po0;
-#pragma unroll
-    for (int k = 0; k < KMAX; ++k)
-      if (k < L) {
-        uint32_t v;
-        asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(img + (uint32_t)(k * S + 4 * lane)));
-        row4[po] = v;                                 // slot L-1 is the arrival plane
-        po += S4;
-        po = po == LS4 ? 0 : po;
-      }
-  }
   // the pipeline block of the observation row
   const float* const mean_l = MS ? sp.obs_mean + sp.off_pipe + lane : nullptr;
   const float* const istd_l = MS ? sp.obs_std + sp.off_pipe + lane : nullptr;
@@ -682,8 +695,8 @@ env_reset_compact_kernel(const __grid_constant__ DevSpec sp, const __grid_consta
   const int i = (int)(idx - e * WS), w = i / S, s = i - w * S;
   const int v = init[per_env ? idx : i];
   static_cast<uint16_t*>(st.inventory)[idx] = (uint16_t)(v < 0 ? 0 : (v > 65535 ? 65535 : v));
-  uint8_t* ring = static_cast<uint8_t*>(st.ring_qty) + (e * WS + (long long)w * S) * L + s;
-  for (int d = 0; d < L; ++d) ring[d * S] = 0;
+  uint8_t* ring = static_cast<uint8_t*>(st.ring_qty) + e * L * WS + i;
+  for (int d = 0; d < L; ++d) ring[(long long)d * WS] = 0;
   if (st.demand_hist) {
     uint16_t* h = static_cast<uint16_t*>(st.demand_hist) + e * (long long)kWindow * WS + i;
     for (int b = 0; b < kWindow; ++b) h[b * WS] = 0;
@@ -705,23 +718,24 @@ env_reset_compact_kernel(const __grid_constant__ DevSpec sp, const __grid_consta
   }
 }
 
-// K5 (compact): units in transit to a cell are the sum of its ring column (every plane is an arrival still to come).
+// K5 (compact): units in transit to a cell are its orders of age 1 .. l (l its lead, the arrivals of step t included):
+// plane (t - a) % L of the placement-indexed ring for a = 1 .. l.
 template <typename IDX>
 __global__ void __launch_bounds__(256)
 base_stock_compact_kernel(const __grid_constant__ DevSpec sp, const __grid_constant__ marlsc_env_state_t st,
-                          const float* __restrict__ level, int level_per_env, float* __restrict__ actions) {
+                          const float* __restrict__ level, int level_per_env, int t, float* __restrict__ actions) {
   const IDX WS = (IDX)(sp.W * sp.S);
   const IDX idx = (IDX)blockIdx.x * (IDX)blockDim.x + (IDX)threadIdx.x;
   if (idx >= (IDX)st.num_envs * WS) return;
   const IDX e = idx / WS;
-  const int i = (int)(idx - e * WS), w = i / sp.S, s = i - w * sp.S;
-  const int L = sp.L;
-  const uint8_t* ring = static_cast<const uint8_t*>(st.ring_qty) + ((long long)e * (long long)WS + (long long)w * sp.S) * L + s;
+  const int i = (int)(idx - e * WS), s = i % sp.S;
+  const int L = sp.L, lead = sp.lead_u8[i], tl = t % L + L;            // age a <= L lives in plane (tl - a) % L
+  const uint8_t* ring = static_cast<const uint8_t*>(st.ring_qty) + (long long)e * L * (long long)WS + i;
   int pending = 0;
-  for (int d0 = 0; d0 < L; d0 += 4) {
+  for (int a0 = 1; a0 <= lead; a0 += 4) {
     int v[4];
 #pragma unroll
-    for (int k = 0; k < 4; ++k) v[k] = d0 + k < L ? (int)ring[(d0 + k) * sp.S] : 0;
+    for (int k = 0; k < 4; ++k) v[k] = a0 + k <= lead ? (int)ring[(long long)((tl - a0 - k) % L) * (long long)WS] : 0;
     pending += (v[0] + v[1]) + (v[2] + v[3]);
   }
   const double mx = sp.action_max[s];
@@ -882,7 +896,7 @@ int launch_split_nch(const LaunchArgs& a, const marlsc_step_io_t& io, const Spli
   if (wk.marks) MARLSC_CUDA(cudaEventRecord(wk.marks[0], s));
   {
     const bool policy = !io.actions && !io.action_qty;
-    const size_t img = (size_t)8 * a.ds.L * a.ds.S;
+    const size_t img = (size_t)8 * 2 * a.ds.L * a.ds.S;   // per warp: L scratch slots and the L pipeline slots
 #define MARLSC_PLACE_L(LT)                                                                                          \
   case LT:                                                                                                          \
     if (policy) compact_place_kernel<MS, true, LT><<<grid_rows, 256, img, s>>>(a.ds, a.st, io, wk.cost_rows, t, m);  \
@@ -960,11 +974,10 @@ int launch_reset_compact(const LaunchArgs& a, const int32_t* init, int per_env, 
 
 int launch_base_stock_compact(const DevSpec& ds, const marlsc_env_state_t& st, const float* level, int level_per_env, int t,
                               float* actions, cudaStream_t s) {
-  (void)t;
   const long long n = st.num_envs * (long long)ds.W * ds.S;
   const unsigned grid = (unsigned)((n + 255) / 256);
-  if (n < (1LL << 32)) base_stock_compact_kernel<unsigned><<<grid, 256, 0, s>>>(ds, st, level, level_per_env, actions);
-  else base_stock_compact_kernel<long long><<<grid, 256, 0, s>>>(ds, st, level, level_per_env, actions);
+  if (n < (1LL << 32)) base_stock_compact_kernel<unsigned><<<grid, 256, 0, s>>>(ds, st, level, level_per_env, t, actions);
+  else base_stock_compact_kernel<long long><<<grid, 256, 0, s>>>(ds, st, level, level_per_env, t, actions);
   g_launches.fetch_add(1, std::memory_order_relaxed);
   MARLSC_CUDA(cudaGetLastError());
   return MARLSC_OK;

@@ -7,11 +7,14 @@
 // the three kernels issued 27 k warp instructions per env-step - 70 % of the row kernels' were address arithmetic of the
 // per-cell ring gather - and moved 154 KB per env-step, 44 KB of it the int32 ring):
 //
-//   * state in the width the values need - on-hand stock and home-demand history uint16, in-transit ring uint8 - and the
-//     ring indexed by ARRIVAL time: an order placed at t with (fixed) lead l goes to plane (t + l) % L of its warehouse
-//     row, ring[e][w][d][s]. Arrivals of step t are plane t % L for every cell and pipeline slot k of the observation
-//     (multi_env.py:941-968) is plane (t + 1 + k) % L for every cell: both are plain row copies, no per-cell plane
-//     arithmetic. The only scattered access left is the single byte a new order writes.
+//   * state in the width the values need - on-hand stock and home-demand history uint16, in-transit ring uint8
+//     ring[e][d][w][s] indexed by PLACEMENT time like the wide one: the orders placed at t are plane t % L. The ring was
+//     first indexed by arrival time (an order placed at t with lead l in plane (t + l) % L of its warehouse row), which
+//     made the arrivals and the pipeline slots of the observation plain row copies. But with a lead per cell one step's
+//     orders land in every plane of a row, and single-byte stores dirty whole sectors, so K1a' wrote the row's L x S
+//     bytes back to record S new ones: 10 KB per env-step at the large config. Indexed by placement time a step writes
+//     one contiguous W x S plane per environment (1 KB); K1a' loads every plane of a row anyway, and finds the per-cell
+//     ages of the arrivals and the pipeline slots in shared memory (multi_env.py:941-968).
 //   * demand as sparse "lines" (marlsc_step_io.lines): the non-zero (order, SKU) cells, pre-sorted into 32 streams by
 //     SKU % 32. Lane l walks stream l - no pass over 80 %-zero dense rows, no shuffles, 2 bytes per line instead of
 //     S + 2 bytes per order.

@@ -4,7 +4,8 @@ timestep (csrc/env_step.cu, csrc/env_compact.cu). Tensor-in / tensor-out counter
 the reference is provided on top of it by ``marlsc_b200.envs.InventoryEnvironment``.
 
 State is struct-of-arrays on the device, env-major (include/marlsc_b200.h ``marlsc_env_state``):
-``inventory [E,W,S]``, ``ring_qty [E,D,W,S]`` (+ ``ring_lead`` for stochastic lead times),
+``inventory [E,W,S]``, ``ring_qty [E,D,W,S]`` indexed by placement time (D = L on the compact layout;
++ ``ring_lead`` for stochastic lead times),
 ``demand_hist [E,5,W,S]``, ``forecast [E,W,S]``. Observations are written once per warehouse as
 ``obs [E,W,obs_dim]``; flattened over W this *is* the centralised-critic global state, so the
 reference's per-agent ``[local_i | global]`` vector is only materialised on request
@@ -159,10 +160,12 @@ class BatchedInventoryEnv:
         E, W, S, D, dev = self.num_envs, self.n_warehouses, self.n_skus, self.ring_depth, self.device
         if self.layout == "compact":
             # uint16 stock / history (int16 storage: values stay below 32768, see _stock_bound), uint8 ring indexed by
-            # arrival time: ring_qty[e, w, a % L, s] holds the order arriving at step a
+            # placement time like the wide one: ring_qty[e, tau % L, w, s] holds the order placed at step tau. Fixed lead
+            # times make the ring depth the longest lead, which pending_matrix relies on.
             Lm = self.max_expected_lead_time
+            assert D == Lm, "the compact layout's ring depth is the longest lead time"
             self.inventory = torch.zeros((E, W, S), dtype=torch.int16, device=dev)
-            self.ring_qty = torch.zeros((E, W, Lm, S), dtype=torch.uint8, device=dev)
+            self.ring_qty = torch.zeros((E, Lm, W, S), dtype=torch.uint8, device=dev)
             self.ring_lead = None
             self.demand_hist = (torch.zeros((E, 5, W, S), dtype=torch.int16, device=dev)
                                 if L.marlsc_env_needs_history(self._h) else None)
@@ -393,8 +396,11 @@ class BatchedInventoryEnv:
             h.update(f"{k}:{None if arr is None else (arr.dtype.str, arr.shape)};".encode())
             if arr is not None:
                 h.update(np.ascontiguousarray(arr).tobytes())
-        return dict(num_envs=self.num_envs, layout=self.layout, spec=h.hexdigest(), episode_metrics=bool(self._metrics),
-                    device_demand=self._dd is not None, device_leads=self._dl is not None, host_samplers=bool(self._host_samplers))
+        fp = dict(num_envs=self.num_envs, layout=self.layout, spec=h.hexdigest(), episode_metrics=bool(self._metrics),
+                  device_demand=self._dd is not None, device_leads=self._dl is not None, host_samplers=bool(self._host_samplers))
+        if self.layout == "compact":   # its ring was once [E,W,L,S] by arrival time: same shape when W = L, other contents
+            fp["ring_qty"] = "uint8 [E,L,W,S] by placement time"
+        return fp
 
     def state_dict(self) -> Dict[str, Any]:
         """Everything that decides this environment's future, copied to the host: the device state, observations,
@@ -429,6 +435,9 @@ class BatchedInventoryEnv:
             if (dst is None) != (src is None):
                 raise ValueError(f"environment snapshot does not match this environment: {k} is present in only one of them")
             if dst is not None:
+                if tuple(dst.shape) != tuple(src.shape):
+                    raise ValueError(f"environment snapshot does not match this environment: {k} has shape "
+                                     f"{tuple(src.shape)} in the snapshot and {tuple(dst.shape)} here")
                 dst.copy_(src)
         for k, v in self._metrics.items():
             v.copy_(sd["metrics"][k])
@@ -527,8 +536,6 @@ class BatchedInventoryEnv:
 
     def pending_matrix(self) -> torch.Tensor:
         """Units in transit per (env, warehouse, SKU) (reference ``_compute_pending_matrix``)."""
-        if self.layout == "compact":      # every plane of the arrival-indexed ring is an order still on its way
-            return self.ring_qty.sum(dim=2, dtype=torch.int32).to(torch.float32)
         t = self.timestep
         D = self.ring_depth
         tau = torch.tensor([t - 1 - ((t - 1 - d) % D) for d in range(D)], device=self.device).view(1, D, 1, 1)
