@@ -391,9 +391,19 @@ int marlsc_gae(const float* rewards, const float* values, const uint8_t* cut, co
                int32_t T, int64_t N, float gamma, float lam, float* adv, float* targets, void* stream);
 
 /* Per-policy advantage standardisation (x - mean) / max(1e-4, std) in place over n values
- * (RLlib learner connector). workspace: device, >= marlsc_standardize_workspace_bytes(). */
+ * (RLlib learner connector). workspace: device, >= marlsc_standardize_workspace_bytes().
+ * marlsc_standardize is marlsc_standardize_moments followed by marlsc_standardize_apply. */
 size_t marlsc_standardize_workspace_bytes(void);
 int marlsc_standardize(float* x, int64_t n, void* workspace, void* stream);
+
+/* The two halves of marlsc_standardize, for data-parallel callers whose ranks standardise over all their values together.
+ * marlsc_standardize_moments zeroes the workspace and writes three float64 values at its start:
+ *   { sum of x, sum of x^2, n }
+ * A caller may sum these 24 bytes over its ranks (an all-reduce) before marlsc_standardize_apply, which computes
+ * mean = sum / count and std = sqrt(max(0, sumsq / count - mean^2)) from the workspace (the count included, so it may
+ * differ from the n of this call) and writes (x - mean) / max(1e-4, std) over the n values of x. */
+int marlsc_standardize_moments(const float* x, int64_t n, void* workspace, void* stream);
+int marlsc_standardize_apply(float* x, int64_t n, const void* workspace, void* stream);
 
 /* K7 - forward pass of a one-hidden-layer MLP head over every agent-sample of a rollout step (reference:
  * ActorCriticRLModule._forward_actor / _forward_critic over an "mlp" network with one hidden layer,

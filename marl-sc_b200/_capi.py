@@ -161,6 +161,10 @@ def lib() -> C.CDLL:
     L.marlsc_standardize_workspace_bytes.restype = C.c_size_t
     L.marlsc_standardize.argtypes = [vp, i64, vp, vp]
     L.marlsc_standardize.restype = C.c_int
+    L.marlsc_standardize_moments.argtypes = [vp, i64, vp, vp]
+    L.marlsc_standardize_moments.restype = C.c_int
+    L.marlsc_standardize_apply.argtypes = [vp, i64, vp, vp]
+    L.marlsc_standardize_apply.restype = C.c_int
     L.marlsc_last_error.argtypes = []
     L.marlsc_last_error.restype = C.c_char_p
     L.marlsc_abi_version.argtypes = []

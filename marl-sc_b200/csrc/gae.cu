@@ -66,9 +66,11 @@ gae_kernel(const float* __restrict__ rewards, const float* __restrict__ values, 
   }
 }
 
-// ---- standardisation: sum and sum of squares in double, then (x - mean) / max(1e-4, std) -----------
+// ---- standardisation: sum, sum of squares and count in double, then (x - mean) / max(1e-4, std) -----
+// The three doubles are the workspace's public layout (include/marlsc_b200.h): a data-parallel caller sums them over
+// its ranks between the two kernels.
 struct StdWs {
-  double sum, sumsq;
+  double sum, sumsq, count;
 };
 
 __global__ void __launch_bounds__(256) moments_kernel(const float* __restrict__ x, long long n, StdWs* ws) {
@@ -98,17 +100,23 @@ __global__ void __launch_bounds__(256) moments_kernel(const float* __restrict__ 
     }
     atomicAdd(&ws->sum, a);
     atomicAdd(&ws->sumsq, b);
+    if (blockIdx.x == 0) ws->count = (double)n;
   }
 }
 
 __global__ void __launch_bounds__(256) standardize_kernel(float* __restrict__ x, long long n, const StdWs* __restrict__ ws) {
-  const double mean = ws->sum / (double)n;
-  double var = ws->sumsq / (double)n - mean * mean;
+  const double mean = ws->sum / ws->count;
+  double var = ws->sumsq / ws->count - mean * mean;
   if (var < 0.0) var = 0.0;
   const float m = (float)mean;
   const float sd = fmaxf(1e-4f, (float)sqrt(var));
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
     x[i] = (x[i] - m) / sd;
+}
+
+unsigned std_grid(long long n) {
+  const long long want = (n + 255) / 256;
+  return (unsigned)(want < 148 * 8 ? want : 148 * 8);
 }
 
 }  // namespace
@@ -131,19 +139,29 @@ int marlsc_gae(const float* rewards, const float* values, const uint8_t* cut, co
 
 size_t marlsc_standardize_workspace_bytes(void) { return sizeof(StdWs); }
 
-int marlsc_standardize(float* x, int64_t n, void* workspace, void* stream) {
+int marlsc_standardize_moments(const float* x, int64_t n, void* workspace, void* stream) {
   if (!x || !workspace) return set_error(MARLSC_EINVAL, "x and workspace must not be NULL");
   if (n < 1) return set_error(MARLSC_EINVAL, "n must be positive");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   MARLSC_CUDA(cudaMemsetAsync(workspace, 0, sizeof(StdWs), s));
-  const int block = 256;
-  long long want = (n + block - 1) / block;
-  const unsigned grid = (unsigned)(want < 148 * 8 ? want : 148 * 8);
-  moments_kernel<<<grid, block, 0, s>>>(x, n, static_cast<StdWs*>(workspace));
-  standardize_kernel<<<grid, block, 0, s>>>(x, n, static_cast<const StdWs*>(workspace));
-  g_launches.fetch_add(2, std::memory_order_relaxed);
+  moments_kernel<<<std_grid(n), 256, 0, s>>>(x, n, static_cast<StdWs*>(workspace));
+  g_launches.fetch_add(1, std::memory_order_relaxed);
   MARLSC_CUDA(cudaGetLastError());
   return MARLSC_OK;
+}
+
+int marlsc_standardize_apply(float* x, int64_t n, const void* workspace, void* stream) {
+  if (!x || !workspace) return set_error(MARLSC_EINVAL, "x and workspace must not be NULL");
+  if (n < 1) return set_error(MARLSC_EINVAL, "n must be positive");
+  standardize_kernel<<<std_grid(n), 256, 0, static_cast<cudaStream_t>(stream)>>>(x, n, static_cast<const StdWs*>(workspace));
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  MARLSC_CUDA(cudaGetLastError());
+  return MARLSC_OK;
+}
+
+int marlsc_standardize(float* x, int64_t n, void* workspace, void* stream) {
+  const int rc = marlsc_standardize_moments(x, n, workspace, stream);
+  return rc != MARLSC_OK ? rc : marlsc_standardize_apply(x, n, workspace, stream);
 }
 
 }  // extern "C"

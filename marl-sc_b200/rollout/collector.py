@@ -3,7 +3,9 @@ GAE scan kernel. Replaces RLlib's EnvRunner / MultiAgentEpisode / learner-connec
 reference configures (reference: src/algorithms/ippo.py:145-214, mappo.py:142-209; SURVEY.md A17-A18).
 
 Buffers are time-major and preallocated; the env writes observations and rewards straight into them.
-Environments never interact, so a multi-GPU run shards them by rank with no communication here.
+Environments never interact, so a multi-GPU run shards them by rank and steps them with no communication. With a
+``process_group`` the collector standardises the advantages over every rank's batch and merges the ranks' observation
+filter moments after each collection.
 """
 from __future__ import annotations
 
@@ -11,6 +13,7 @@ from dataclasses import dataclass
 from typing import Callable, Optional, Union
 
 import torch
+import torch.distributed as dist
 
 from ..envs import BatchedInventoryEnv, DeviceOrders
 from .gae import compute_gae, standardize_, standardize_columns_
@@ -48,7 +51,7 @@ class RolloutCollector:
     def __init__(self, env: BatchedInventoryEnv, policy: Union[ActorCritic, CentralizedActorCritic], horizon: int,
                  gamma: float = 0.99, lam: float = 0.95, demand_fn: Optional[Callable[[int], DeviceOrders]] = None,
                  standardize_advantages: bool = True, seed: int = 0, keep_dist_inputs: bool = False,
-                 obs_filter=None):
+                 obs_filter=None, process_group=None):
         self.env, self.policy, self.T = env, policy, int(horizon)
         self.gamma, self.lam = float(gamma), float(lam)
         self.demand_fn = demand_fn            # step index -> DeviceOrders; None = env host samplers
@@ -56,6 +59,10 @@ class RolloutCollector:
         # running MeanStdFilter (obs_normalization == "meanstd"), applied in place: per local column shared by the agents,
         # or, for the centralised policy, per global column over the [E, W*D] view
         self.obs_filter = obs_filter
+        # data parallel: advantage moments all-reduced, filter buffers gathered and merged in rank order after collect()
+        self.group = process_group if process_group is not None and dist.get_world_size(process_group) > 1 else None
+        if self.group is not None and obs_filter is not None:
+            obs_filter.track_buffer()
         E, W, S, D, dev = env.num_envs, env.n_warehouses, env.n_skus, env.obs_dim, env.device
         T = self.T
         central = isinstance(policy, CentralizedActorCritic)
@@ -126,9 +133,11 @@ class RolloutCollector:
             # RLlib standardises the advantages per module batch: over everything with a shared policy, per
             # warehouse column with independent policies
             if pol.n_policies == 1:
-                standardize_(self.adv)
+                standardize_(self.adv, self.group)
             else:
-                standardize_columns_(self.adv, pol.n_policies)
+                standardize_columns_(self.adv, pol.n_policies, self.group)
+        if self.group is not None and flt is not None:
+            flt.sync(self.group)
         ls_old = pol.clamped_log_std().detach().reshape(pol.n_policies, -1).clone() if self.mean_old is not None else None
         return Rollout(self.obs, self.actions, self.logp, self.rewards, self.values, self.adv, self.targets, cut,
                        self.mean_old, ls_old)

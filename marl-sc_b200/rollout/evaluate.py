@@ -10,6 +10,7 @@ from typing import Callable, Dict, Optional, Union
 
 import numpy as np
 import torch
+import torch.distributed as dist
 
 from ..envs import BatchedInventoryEnv
 from ..envs.batched_env import COST_METRICS, METRICS_PER_ENV, METRICS_PER_ROW, fill_rate
@@ -40,6 +41,31 @@ class EpisodeMetrics:
         summed units."""
         x = self.values[name]
         return x if x.dim() == 2 else x.sum(-1)
+
+    def gather(self, group=None) -> "EpisodeMetrics":
+        """Every rank's metrics of ``group`` (default: the default process group) joined along the environment axis in rank
+        order, on every rank; the ranks may hold different numbers of environments. One all-reduce."""
+        world, rank = dist.get_world_size(group), dist.get_rank(group)
+        names = list(self.values)
+        first = self.values[names[0]]
+        E = first.shape[1]
+        dev = first.device
+        sizes = torch.zeros(world, dtype=torch.float64, device=dev)
+        sizes[rank] = E
+        dist.all_reduce(sizes, op=dist.ReduceOp.SUM, group=group)
+        sizes = [int(n) for n in sizes.tolist()]
+        off = sum(sizes[:rank])
+        # [E, ...] per metric -> one [E, F] row block per rank; the other ranks' rows stay 0, so the sum is a gather
+        cols = [self.values[k].movedim(1, 0).reshape(E, -1).to(torch.float64) for k in names]
+        rows = torch.zeros((sum(sizes), sum(c.shape[1] for c in cols)), dtype=torch.float64, device=dev)
+        rows[off:off + E] = torch.cat(cols, dim=1)
+        dist.all_reduce(rows, op=dist.ReduceOp.SUM, group=group)
+        out, c0 = {}, 0
+        for k, c in zip(names, cols):
+            v = self.values[k]
+            out[k] = rows[:, c0:c0 + c.shape[1]].reshape(sum(sizes), v.shape[0], *v.shape[2:]).movedim(0, 1).to(v.dtype).contiguous()
+            c0 += c.shape[1]
+        return EpisodeMetrics(out)
 
     def summary(self) -> Dict[str, Dict[str, float]]:
         """Mean and (population) standard deviation of every metric over all environments of all episodes, one sample per

@@ -8,6 +8,7 @@ from __future__ import annotations
 from typing import Optional, Tuple
 
 import torch
+import torch.distributed as dist
 
 from .. import _capi
 
@@ -54,25 +55,47 @@ def compute_gae(rewards: torch.Tensor, values: torch.Tensor, gamma: float, lam: 
 _ws = {}
 
 
-def standardize_(x: torch.Tensor) -> torch.Tensor:
-    """In place (x - mean) / max(1e-4, std) over all elements of a float32 CUDA tensor."""
+def _spans_ranks(group) -> bool:
+    return group is not None and dist.get_world_size(group) > 1
+
+
+def standardize_(x: torch.Tensor, group=None) -> torch.Tensor:
+    """In place (x - mean) / max(1e-4, std) over all elements of a float32 CUDA tensor. With a process ``group`` of more
+    than one rank the moments are those of every rank's ``x`` together: K3's moments kernel, one all-reduce of its three
+    float64 sums (sum, sum of squares, count), then K3's apply kernel."""
     if not x.is_cuda or x.dtype != torch.float32 or not x.is_contiguous():
         raise ValueError("standardize_ needs a contiguous float32 CUDA tensor")
     L = _capi.lib()
     ws = _ws.get(x.device)
     if ws is None:
         ws = _ws[x.device] = torch.zeros(max(16, int(L.marlsc_standardize_workspace_bytes())), dtype=torch.uint8, device=x.device)
-    _capi.check(L.marlsc_standardize(x.data_ptr(), x.numel(), ws.data_ptr(), _stream(x)))
+    if not _spans_ranks(group):
+        _capi.check(L.marlsc_standardize(x.data_ptr(), x.numel(), ws.data_ptr(), _stream(x)))
+        return x
+    _capi.check(L.marlsc_standardize_moments(x.data_ptr(), x.numel(), ws.data_ptr(), _stream(x)))
+    dist.all_reduce(ws[:24].view(torch.float64), op=dist.ReduceOp.SUM, group=group)
+    _capi.check(L.marlsc_standardize_apply(x.data_ptr(), x.numel(), ws.data_ptr(), _stream(x)))
     return x
 
 
-def standardize_columns_(x: torch.Tensor, n_columns: int) -> torch.Tensor:
+def standardize_columns_(x: torch.Tensor, n_columns: int, group=None) -> torch.Tensor:
     """In place ``(x - mean_c) / max(1e-4, std_c)`` per last-axis column c (one column per independent policy:
-    RLlib standardises the advantages of every module's batch on their own)."""
+    RLlib standardises the advantages of every module's batch on their own). With a process ``group`` of more than one
+    rank the per-column float64 sums, sums of squares and counts are all-reduced first, so every column is standardised
+    over all ranks' values."""
     if x.shape[-1] != n_columns:
         raise ValueError("the last axis must be the policy axis")
     flat = x.view(-1, n_columns)
-    mean = flat.mean(0)
-    std = flat.std(0, unbiased=False).clamp_min(1e-4)
-    flat.sub_(mean).div_(std)
+    if not _spans_ranks(group):
+        mean = flat.mean(0)
+        std = flat.std(0, unbiased=False).clamp_min(1e-4)
+        flat.sub_(mean).div_(std)
+        return x
+    x64 = flat.to(torch.float64)
+    m = torch.cat([x64.sum(0), (x64 * x64).sum(0), x64.new_full((n_columns,), float(flat.shape[0]))])
+    dist.all_reduce(m, op=dist.ReduceOp.SUM, group=group)
+    s, q, n = m.view(3, n_columns)
+    mean = s / n
+    std = torch.sqrt(torch.clamp(q / n - mean * mean, min=0.0)).clamp_min(1e-4)
+    flat.sub_(mean.to(flat.dtype)).div_(std.to(flat.dtype))
     return x

@@ -9,7 +9,31 @@ policy.
 """
 from __future__ import annotations
 
+from typing import Sequence, Tuple
+
 import torch
+import torch.distributed as dist
+
+Moments = Tuple[torch.Tensor, torch.Tensor, torch.Tensor]      # (count, mean, M2): float64 [], [D], [D]
+
+
+def chan_merge(a: Moments, b) -> Moments:
+    """The moments of the union of two sample sets (Chan et al.'s pairwise update); ``b``'s count may be a number. The two
+    sets must not both be empty."""
+    ca, ma, qa = a
+    cb, mb, qb = b
+    tot = ca + cb
+    delta = mb - ma
+    return tot, ma + delta * (cb / tot), qa + (qb + delta * delta * (ca * cb / tot))
+
+
+def merge_buffers(base: Moments, buffers: Sequence[Moments]) -> Moments:
+    """``base`` merged with every buffer in turn, in the order given (rank order in a data-parallel run, so that every
+    rank computes the same bits)."""
+    out = base
+    for b in buffers:
+        out = chan_merge(out, b)
+    return out
 
 
 class MeanStdFilter:
@@ -18,6 +42,9 @@ class MeanStdFilter:
         self.mean = torch.zeros(obs_dim, dtype=torch.float64, device=device)
         self.m2 = torch.zeros(obs_dim, dtype=torch.float64, device=device)
         self.eps, self.update = eps, update
+        # data-parallel runs (track_buffer): the moments at the last sync, and those added locally since
+        self.synced: Moments = None
+        self.buffer: Moments = None
 
     @torch.no_grad()
     def __call__(self, obs: torch.Tensor) -> torch.Tensor:
@@ -27,11 +54,9 @@ class MeanStdFilter:
             n = float(flat.shape[0])
             bm = flat.mean(0, dtype=torch.float64)
             bm2 = ((flat.to(torch.float64) - bm) ** 2).sum(0)
-            tot = self.count + n
-            delta = bm - self.mean
-            self.mean += delta * (n / tot)
-            self.m2 += bm2 + delta * delta * (self.count * n / tot)
-            self.count = tot
+            self.count, self.mean, self.m2 = chan_merge((self.count, self.mean, self.m2), (n, bm, bm2))
+            if self.buffer is not None:
+                self.buffer = chan_merge(self.buffer, (n, bm, bm2))
         std = torch.sqrt(self.m2 / torch.clamp(self.count - 1.0, min=1.0))
         flat.sub_(self.mean.to(obs.dtype)).div_((std + self.eps).to(obs.dtype))
         return obs
@@ -41,3 +66,29 @@ class MeanStdFilter:
 
     def load_state_dict(self, sd):
         self.count, self.mean, self.m2 = sd["count"].clone(), sd["mean"].clone(), sd["m2"].clone()
+        if self.buffer is not None:
+            self.track_buffer()
+
+    # ------------------------------------------------------------------ data-parallel runs
+    def track_buffer(self) -> None:
+        """From now on keep the moments this process adds apart (``buffer``) from those of the last sync (``synced``), the
+        way RLlib's ``MeanStdFilter`` keeps a buffer per env runner."""
+        self.synced = (self.count.clone(), self.mean.clone(), self.m2.clone())
+        self.buffer = (torch.zeros_like(self.count), torch.zeros_like(self.mean), torch.zeros_like(self.m2))
+
+    @torch.no_grad()
+    def sync(self, group=None) -> None:
+        """Gather every rank's buffer ``(count, mean, M2)`` and merge them, in rank order, into the moments of the last
+        sync; every rank then holds the same filter and starts an empty buffer. Needs ``track_buffer()``."""
+        if self.buffer is None:
+            raise RuntimeError("MeanStdFilter.sync needs track_buffer() first")
+        world, rank = dist.get_world_size(group), dist.get_rank(group)
+        D = self.mean.numel()
+        rows = torch.zeros((world, 2 * D + 1), dtype=torch.float64, device=self.mean.device)
+        rows[rank, 0] = self.buffer[0]
+        rows[rank, 1:D + 1] = self.buffer[1]
+        rows[rank, D + 1:] = self.buffer[2]
+        dist.all_reduce(rows, op=dist.ReduceOp.SUM, group=group)      # an all-gather: each row has one non-zero owner
+        bufs = [(r[0], r[1:D + 1], r[D + 1:]) for r in rows]
+        self.count, self.mean, self.m2 = merge_buffers(self.synced, bufs)
+        self.track_buffer()

@@ -278,7 +278,8 @@ class PPOLearner:
         """One learner update on a rollout: ``num_epochs`` passes, each over a fresh on-device permutation of the
         (timestep, environment) samples cut into ``num_minibatches`` minibatches (reference ippo.py:149-152:
         ``minibatch_size = batch_size // num_minibatches``, ``shuffle_batch_per_epoch=True``). All agents of a sample
-        stay together, so a minibatch is ``[B, W, ...]``. Adapts the KL coefficient afterwards when ``use_kl_loss``."""
+        stay together, so a minibatch is ``[B, W, ...]``. Adapts the KL coefficient afterwards when ``use_kl_loss``. With a
+        default process group of several ranks the statistics (and so the KL adaptation) are the means over the ranks."""
         E_ = ro.rewards.shape[1]
         T = ro.rewards.shape[0]
         n = T * E_
@@ -306,7 +307,14 @@ class PPOLearner:
                     break
             if max_minibatches is not None and steps >= max_minibatches:
                 break
-        res = {name: float(v) / steps for name, v in sums.items()}      # one device->host read per metric
+        if self.buckets._distributed():
+            # one all-reduce of the summed statistics: every rank reports the same means and adapts the same kl_coeff
+            names = list(sums)
+            tot = torch.stack([sums[k].to(torch.float64) for k in names])
+            dist.all_reduce(tot, op=dist.ReduceOp.SUM)
+            res = {name: v / steps for name, v in zip(names, (tot / dist.get_world_size()).tolist())}
+        else:
+            res = {name: float(v) / steps for name, v in sums.items()}      # one device->host read per metric
         if kl_on:
             if res["kl"] > 2.0 * self.kl_target:
                 self.kl_coeff *= 1.5

@@ -1,12 +1,19 @@
-"""Single-process training from an algorithm config: IPPO, MAPPO and CPPO on the device, with the config's learning-rate
-schedule, periodic evaluation, checkpoints and resume (the reference's ``run_experiment.py --mode single``,
-``ExperimentRunner.run``, runner.py:112-214).
+"""Training from an algorithm config: IPPO, MAPPO and CPPO on the device, with the config's learning-rate schedule, periodic
+evaluation, checkpoints and resume (the reference's ``run_experiment.py --mode single``, ``ExperimentRunner.run``,
+runner.py:112-214), on one GPU or data-parallel on several.
 
 One iteration is: set the learning rate, collect ``horizon`` steps of ``num_envs`` environments (``RolloutCollector``: K1 /
 K4 / K7 / K2 / K3), one ``PPOLearner.update`` (``num_epochs`` x ``num_minibatches`` K6 steps), every ``eval_interval``
 iterations ``evaluate()`` on a separate environment batch, and one JSON line in ``training_metrics.jsonl``. A checkpoint
 holds everything the next iteration depends on - model, optimiser, filter, generators, the collector's carried observation
-and both environments' ``state_dict()`` - so a resumed run continues the same trajectory."""
+and both environments' ``state_dict()`` - so a resumed run continues the same trajectory.
+
+Under a default process group of more than one rank (``torchrun``), every rank holds ``num_envs / world`` of the training
+environments and its shard of the evaluation environments, and the ranks agree on everything the single-GPU algorithm computes
+over the whole batch: the gradients (``GradBuckets``), the advantage standardisation and the ``meanstd`` filter
+(``RolloutCollector(process_group=...)``), the learner statistics and KL coefficient (``PPOLearner.update``), the evaluation
+metrics (``EpisodeMetrics.gather``) and so the best checkpoint. A checkpoint is then a main file written by rank 0 with the
+shared state plus one ``checkpoint_<tag>.rank<r>.pt`` shard per rank with that rank's environments and generators."""
 from __future__ import annotations
 
 import json
@@ -15,11 +22,13 @@ import time
 import warnings
 from typing import Any, Callable, Dict, Optional
 
+import numpy as np
 import torch
+import torch.distributed as dist
 
 from ..config.schema import CPPOConfig, EnvironmentConfig
 from ..seeds import SeedManager
-from .collector import RolloutCollector
+from .collector import RolloutCollector, shard_envs
 from .evaluate import evaluate
 from .obs_filter import MeanStdFilter
 from .obs_stats import compute_obs_statistics
@@ -28,6 +37,8 @@ from .ppo import PPOLearner, lr_schedule
 
 METRICS_FILE = "training_metrics.jsonl"
 CHECKPOINT_VERSION = 1
+# what a rank's checkpoint shard holds in a data-parallel run; the main file holds the rest, the same on every rank
+RANK_KEYS = ("learner_gen", "collector", "env", "eval_env")
 
 
 def unsupported_algorithm_fields(algo_config) -> list:
@@ -55,7 +66,26 @@ def unsupported_algorithm_fields(algo_config) -> list:
     return bad
 
 
-def _check(env_config: EnvironmentConfig, algo_config, num_envs: int, horizon: Optional[int]) -> int:
+def _rank_world() -> tuple:
+    """(rank, world size) of the default process group; (0, 1) without one."""
+    if dist.is_available() and dist.is_initialized():
+        return dist.get_rank(), dist.get_world_size()
+    return 0, 1
+
+
+def _rank_seed(seed: int, rank: int) -> int:
+    """The root seed of a rank's streams in a data-parallel run: distinct per rank, a function of ``(seed, rank)`` alone."""
+    return int(np.random.SeedSequence([seed, rank]).generate_state(1, dtype=np.uint32)[0])
+
+
+def shard_path(path: str, rank: int) -> str:
+    """``checkpoint_<tag>.rank<r>.pt`` next to the main file ``checkpoint_<tag>.pt``."""
+    root, ext = os.path.splitext(path)
+    return f"{root}.rank{rank}{ext}"
+
+
+def _check(env_config: EnvironmentConfig, algo_config, num_envs: int, horizon: Optional[int], num_eval_envs: int = 1,
+           world: int = 1) -> int:
     """The horizon of a run, after refusing what the trainer cannot honour; touches no CUDA state."""
     bad = unsupported_algorithm_fields(algo_config)
     if bad:
@@ -65,6 +95,12 @@ def _check(env_config: EnvironmentConfig, algo_config, num_envs: int, horizon: O
         raise ValueError(f"the trainer draws demand on the device (poisson) or from the empirical frame, not from a '{ds}' sampler")
     if int(num_envs) < 1:
         raise ValueError("num_envs must be positive")
+    if world > 1:
+        # equal shards: the mean of the ranks' minibatch gradients is then the gradient of the global minibatch
+        if int(num_envs) % world != 0:
+            raise ValueError(f"num_envs ({num_envs}) must be a multiple of the world size ({world})")
+        if int(num_eval_envs) < world:
+            raise ValueError(f"num_eval_envs ({num_eval_envs}) must be at least the world size ({world})")
     if horizon is None:
         bs = algo_config.shared.batch_size
         if bs % int(num_envs) != 0:
@@ -80,15 +116,19 @@ class Trainer:
     ``num_envs x horizon`` env steps each (``horizon`` defaults to ``batch_size / num_envs``) and writes
     ``out_dir/training_metrics.jsonl``, ``checkpoint_<iter>.pt`` every ``checkpoint_freq`` iterations,
     ``checkpoint_best.pt`` (highest mean evaluation ``episode_return``, summed over the warehouses) and
-    ``checkpoint_final.pt``. ``Trainer.resume(path)`` continues from a checkpoint."""
+    ``checkpoint_final.pt``. ``Trainer.resume(path)`` continues from a checkpoint. Under a default process group of several
+    ranks ``num_envs`` and ``num_eval_envs`` are global: ``num_envs`` must be a multiple of the world size, and every rank
+    needs at least one evaluation environment."""
 
     def __init__(self, env_config: EnvironmentConfig, algo_config, num_envs: int, out_dir: str, seed: int = 0,
                  device=None, horizon: Optional[int] = None, num_eval_envs: Optional[int] = None,
                  env_meta: Optional[Dict[str, Any]] = None, _obs_stats=None):
-        self.horizon = _check(env_config, algo_config, num_envs, horizon)
+        self.rank, self.world = _rank_world()
+        self.num_eval_envs = int(num_eval_envs) if num_eval_envs is not None else min(int(num_envs), 1024)
+        self.horizon = _check(env_config, algo_config, num_envs, horizon, self.num_eval_envs, self.world)
         self.env_config, self.algo_config = env_config, algo_config
         self.num_envs, self.seed = int(num_envs), int(seed)
-        self.num_eval_envs = int(num_eval_envs) if num_eval_envs is not None else min(self.num_envs, 1024)
+        self.group = dist.group.WORLD if self.world > 1 else None
         self.out_dir = str(out_dir)
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
         sh, sp = algo_config.shared, algo_config.algorithm_specific
@@ -98,17 +138,26 @@ class Trainer:
         meta = dict(env_meta or {})
         meta.update(env_meta_from_algorithm_config(algo_config))
         norm = meta["obs_normalization"]
-        seeds = SeedManager(self.seed)
+        # environments, demand, leads, collector and learner draw per rank; the initial weights and the fixed observation
+        # statistics depend on the seed alone
+        seeds = SeedManager(self.seed if self.world == 1 else _rank_seed(self.seed, self.rank))
         if norm in ("meanstd_custom", "meanstd_grouped"):
-            # fixed statistics, once, before the environments are built (runner.py:83-93)
-            self.obs_stats = _obs_stats if _obs_stats is not None else compute_obs_statistics(
-                env_config, SeedManager(self.seed), mode=norm, device=self.device)
+            # fixed statistics, once, before the environments are built (runner.py:83-93); computed on rank 0 and broadcast
+            self.obs_stats = _obs_stats
+            if self.obs_stats is None and self.rank == 0:
+                self.obs_stats = compute_obs_statistics(env_config, SeedManager(self.seed), mode=norm, device=self.device)
+            if _obs_stats is None and self.world > 1:
+                box = [self.obs_stats]
+                dist.broadcast_object_list(box, src=0)
+                self.obs_stats = box[0]
             meta["obs_stats"] = self.obs_stats
         else:
             self.obs_stats = None
         from ..envs import BatchedInventoryEnv
-        self.env = self._make_env(BatchedInventoryEnv, self.num_envs, seeds.get_seed_int("train"), meta, False)
-        self.eval_env = self._make_env(BatchedInventoryEnv, self.num_eval_envs, seeds.get_seed_int("eval"), meta, True)
+        n_train = len(shard_envs(self.num_envs, self.rank, self.world))
+        n_eval = len(shard_envs(self.num_eval_envs, self.rank, self.world))
+        self.env = self._make_env(BatchedInventoryEnv, n_train, seeds.get_seed_int("train"), meta, False)
+        self.eval_env = self._make_env(BatchedInventoryEnv, n_eval, seeds.get_seed_int("eval"), meta, True)
         W, S, D = self.env.n_warehouses, self.env.n_skus, self.env.obs_dim
         self.central = isinstance(algo_config, CPPOConfig)
         with torch.random.fork_rng(devices=[]):
@@ -119,13 +168,15 @@ class Trainer:
         self.filter_dim = W * D if self.central else D
         self.obs_filter = MeanStdFilter(self.filter_dim, self.device) if norm == "meanstd" else None
         self.collector = RolloutCollector(self.env, self.policy, self.horizon, gamma=sp.gamma, lam=sp.lam, seed=col_seed,
-                                          keep_dist_inputs=bool(sp.use_kl_loss), obs_filter=self.obs_filter)
+                                          keep_dist_inputs=bool(sp.use_kl_loss), obs_filter=self.obs_filter,
+                                          process_group=self.group)
         self.learner = PPOLearner.from_algorithm_config(self.policy, algo_config, seed=learn_seed)
         self.iteration = 0
         self.best_return: Optional[float] = None
         os.makedirs(self.out_dir, exist_ok=True)
         self.metrics_path = os.path.join(self.out_dir, METRICS_FILE)
-        open(self.metrics_path, "w").close()
+        if self.rank == 0:
+            open(self.metrics_path, "w").close()
 
     def _make_env(self, cls, n: int, seed: int, meta: Dict[str, Any], eval_env: bool):
         with warnings.catch_warnings():
@@ -155,23 +206,33 @@ class Trainer:
         self.learner.set_lr(lr)
         t0 = self._sync()
         ro = self.collector.collect()
-        reward = float(ro.rewards.reshape(self.horizon, self.num_envs, -1).sum(-1).mean())
+        reward = ro.rewards.reshape(self.horizon, self.env.num_envs, -1).sum(-1).mean()
+        if self.world > 1:
+            dist.all_reduce(reward, op=dist.ReduceOp.SUM)
+            reward = reward / self.world
+        reward = float(reward)
         t1 = self._sync()
         stats = self.learner.update(ro)
         t2 = self._sync()
         self.iteration += 1
         line: Dict[str, Any] = dict(iteration=self.iteration, env_steps=self.iteration * self.steps_per_iteration, lr=lr,
                                     learner=stats, reward_mean=reward, collect_s=t1 - t0, update_s=t2 - t1, eval_s=0.0)
+        if self.world > 1:
+            line["ranks"] = self.world
         if self.iteration % sh.eval_interval == 0:
             frozen = None
             if self.obs_filter is not None:
                 frozen = MeanStdFilter(self.filter_dim, self.device, update=False)
                 frozen.load_state_dict(self.obs_filter.state_dict())
-            summary = evaluate(self.eval_env, self.policy, sh.num_eval_episodes, obs_filter=frozen).summary()
+            metrics = evaluate(self.eval_env, self.policy, sh.num_eval_episodes, obs_filter=frozen)
+            if self.world > 1:
+                metrics = metrics.gather(self.group)
+            summary = metrics.summary()
             line["eval_s"] = self._sync() - t2
             line["eval"] = summary
-        with open(self.metrics_path, "a") as f:
-            f.write(json.dumps(line) + "\n")
+        if self.rank == 0:
+            with open(self.metrics_path, "a") as f:
+                f.write(json.dumps(line) + "\n")
         best = "eval" in line and (self.best_return is None or line["eval"]["episode_return"]["mean"] > self.best_return)
         if best:
             self.best_return = line["eval"]["episode_return"]["mean"]
@@ -206,7 +267,19 @@ class Trainer:
             iteration=self.iteration, env_steps=self.iteration * self.steps_per_iteration, best_return=self.best_return)
 
     def save(self, path: str) -> None:
-        torch.save(self.state_dict(), path)
+        """One file with one process. With several ranks: every rank's shard (``shard_path``), a barrier, then rank 0's main
+        file with the shared state and ``world_size``, so that a main file on disk means the checkpoint is complete."""
+        sd = self.state_dict()
+        if self.world == 1:
+            torch.save(sd, path)
+            return
+        if self.rank == 0 and os.path.exists(path):
+            os.remove(path)                       # a rewritten tag (checkpoint_best) is incomplete until its main file returns
+        dist.barrier()
+        torch.save(dict({k: sd[k] for k in RANK_KEYS}, rank=self.rank, iteration=self.iteration), shard_path(path, self.rank))
+        dist.barrier()
+        if self.rank == 0:
+            torch.save(dict({k: v for k, v in sd.items() if k not in RANK_KEYS}, world_size=self.world), path)
 
     def _load(self, ck: Dict[str, Any]) -> None:
         self.policy.load_state_dict(ck["policy"])
@@ -228,21 +301,35 @@ class Trainer:
                device=None) -> "Trainer":
         """Rebuild a run from one of its checkpoints and continue it in ``out_dir`` (default: the checkpoint's directory),
         whose metrics file keeps the lines up to the checkpoint's iteration. An empirical run passes its ``env_meta``
-        again: the demand frame is not stored."""
+        again: the demand frame is not stored. A checkpoint of a data-parallel run resumes under the same world size only,
+        every rank from the main file and its own shard."""
         from ..config.loader import algorithm_config_from_dict, environment_config_from_dict
         ck = torch.load(path, map_location="cpu", weights_only=False)
         if ck.get("version") != CHECKPOINT_VERSION:
             raise ValueError(f"{path}: checkpoint version {ck.get('version')!r}, this trainer reads {CHECKPOINT_VERSION}")
+        rank, world = _rank_world()
+        saved = int(ck.get("world_size", 1))
+        if saved != world:
+            raise ValueError(f"{path} was written by a run of world size {saved}; this process group has world size {world}")
+        if world > 1:
+            sp = shard_path(path, rank)
+            if not os.path.exists(sp):
+                raise ValueError(f"{path}: the checkpoint shard of rank {rank}, {sp}, is missing")
+            shard = torch.load(sp, map_location="cpu", weights_only=False)
+            if shard.get("rank") != rank or shard.get("iteration") != ck["iteration"]:
+                raise ValueError(f"{sp} is not rank {rank}'s shard of iteration {ck['iteration']}")
+            ck.update({k: shard[k] for k in RANK_KEYS})
         out = out_dir if out_dir is not None else os.path.dirname(os.path.abspath(path))
         metrics = os.path.join(out, METRICS_FILE)
         kept = []
-        if os.path.exists(metrics):
+        if rank == 0 and os.path.exists(metrics):
             with open(metrics) as f:
                 kept = [ln for ln in f if ln.strip() and json.loads(ln)["iteration"] <= ck["iteration"]]
         meta = dict(ck["env_meta"]) if env_meta is None else dict(env_meta)
         tr = cls(environment_config_from_dict(ck["env_config"]), algorithm_config_from_dict(ck["algo_config"]), out_dir=out,
                  device=device, env_meta=meta, _obs_stats=ck["obs_stats"], **ck["args"])
         tr._load(ck)
-        with open(tr.metrics_path, "w") as f:
-            f.writelines(kept)
+        if rank == 0:
+            with open(tr.metrics_path, "w") as f:
+                f.writelines(kept)
         return tr
